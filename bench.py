@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: Lanczos (full re-orthogonalisation) forward + adjoint.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): sparse SPD operator, n = 1M rows, 11 entries per row
 (COO layout of `suite_sparse_load`), Krylov depth 100, fp32, cotangents on the tridiagonal
@@ -21,6 +21,11 @@ the timed region ends with ONE `ncclAllReduce` of it (hutchinson.py:54 over GPUs
 
 `--impl reference`: the reference's algorithm on the host CPUs (the NumPy/SciPy oracle port --
 JAX is not installed in this image, so the reference itself cannot run), bounded sample.
+
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what they computed as `DIR/<name>.npy` in the run's
+dtype (`dump_outputs`): `H` (lanes, probes, K, K) of the last forward, `dv` (lanes, probes, n) of the last adjoint
+and `dparams` (nnz), the parameter cotangent summed over the probes, the lanes and the timed steps.  The inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 """
 
 from __future__ import annotations
@@ -64,6 +69,22 @@ def algorithmic_bytes(n, nnz, K, w):
     fwd = 3 * n * w * K * (K + 1) / 2 + K * (nnz * (w + 4) + 4 * (n + 1)) + 8 * K * n * w
     adj = 3 * n * w * K * (K + 1) + K * (nnz * (3 * w + 4) + 4 * (n + 1)) + 10 * K * n * w
     return fwd, adj
+
+
+DUMP_SAMPLE = 1 << 21  # elements kept of a larger output: three outputs stay under 64 MB even in fp64
+
+
+def dump_outputs(directory, arrays, seed=0):
+    """Write each array as `directory/<name>.npy`.  An array of more than DUMP_SAMPLE elements is written as its
+    elements at DUMP_SAMPLE flat indices drawn from `seed` (ascending), the same indices on every run."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        if a.size > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(seed).choice(a.size, DUMP_SAMPLE, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a))
 
 
 def measured_peaks():
@@ -212,8 +233,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the other BASELINE configurations (`extra`)")
     ap.add_argument("--quick", action="store_true", help="device-timed steps only (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference keeps none")
         return run_reference(args)
 
     # stdout carries exactly ONE line, the JSON: whatever libraries print on file descriptor 1 while the
@@ -354,6 +380,12 @@ def main():
     sampler.start()
     ms_total, launches = timed(lambda first: step_device(first=first), args.steps)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:  # read before the end-to-end steps below reuse the plans and grad_total
+        dump_outputs(args.dump_outputs, {
+            "H": np.stack([pl.H.numpy(pl.stream) for pl in plans]).reshape(L, per_lane, DEPTH, DEPTH),
+            "dv": np.stack([pl.dv.numpy(pl.stream) for pl in plans]).reshape(L, per_lane, N_ROWS),
+            "dparams": grad_total.numpy(main_stream),
+        })  # fmt: skip
     ms_per_step = ms_total / args.steps
     value = world * probes_per_gpu * DEPTH / (ms_per_step * 1e-3)
 

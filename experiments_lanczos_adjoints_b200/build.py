@@ -67,9 +67,12 @@ def _compile(nvcc, src, obj, verbose):
 
 def build(force: bool = False, verbose: bool = False) -> str:
     """Build (or reuse) the library.  Safe when several ranks import the package at once: an exclusive
-    file lock serialises the builders and the late-comers find the finished library."""
+    file lock serialises the builders and the late-comers find the finished library.  A library that is
+    up to date is returned without writing to the tree, so a built tree may be read-only."""
     import fcntl
 
+    if not force and _is_current(_digests()[1]):
+        return LIB
     os.makedirs(OBJ, exist_ok=True)
     with open(os.path.join(OBJ, ".lock"), "w") as lock:
         fcntl.flock(lock, fcntl.LOCK_EX)
@@ -79,14 +82,24 @@ def build(force: bool = False, verbose: bool = False) -> str:
             fcntl.flock(lock, fcntl.LOCK_UN)
 
 
-def _build_locked(force: bool, verbose: bool) -> str:
+def _digests():
+    """Per-source digests and the library's digest over all of them (what STAMP records)."""
     headers = _headers_digest()
     digests = {src: _file_digest(src, headers) for src in sources()}
-    total = hashlib.sha256("".join(digests[s] for s in sorted(digests)).encode()).hexdigest()
-    if not force and os.path.exists(LIB) and os.path.exists(STAMP):
-        with open(STAMP) as f:
-            if f.read().strip() == total:
-                return LIB
+    return digests, hashlib.sha256("".join(digests[s] for s in sorted(digests)).encode()).hexdigest()
+
+
+def _is_current(total: str) -> bool:
+    if not (os.path.exists(LIB) and os.path.exists(STAMP)):
+        return False
+    with open(STAMP) as f:
+        return f.read().strip() == total
+
+
+def _build_locked(force: bool, verbose: bool) -> str:
+    digests, total = _digests()
+    if not force and _is_current(total):
+        return LIB
     nvcc = find_nvcc()
     if nvcc is None:
         if os.path.exists(LIB):

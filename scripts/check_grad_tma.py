@@ -3,6 +3,7 @@ operand (every block staged), a random sparse operand (no block staged) and a ba
 import os
 import subprocess
 import sys
+import tempfile
 
 import numpy as np
 
@@ -42,12 +43,13 @@ if len(sys.argv) > 1 and sys.argv[1] == "child":
     sys.exit(0)
 
 res = {}
+tmp = tempfile.TemporaryDirectory()
 for flag in ("0", "1"):
-    path = f"/tmp/grad_tma_{flag}.npz"
+    path = os.path.join(tmp.name, f"grad_tma_{flag}.npz")
     subprocess.run([sys.executable, __file__, "child", path], check=True, env=dict(os.environ, BL_GRAD_TMA=flag))
-    res[flag] = np.load(path)
+    res[flag] = dict(np.load(path))
 ok = True
-for k in res["0"].files:
+for k in res["0"]:
     a, b = res["0"][k], res["1"][k]
     same = np.array_equal(a, b)
     ok = ok and same and np.isfinite(a).all() and np.abs(a).max() > 0

@@ -3,6 +3,7 @@
 import os
 import subprocess
 import sys
+import tempfile
 
 import numpy as np
 
@@ -34,10 +35,11 @@ if len(sys.argv) > 1 and sys.argv[1] == "child":
     sys.exit(0)
 
 res = {}
+tmp = tempfile.TemporaryDirectory()
 for flag in ("0", "1"):
-    path = f"/tmp/spmv_dots_{flag}.npz"
+    path = os.path.join(tmp.name, f"spmv_dots_{flag}.npz")
     subprocess.run([sys.executable, __file__, "child", path], check=True, env=dict(os.environ, BL_SPMV_DOTS=flag))
-    res[flag] = np.load(path)
+    res[flag] = dict(np.load(path))
 ok = True
 for name, n, K, dtype in CASES:
     tol = 2e-5 if dtype == np.float32 else 1e-11

@@ -30,6 +30,17 @@ def test_library_exports_every_declared_symbol():
     assert b"sm_100a" in _lib.load().bl_version()
 
 
+def test_up_to_date_library_is_reused_without_writing_to_the_tree(tmp_path, monkeypatch):
+    """A built tree may be read-only: loading the library then creates no object directory or lock file."""
+    from experiments_lanczos_adjoints_b200 import build
+
+    build.build()
+    stamp = os.stat(build.STAMP).st_mtime_ns
+    monkeypatch.setattr(build, "OBJ", str(tmp_path / "objects"))
+    assert build.build() == build.LIB
+    assert not os.path.exists(tmp_path / "objects") and os.stat(build.STAMP).st_mtime_ns == stamp
+
+
 def test_header_is_valid_c_and_library_links_from_c(tmp_path):
     """Compile tests/c_abi_smoke.c with gcc against include/b200_lanczos.h and run it."""
     import shutil

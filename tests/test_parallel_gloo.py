@@ -146,7 +146,10 @@ def test_sharded_hutchinson_matches_single_process(tmp_path, worker):
     with socket.socket() as s:
         s.bind(("127.0.0.1", 0))
         port = s.getsockname()[1]
-    env = dict(os.environ, BL_ROOT=ROOT, MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), WORLD_SIZE="2")
+    # host logic only: with a device visible, `comm.init_from_env` binds GPU LOCAL_RANK, which a machine with one
+    # GPU does not have for rank 1; hidden devices make the run the same on machines with none, one or several GPUs
+    env = dict(os.environ, BL_ROOT=ROOT, MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), WORLD_SIZE="2",
+               CUDA_VISIBLE_DEVICES="")  # fmt: skip
     procs = [
         subprocess.Popen([sys.executable, str(script)], env=dict(env, RANK=str(r), LOCAL_RANK=str(r)),
                          stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
