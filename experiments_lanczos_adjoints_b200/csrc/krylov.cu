@@ -18,7 +18,6 @@
 #include "krylov_kernels.cuh"
 #include "stream_kernels.cuh"
 #include "step_kernel.cuh"
-#include "spmv_dots.cuh"
 #include "operators.cuh"
 
 namespace bl {
@@ -70,29 +69,22 @@ struct Common {
   double* coefC;
   double* partials_dots;
   double* partials_comb;
-  double* partials_few;  // [kFewMaxHost][few_capacity]: per-block shares of the neighbouring-row dots (k_op_dots, k_sell_spmv_dots)
+  double* partials_few;  // [kFewMax][kMaxDotsGrid]: per-block shares of k_step_tma's phase 0
   long long partials_dots_count = 0;  // doubles behind partials_dots
-  long long few_capacity = 0;         // blocks per value behind partials_few
 };
-constexpr int kFewMaxHost = 4;
-constexpr int kSpmvDotsMinThreads = 256;
-// shares per value the workspace holds: the grid of the streaming kernels or of k_sell_spmv_dots (one block per 8+ slices)
-long long few_capacity_for(int64_t n) {
-  return std::max<long long>(kMaxDotsGrid, (n + kSpmvDotsMinThreads - 1) / kSpmvDotsMinThreads + 1);
-}
 
-size_t common_bytes(int64_t n, int64_t K) {
+size_t common_bytes(int64_t K) {
   size_t b = 0;
   b += 256;                                   // counters
   b += align_up(S_COUNT * 8, 256);            // scal
   b += 4 * align_up((K + 2) * 8, 256);        // red, coefA, coefB, coefC
   b += align_up((size_t)(K + 2) * kMaxDotsGrid * 8, 256);  // partials_dots
   b += align_up((size_t)kMaxCombineGrid * 8, 256);         // partials_comb
-  b += align_up((size_t)kFewMaxHost * few_capacity_for(n) * 8, 256);  // partials_few
+  b += align_up((size_t)kFewMax * kMaxDotsGrid * 8, 256);  // partials_few
   return b + 9 * 256;
 }
 
-void carve_common(Workspace& w, int64_t K, Common& c, int64_t n = 0) {
+void carve_common(Workspace& w, int64_t K, Common& c) {
   c.counters = static_cast<unsigned int*>(w.take(256));
   c.scal = static_cast<double*>(w.take(S_COUNT * 8));
   c.red = static_cast<double*>(w.take((K + 2) * 8));
@@ -102,19 +94,11 @@ void carve_common(Workspace& w, int64_t K, Common& c, int64_t n = 0) {
   c.partials_dots = static_cast<double*>(w.take((size_t)(K + 2) * kMaxDotsGrid * 8));
   c.partials_dots_count = (long long)(K + 2) * kMaxDotsGrid;
   c.partials_comb = static_cast<double*>(w.take((size_t)kMaxCombineGrid * 8));
-  c.few_capacity = few_capacity_for(n);
-  c.partials_few = static_cast<double*>(w.take((size_t)kFewMaxHost * c.few_capacity * 8));
+  c.partials_few = static_cast<double*>(w.take((size_t)kFewMax * kMaxDotsGrid * 8));
 }
 
-// BL_STREAM=0 forces the register-staged (LDG) kernels; default: TMA-staged kernels for n >= 8192.
-int stream_mode() {
-  static int mode = [] {
-    const char* e = std::getenv("BL_STREAM");
-    return e ? std::atoi(e) : 1;
-  }();
-  return mode;
-}
-bool use_tma(int64_t n) { return stream_mode() != 0 && n >= 8192; }
+// TMA-staged kernels for n >= 8192; below that the register-staged (LDG) kernels.
+bool use_tma(int64_t n) { return n >= 8192; }
 
 template <typename T>
 constexpr int dots_tile() { return BL_DOTS_TILE_BYTES / (int)sizeof(T); }  // row segment per copy
@@ -135,7 +119,7 @@ int tma_grid(int64_t n, int tile) {
   return (int)std::max<int64_t>(1, std::min<int64_t>(std::min(blocks_per_sm() * sm_count(), kMaxDotsGrid), (n + tile - 1) / tile));
 }
 
-// Launch with the programmatic-dependent-launch attribute (BL_PDL=0 disables it): the kernel's
+// Launch with the programmatic-dependent-launch attribute: the kernel's
 // prologue and its first TMA loads overlap the tail (imbalance, last-block reduction) of the
 // kernel in front of it; the kernel itself executes griddepcontrol.wait before reading anything
 // its predecessor wrote.
@@ -217,30 +201,14 @@ int finish_sharded(const Common& c, Epi epi, int count, cudaStream_t s) {
   return BL_OK;
 }
 
-// L2 "snake" order (BL_SNAKE=0 disables it): consecutive streaming kernels walk the basis in
+// L2 "snake" order: consecutive streaming kernels walk the basis in
 // opposite directions, so a kernel starts on the tiles its predecessor read last — the part of
 // the basis that is still in the 126 MB L2.  Each block owns the same column range in every
 // kernel (same grid, same partition), which makes the reuse exact.
-bool snake_enabled() {
-  static int mode = [] {
-    const char* e = std::getenv("BL_SNAKE");
-    return e ? std::atoi(e) : 1;
-  }();
-  return mode != 0;
-}
 thread_local int g_direction = 0;  // toggled per streaming launch; host-side launch order is the stream order
 int next_direction() {
-  if (!snake_enabled()) return 0;
   g_direction ^= 1;
   return g_direction;
-}
-
-bool pdl_enabled() {
-  static int mode = [] {
-    const char* e = std::getenv("BL_PDL");
-    return e ? std::atoi(e) : 1;
-  }();
-  return mode != 0;
 }
 
 template <typename... KArgs, typename... Args>
@@ -254,7 +222,7 @@ cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, size_t sme
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
@@ -274,28 +242,8 @@ int set_smem(F* kernel, size_t bytes) {
   return BL_OK;
 }
 
-// BL_DOTS_FEW=0 sends dots with <= 4 rows through the TMA pipeline like the wide ones (A/B measurements).
-bool few_rows_enabled() {
-  static const bool enabled = [] {
-    const char* e = std::getenv("BL_DOTS_FEW");
-    return !(e && e[0] == '0');
-  }();
-  return enabled;
-}
-
-// Basis rows are copied with the L2 evict_first policy by the separate streaming kernels too (the step kernel:
-// BL_STEP_L2): measured +4 % for one run alone; BL_ROWS_L2=0 switches it off.
-int rows_evict_first() {
-  static const int on = [] {
-    const char* e = std::getenv("BL_ROWS_L2");
-    return e ? std::atoi(e) : 1;
-  }();
-  return on;
-}
-
 RowSource row_source(const RowBlock& b0, const RowBlock* b1, size_t w) {
   RowSource r;
-  r.evict_first = rows_evict_first();
   r.base0 = static_cast<const char*>(b0.base) + (long long)b0.row0 * b0.ld * (long long)w;
   r.ldb0 = b0.ld * (long long)w;
   r.n0 = b0.nrows;
@@ -319,7 +267,7 @@ int launch_dots(const Grid& g, const Common& c, RowBlock blk, const T* x, int64_
   if (sharded) epi.mode = EPI_NONE;
   {
   ProfScope prof(BL_PROF_DOTS, (double)(blk.nrows + 1) * n * sizeof(T), s);
-  if (use_tma(n) && blk.nrows <= 4 && few_rows_enabled()) {
+  if (use_tma(n) && blk.nrows <= 4) {
     FewRows fr;
     for (int j = 0; j < blk.nrows; ++j)
       fr.row[j] = static_cast<const char*>(blk.base) + (long long)(blk.row0 + j) * blk.ld * (long long)sizeof(T);
@@ -513,13 +461,13 @@ int launch_fused_tile(const Common& c, const FusedSpec& f, int dtype, int sr, cu
   return BL_OK;
 }
 
-// `*fused` is false on return when no tile shape fits shared memory or the TMA path is off;
+// `*fused` is false on return when no tile shape fits shared memory or n is below the TMA threshold;
 // the caller then runs combine and dots separately.
 template <typename T>
 int launch_fused(const Common& c, const FusedSpec& f, int dtype, cudaStream_t s, bool* fused) {
   *fused = false;
   // k_fused_tma keeps one register accumulator per resident box: at most 16 boxes = 128 rows
-  if (!use_tma(f.n) || stream_mode() == 2 || f.n >= ((int64_t)1 << 31) || f.res.nrows > 128) return BL_OK;
+  if (!use_tma(f.n) || f.n >= ((int64_t)1 << 31) || f.res.nrows > 128) return BL_OK;
   // every tile pays a fixed chain (exchange, barriers, sweep hand-over) of about a microsecond: with
   // fewer than ~16 rows per tile that costs more than the second read of the rows it saves
   if (f.res.nrows + f.str0.nrows + f.str1.nrows < 16) return BL_OK;
@@ -546,8 +494,8 @@ int launch_fused(const Common& c, const FusedSpec& f, int dtype, cudaStream_t s,
 }
 
 // out = (sum of <= kXTerms vector terms) / div and red[j] = <row_j, out> over a block of basis rows: the symmetric
-// loops' replacement for the fused kernel (k_xdots_tma, stream_kernels.cuh).  `*done` stays false when the TMA
-// path is off or the shape does not fit; the caller then runs its general kernels.  BL_XDOTS=0 disables it.
+// loops' replacement for the fused kernel (k_xdots_tma, stream_kernels.cuh).  `*done` stays false when n is
+// below the TMA threshold or the shape does not fit; the caller then runs its general kernels.
 struct XDotsSpec {
   int64_t n = 0;
   void* out = nullptr;
@@ -556,19 +504,7 @@ struct XDotsSpec {
   RowBlock rows;
   const double* out_div_ptr = nullptr;
   Epi epi;
-  // the neighbouring-row dots arrive as per-block shares (k_op_dots): the kernel adds them up and runs pre_epi first
-  const double* pre_partials = nullptr;
-  int pre_count = 0, pre_grid = 0;
-  Epi pre_epi;
 };
-
-bool xdots_enabled() {
-  static const bool enabled = [] {
-    const char* e = std::getenv("BL_XDOTS");
-    return !(e && e[0] == '0');
-  }();
-  return enabled;
-}
 
 template <typename T>
 int launch_xdots(const Common& c, const XDotsSpec& f, cudaStream_t s, bool* done) {
@@ -576,9 +512,7 @@ int launch_xdots(const Common& c, const XDotsSpec& f, cudaStream_t s, bool* done
   constexpr int TILE = kConsumerThreads * Vec<T>::N;  // 4 KB row segments
   const size_t smem = (size_t)(kStages * kGroup + 2) * TILE * sizeof(T) + (2 * kStages + 4) * 8 +
                       (size_t)f.rows.nrows * 8 + 16;
-  if (!xdots_enabled() || !use_tma(f.n) || stream_mode() == 2 || f.nvec > kXTerms || f.rows.nrows < 1 ||
-      smem > 112 * 1024)
-    return BL_OK;
+  if (!use_tma(f.n) || f.nvec > kXTerms || f.rows.nrows < 1 || smem > 112 * 1024) return BL_OK;
   *done = true;
   XDotsArgs a;
   a.src = row_source(f.rows, nullptr, sizeof(T));
@@ -593,12 +527,6 @@ int launch_xdots(const Common& c, const XDotsSpec& f, cudaStream_t s, bool* done
   a.epi = f.epi;
   a.epi.red = c.red;
   a.epi.scal = c.scal;
-  a.pre_partials = f.pre_partials;
-  a.pre_count = f.pre_count;
-  a.pre_grid = f.pre_grid;
-  a.pre_epi = f.pre_epi;
-  a.pre_epi.red = c.red;
-  a.pre_epi.scal = c.scal;
   const Epi full_epi = a.epi;
   int prc = BL_OK;
   const bool peer = arm_peer_epilogue(a.epi, f.rows.nrows, &prc);
@@ -616,33 +544,10 @@ int launch_xdots(const Common& c, const XDotsSpec& f, cudaStream_t s, bool* done
   return BL_OK;
 }
 
-// One launch for the three basis-streaming phases of a symmetric-loop step (k_step_tma, step_kernel.cuh).
-// BL_STEP=0 disables it, 1 (default) uses it for lockstep batches, 2 also for a single run; BL_STEP_PDL=0 launches
-// it without the programmatic-dependent-launch attribute.  The kernel's blocks wait for one another, so the launch is cooperative (the driver starts the
-// grid only when all of it is resident: kernels of other streams cannot wedge it) and the grid is capped at
-// what fits the device.
-int step_mode() {
-  static const int mode = [] {
-    const char* e = std::getenv("BL_STEP");
-    return e ? std::atoi(e) : 1;
-  }();
-  return mode;
-}
-bool step_pdl() {
-  static const bool on = [] {
-    const char* e = std::getenv("BL_STEP_PDL");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
+// One launch for the three basis-streaming phases of a symmetric-loop step (k_step_tma, step_kernel.cuh).  The kernel's
+// blocks wait for one another, so the launch is cooperative (the driver starts the grid only when all of it is
+// resident: kernels of other streams cannot wedge it) and the grid is capped at what fits the device.
 std::atomic<int> g_step_pdl_ok{1};  // cleared when the driver refuses cooperative + programmatic launch together
-bool step_coop() {  // BL_STEP_COOP=0: plain launch (measurements on ONE stream only: nothing else may hold SM slots)
-  static const bool on = [] {
-    const char* e = std::getenv("BL_STEP_COOP");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
 std::atomic<int> g_step_trace_next{-1};  // bl_step_trace_begin arms it; every k_step_tma launch takes a slot
 
 struct StepItem {  // one run's share of a k_step_tma launch
@@ -652,25 +557,9 @@ struct StepItem {  // one run's share of a k_step_tma launch
   const StepOp* op = nullptr;  // the step's operator call rides in the launch (same for every run of a batch)
 };
 
-constexpr int kOpStagesHost = step::kOpStages;
-// BL_STEP_OP=0: the operator call stays its own launch (A/B measurements).
-bool step_op_enabled() {
-  static const bool on = [] {
-    const char* e = std::getenv("BL_STEP_OP");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-
 // The operator call of a Krylov step as phase S of k_step_tma: operands stored as SELL-32 only (SparseOperator).
 // norm: the forward's q = v / len on the way, rows written up to n_pad.
 bool make_step_op(bl_operator_t* op, int dtype, bool transpose, bool norm, int64_t n, int64_t n_pad, StepOp* so) {
-  if (!step_op_enabled() || step_mode() == 0) return false;
-  static const int sides = [] {  // BL_STEP_OP_SIDES: bit 0 forward sweeps, bit 1 adjoint sweeps (debugging)
-    const char* e = std::getenv("BL_STEP_OP_SIDES");
-    return e ? std::atoi(e) : 3;
-  }();
-  if (!(sides & (transpose ? 2 : 1))) return false;
   SellView v;
   if (!op->sell_view(dtype, transpose, &v)) return false;
   if (v.nrows != n || (norm && n_pad > v.nslices * 32)) return false;
@@ -682,24 +571,13 @@ bool make_step_op(bl_operator_t* op, int dtype, bool transpose, bool norm, int64
   so->nrows = v.nrows;
   so->n_pad = n_pad;
   so->norm = norm ? 1 : 0;
-  static const int hints = [] {  // BL_STEP_L2: bit 0 basis rows evict_first, bit 1 operand evict_last
-    const char* e = std::getenv("BL_STEP_L2");
-    return e ? std::atoi(e) : 1;
-  }();
-  so->l2_hints = hints;
-  static const int depth = [] {  // BL_STEP_DEPTH: fine stages of phase S's ring the producer keeps in flight (4..12)
-    const char* e = std::getenv("BL_STEP_DEPTH");
-    const int d = e ? std::atoi(e) : 8;
-    return d < 4 ? 4 : (d > kOpStagesHost ? kOpStagesHost : d);
-  }();
-  so->depth = depth;
   return true;
 }
 
 template <typename T>
 size_t step_smem_bytes(int count, int acc_stride, int coef_stride) {
   constexpr int TILE = kConsumerThreads * Vec<T>::N;
-  return (size_t)(kStages * kGroup + 2) * TILE * sizeof(T) + (2 * kStages + 2 + 2 * kOpStagesHost) * 8 +
+  return (size_t)(kStages * kGroup + 2) * TILE * sizeof(T) + (2 * kStages + 2 + 2 * step::kOpStages) * 8 +
          (size_t)count * acc_stride * 8 + (size_t)count * coef_stride * sizeof(T) + 16;
 }
 
@@ -728,19 +606,17 @@ bool step_fits(int blocks) {
 }
 
 // The step of `count` runs (same n, same dtype) in ceil(count / kStepBatch) launches.  `*done` stays false -- nothing
-// launched -- when the kernel does not apply (switched off, row sharding, shape); the caller then runs the separate
-// kernels for every run.  min_batch: BL_STEP=1 (default) uses the kernel for batches of two or more runs only -- for
-// ONE run an in-kernel reduction costs what a kernel boundary with programmatic dependent launch costs (measured:
-// 24.3 vs 23.6 ms per forward + adjoint at n = 1M, depth 100) -- BL_STEP=2 for every run, BL_STEP=0 never.
+// launched -- when the kernel does not apply (one run, row sharding, shape); the caller then runs the separate
+// kernels for every run.  Batches of two or more runs only: for ONE run an in-kernel reduction costs what a kernel
+// boundary with programmatic dependent launch costs (measured: 24.3 vs 23.6 ms per forward + adjoint at n = 1M,
+// depth 100).
 template <typename T>
 int launch_step(std::vector<StepItem>& items, cudaStream_t s, bool* done) {
   *done = false;
   constexpr int TILE = kConsumerThreads * Vec<T>::N;
   const int total = (int)items.size();
-  const int mode = step_mode();
-  const StepOp* sop = total > 0 ? items[0].op : nullptr;
-  if (total < 1 || mode == 0 || (mode == 1 && total < 2) || !xdots_enabled() || stream_mode() == 2 || is_sharded())
-    return BL_OK;
+  if (total < 2 || is_sharded()) return BL_OK;
+  const StepOp* sop = items[0].op;
   const long long n = items[0].a.n;
   if (!use_tma(n)) return BL_OK;
   int acc_stride = kFewSlots, coef_stride = kGroup;
@@ -754,13 +630,12 @@ int launch_step(std::vector<StepItem>& items, cudaStream_t s, bool* done) {
   // largest batch per launch whose per-run coefficient blocks still fit beside the ring (two blocks per SM)
   int per_launch = std::min(total, kStepBatch);
   while (per_launch > 1 && step_smem_bytes<T>(per_launch, acc_stride, coef_stride) > 112 * 1024) --per_launch;
-  if (step_smem_bytes<T>(per_launch, acc_stride, coef_stride) > 112 * 1024) return BL_OK;
-  if (mode == 1 && per_launch < 2) return BL_OK;
+  if (per_launch < 2) return BL_OK;
   BL_CHECK(set_smem(k_step_tma<T, TILE>, 112 * 1024));
   if (!step_fits<T>(blocks_per_sm())) return BL_OK;
   *done = true;
   const int grid = tma_grid<T>(n, TILE);
-  const bool pdl = pdl_enabled() && step_pdl() && g_step_pdl_ok.load(std::memory_order_relaxed) != 0;
+  const bool pdl = g_step_pdl_ok.load(std::memory_order_relaxed) != 0;
   for (int first = 0; first < total; first += per_launch) {
     StepBatch B;
     B.count = std::min(per_launch, total - first);
@@ -802,21 +677,14 @@ int launch_step(std::vector<StepItem>& items, cudaStream_t s, bool* done) {
     cfg.dynamicSmemBytes = smem;
     cfg.stream = s;
     cudaLaunchAttribute attr[2];
-    int na = 0;
-    if (step_coop()) {
-      attr[na].id = cudaLaunchAttributeCooperative;
-      attr[na].val.cooperative = 1;
-      ++na;
-    }
-    if (pdl) {
-      attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      attr[na].val.programmaticStreamSerializationAllowed = 1;
-      ++na;
-    }
+    attr[0].id = cudaLaunchAttributeCooperative;
+    attr[0].val.cooperative = 1;
+    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = na;
+    cfg.numAttrs = pdl ? 2 : 1;
     cudaError_t err = cudaLaunchKernelEx(&cfg, k_step_tma<T, TILE>, B);
-    if (err != cudaSuccess && pdl && step_coop()) {  // cooperative + programmatic refused together: cooperative alone
+    if (err != cudaSuccess && pdl) {  // cooperative + programmatic refused together: cooperative alone
       (void)cudaGetLastError();
       g_step_pdl_ok.store(0, std::memory_order_relaxed);
       cfg.numAttrs = 1;
@@ -825,119 +693,6 @@ int launch_step(std::vector<StepItem>& items, cudaStream_t s, bool* done) {
     BL_CUDA(err);
     BL_LAUNCHED();
   }
-  return BL_OK;
-}
-
-// BL_OP_DOTS=1: one run alone takes its operator call and the block-local part of the neighbouring-row dots from ONE
-// plain launch (k_op_dots; 611 launches per run instead of 811).  Off by default: measured 23.8 vs 22.9 ms per forward +
-// adjoint at n = 1M -- inside a kernel whose blocks carry the 96 KB ring the operator call has 16 warps per SM instead
-// of the stand-alone SpMV's 40, and what the k_dots_few launch cost comes back as the longer operator kernel.
-bool op_dots_enabled() {
-  static const bool on = [] {
-    const char* e = std::getenv("BL_OP_DOTS");
-    return e && e[0] == '1';
-  }();
-  return on;
-}
-
-// Operator call + block-local neighbouring-row dots of `items.size()` runs in one PLAIN launch (k_op_dots); the shares
-// land in each run's c.partials_few and the run's next k_xdots_tma launch finishes the reduction (XDotsSpec::pre_*).
-// `*done` stays false when the kernel does not apply.  `*grid_out`: blocks that wrote shares.
-template <typename T>
-int launch_op_dots(std::vector<StepItem>& items, double op_bytes, cudaStream_t s, bool* done, int* grid_out) {
-  *done = false;
-  constexpr int TILE = kConsumerThreads * Vec<T>::N;
-  const int total = (int)items.size();
-  if (total < 1 || total > kStepBatch || !op_dots_enabled() || !xdots_enabled() || stream_mode() != 1 || is_sharded())
-    return BL_OK;
-  const StepOp* sop = items[0].op;
-  const long long n = items[0].a.n;
-  if (sop == nullptr || !use_tma(n)) return BL_OK;
-  for (const StepItem& it : items)
-    if (it.op != sop || it.a.n != n || it.a.few_n < 1 || it.a.few_n > kFewMax || it.a.op_x == nullptr || it.a.op_x == it.a.few_x)
-      return BL_OK;
-  const size_t smem = step_smem_bytes<T>(total, kFewSlots, kGroup);
-  if (smem > 112 * 1024) return BL_OK;
-  BL_CHECK(set_smem(k_op_dots<T, TILE>, 112 * 1024));
-  const int grid = tma_grid<T>(n, TILE);
-  if (grid > kMaxDotsGrid) return BL_OK;
-  *done = true;
-  *grid_out = grid;
-  StepBatch B;
-  B.count = total;
-  B.acc_stride = kFewSlots;
-  B.coef_stride = kGroup;
-  B.op = *sop;
-  double bytes = op_bytes;  // + the rows of the dots (the operand's output is still on the chip)
-  for (int p = 0; p < total; ++p) {
-    B.a[p] = items[p].a;
-    B.a[p].partials = items[p].c->partials_few;
-    bytes += (double)items[p].a.few_n * n * sizeof(T);
-  }
-  ProfScope prof(BL_PROF_MATVEC, bytes, s);
-  k_op_dots<T, TILE><<<grid, kStreamThreads, smem, s>>>(B);
-  BL_LAUNCHED();
-  return BL_OK;
-}
-
-// BL_SPMV_DOTS=1: one run alone takes its operator call and the shares of its neighbouring-row dots from ONE launch
-// (k_sell_spmv_dots; 611 launches per run instead of 811).  Off by default: measured 23.8 (256 threads per block) / 23.9
-// (512) / 24.3 ms (1024) against 23.0 ms per forward + adjoint at n = 1M -- under programmatic dependent launch the 200
-// k_dots_few launches it removes were mostly hidden already, and adding up thousands of shares in every block of the
-// next kernel costs more than what was left of them.
-// BL_SPMV_DOTS_THREADS: threads per block of k_sell_spmv_dots (256..1024; shares per value = slices / warps per block).
-int spmv_dots_threads() {
-  static const int t = [] {
-    const char* on = std::getenv("BL_SPMV_DOTS");
-    if (!(on && on[0] == '1')) return 0;
-    const char* e = std::getenv("BL_SPMV_DOTS_THREADS");
-    int v = e ? std::atoi(e) : 512;
-    v = std::max(kSpmvDotsMinThreads, std::min(kSpmvDotsMaxWarps * 32, v));
-    return v / 32 * 32;
-  }();
-  return t;
-}
-
-// Operator call of one run (SELL-32 operand) + per-block shares of <few_j, y> in c.partials_few, one PLAIN launch
-// (k_sell_spmv_dots).  `*grid_out` stays 0 -- nothing launched -- when the kernel does not apply.
-template <typename T>
-int launch_spmv_dots(bl_operator_t* op, int dtype, bool transpose, int64_t n, int64_t n_pad, const T* x, const double* len,
-                     T* q, T* y, int few_n, const void* const* few_rows, int self, const Common& c, double op_bytes,
-                     cudaStream_t s, int* grid_out) {
-  *grid_out = 0;
-  const int threads = spmv_dots_threads();
-  if (threads == 0 || !xdots_enabled() || stream_mode() != 1 || is_sharded() || !use_tma(n) || few_n < 1 || few_n > kFewMax ||
-      x == y)
-    return BL_OK;
-  SellView v;
-  if (!op->sell_view(dtype, transpose, &v)) return BL_OK;
-  const bool norm = len != nullptr;
-  if (v.nrows != n || (norm && n_pad > v.nslices * 32)) return BL_OK;
-  const int wpb = threads / 32;
-  const long long grid = (v.nslices + wpb - 1) / wpb;
-  if (grid < 1 || grid > c.few_capacity) return BL_OK;
-  SpmvDotsArgs a;
-  a.slice_ptr = v.slice_ptr;
-  a.col = v.col;
-  a.val = v.val;
-  a.nslices = v.nslices;
-  a.nrows = v.nrows;
-  a.n_pad = n_pad;
-  a.x = x;
-  a.y = y;
-  a.len = len;
-  a.q = q;
-  a.few_n = few_n;
-  for (int j = 0; j < few_n; ++j) a.few_row[j] = few_rows[j];
-  a.self = self;
-  a.partials = c.partials_few;
-  ProfScope prof(BL_PROF_MATVEC, op_bytes + (double)few_n * n * sizeof(T), s);
-  if (norm)
-    k_sell_spmv_dots<T, true, 6><<<(int)grid, threads, 0, s>>>(a);
-  else
-    k_sell_spmv_dots<T, false, 6><<<(int)grid, threads, 0, s>>>(a);
-  BL_LAUNCHED();
-  *grid_out = (int)grid;
   return BL_OK;
 }
 
@@ -983,14 +738,9 @@ int check_basis(int dtype, int64_t n, int64_t K, int64_t ld, const void* Q) {
   return BL_OK;
 }
 
-// BL_FWD_SYMMETRIC of the caller's flags (needs the second pass); BL_SYMMETRIC_FORWARD=0 in the
-// environment switches it off (A/B measurements, debugging).
+// BL_FWD_SYMMETRIC of the caller's flags (needs the second pass)
 bool symmetric_forward(int flags) {
-  static const bool enabled = [] {
-    const char* e = std::getenv("BL_SYMMETRIC_FORWARD");
-    return !(e && e[0] == '0');
-  }();
-  return enabled && (flags & BL_FWD_SYMMETRIC) != 0 && (flags & BL_FWD_SECOND_PASS) != 0;
+  return (flags & BL_FWD_SYMMETRIC) != 0 && (flags & BL_FWD_SECOND_PASS) != 0;
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1040,19 +790,6 @@ struct FwdRun {
     ProfScope prof(BL_PROF_MATVEC, op->matvec_bytes(dtype), s);
     return op->matvec(dtype, q_row(i), r, s);
   }
-  // the same as ONE launch that also leaves the first pass's dots <q_j, A q_i>, j = first_lo(i)..i, as per-block shares
-  // (k_sell_spmv_dots; symmetric loops of one run alone).  `*pre_grid` stays 0 when it does not apply.
-  int advance_dots(int i, int* pre_grid) {
-    *pre_grid = 0;
-    if (!(second_pass && local_first)) return BL_OK;
-    const int j0 = first_lo(i);
-    const void* few[kFewMax];
-    for (int j = j0; j <= i; ++j) few[j - j0] = q_row(j);
-    BL_CHECK(launch_spmv_dots<T>(op, dtype, false, n, ld, r, c.scal + S_LEN, q_row(i), alt, i + 1 - j0, few, i - j0, c,
-                                 op->matvec_bytes(dtype) + 1.0 * n * sizeof(T), s, pre_grid));
-    if (*pre_grid > 0) std::swap(r, alt);
-    return BL_OK;
-  }
   int finish() {
     if (r != r_out) {
       BL_CUDA(cudaMemcpyAsync(r_out, r, (size_t)n * sizeof(T), cudaMemcpyDeviceToDevice, s));
@@ -1063,7 +800,7 @@ struct FwdRun {
 
   int begin() {
   Workspace w(workspace, wbytes);
-  carve_common(w, K, c, n);
+  carve_common(w, K, c);
   alt = static_cast<T*>(w.take((size_t)ld * sizeof(T)));
   r_out = r;
   BL_REQUIRE(w.ok(), "workspace too small (bl_arnoldi_workspace_bytes)");
@@ -1157,18 +894,8 @@ struct FwdRun {
     return true;
   }
   void unfuse() { std::swap(r, alt); }
-  bool skip_step = false;  // the batch driver already tried the step kernel for this step
-  // pre_grid > 0: the operator call came from k_op_dots, which left the first pass's dots as per-block shares
-  int post(int i, int pre_grid = 0) {
+  int post(int i) {
     const int m = i + 1;
-    if (!skip_step && pre_grid == 0) {
-      std::vector<StepItem> items(1);
-      if (step_item(i, items[0])) {
-        bool stepped = false;
-        BL_CHECK(launch_step<T>(items, s, &stepped));
-        if (stepped) return BL_OK;
-      }
-    }
     Epi epi_a;  // h = Q^H v (active columns only)                              arnoldi.py:87
     epi_a.mode = EPI_FWD_A;
     epi_a.i = i;
@@ -1182,8 +909,9 @@ struct FwdRun {
     norm_epi.i = i;
     norm_epi.K = K;
     norm_epi.H = H;
+    BL_CHECK(launch_dots<T>(g, c, rows(Q, ld, epi_a.j0, epi_a.m), r, n, epi_a, s));
     bool fused = false;
-    auto pass_b_xdots = [&](bool with_pre) {
+    if (second_pass && local_first) {
       // symmetric loop: v = v - h_{i-1} q_{i-1} - h_i q_i is a three-vector combination, and h2 = Q^H v streams
       // every active row once (no row is needed twice: nothing stays resident)   arnoldi.py:88,92
       XDotsSpec f;
@@ -1193,18 +921,7 @@ struct FwdRun {
       for (int j = first_lo(i); j < m; ++j) f.vec[f.nvec++] = term(q_row(j), -1.0, c.coefA + j);
       f.rows = rows(Q, ld, 0, m);
       f.epi = pass_b_epi(i);
-      if (with_pre) {
-        f.pre_partials = c.partials_few;
-        f.pre_count = epi_a.m;
-        f.pre_grid = pre_grid;
-        f.pre_epi = epi_a;
-      }
-      return launch_xdots<T>(c, f, s, &fused);
-    };
-    if (pre_grid > 0 && second_pass && local_first) BL_CHECK(pass_b_xdots(true));
-    if (!fused) {
-      BL_CHECK(launch_dots<T>(g, c, rows(Q, ld, epi_a.j0, epi_a.m), r, n, epi_a, s));
-      if (second_pass && local_first) BL_CHECK(pass_b_xdots(false));
+      BL_CHECK(launch_xdots<T>(c, f, s, &fused));
     }
     if (second_pass && !fused) {
       // v = v - Q h and, from the same read of Q, h2 = Q^H v (the second pass's coefficients;
@@ -1252,35 +969,7 @@ int arnoldi_forward_t(bl_operator_t* op, int dtype, int64_t n, int K, int flags,
   FwdRun<T> run{op, dtype, n, K, (flags & BL_FWD_SECOND_PASS) != 0, v, Q, ld, H, r, c_out, workspace, wbytes, s, {}, {}};
   run.local_first = symmetric_forward(flags);
   BL_CHECK(run.begin());
-  StepOp sop;
-  const bool fuse = run.second_pass && run.local_first && make_step_op(op, dtype, false, true, n, ld, &sop);
   for (int i = 0; i < K; ++i) {
-    if (fuse) {  // operator call + Gram-Schmidt step in one launch
-      std::vector<StepItem> items(1);
-      sop.wait_first = i == 0;
-      if (run.fused_item(i, &sop, items[0])) {
-        bool stepped = false;
-        BL_CHECK(launch_step<T>(items, s, &stepped));
-        if (stepped) continue;
-        // one run alone: operator call + block-local dots as one plain launch, reduction finished by k_xdots_tma
-        bool done = false;
-        int pre_grid = 0;
-        BL_CHECK(launch_op_dots<T>(items, op->matvec_bytes(dtype) + 1.0 * n * sizeof(T), s, &done, &pre_grid));
-        if (done) {
-          BL_CHECK(run.post(i, pre_grid));
-          continue;
-        }
-        run.unfuse();
-      }
-    }
-    {  // one run alone: operator call + shares of the neighbouring-row dots in one plain launch, finished by k_xdots_tma
-      int pre_grid = 0;
-      BL_CHECK(run.advance_dots(i, &pre_grid));
-      if (pre_grid > 0) {
-        BL_CHECK(run.post(i, pre_grid));
-        continue;
-      }
-    }
     BL_CHECK(run.advance(i));
     BL_CHECK(run.post(i));
   }
@@ -1355,24 +1044,14 @@ int arnoldi_forward_batch_t(bl_operator_t* op, int dtype, int64_t n, int K, int 
       if (eligible) BL_CHECK(launch_step<T>(items, s, &stepped));
       if (stepped) continue;
     }
-    for (int p = 0; p < P; ++p) {
-      runs[p].skip_step = P > 1;  // the batch did not apply: neither does a batch of one under BL_STEP=1
-      BL_CHECK(runs[p].post(i));
-    }
+    for (int p = 0; p < P; ++p) BL_CHECK(runs[p].post(i));
   }
   for (int p = 0; p < P; ++p) BL_CHECK(runs[p].finish());
   return BL_OK;
 }
 
-// BL_ADJ_SYMMETRIC of the caller's flags; BL_SYMMETRIC_ADJOINT=0 in the environment switches the
-// shortcut off (A/B measurements, debugging).
-bool symmetric_shortcut(int flags) {
-  static const bool enabled = [] {
-    const char* e = std::getenv("BL_SYMMETRIC_ADJOINT");
-    return !(e && e[0] == '0');
-  }();
-  return enabled && (flags & BL_ADJ_SYMMETRIC) != 0;
-}
+// BL_ADJ_SYMMETRIC of the caller's flags
+bool symmetric_shortcut(int flags) { return (flags & BL_ADJ_SYMMETRIC) != 0; }
 
 // ---------------------------------------------------------------------------------------
 // One Arnoldi adjoint run, split at the operator call (see FwdRun): begin(), then for idx = K-1..0
@@ -1430,7 +1109,7 @@ struct AdjRun {
 
   int begin() {
   Workspace w(workspace, wbytes);
-  carve_common(w, K, c, n);
+  carve_common(w, K, c);
   eta = static_cast<double*>(w.take((size_t)K * 8));
   Gamma = static_cast<double*>(w.take((size_t)K * K * 8));
   PiGamma = static_cast<double*>(w.take((size_t)K * K * 8));
@@ -1587,36 +1266,12 @@ struct AdjRun {
     item.bytes += op->apply_transpose_bytes(dtype);
     return true;
   }
-  // z = A^T Lambda[idx] and the shares of its dots with rows band_lo(idx)..idx in one plain launch (k_sell_spmv_dots;
-  // banded Gamma, deferred parameter cotangent, one run alone).  `*pre_grid` stays 0 when it does not apply.
-  int apply_transpose_dots(int idx, int* pre_grid) {
-    *pre_grid = 0;
-    if (!(banded && defer_grad && reortho_full && idx > 0)) return BL_OK;
-    const int j0 = band_lo(idx);
-    const void* few[kFewMax];
-    for (int j = j0; j <= idx; ++j) few[j - j0] = q_row(j);
-    return launch_spmv_dots<T>(op, dtype, true, n, ld, lam_row(idx), nullptr, nullptr, z, idx + 1 - j0, few, -1, c,
-                               op->apply_transpose_bytes(dtype), s, pre_grid);
-  }
   void stepped(int idx) {  // the step kernel of idx also did pre(idx - 1)
     pre_done = idx - 1;
     have_reproj = false;
   }
-  bool skip_step = false;  // the batch driver already tried the step kernel for this step
-  // pre_grid > 0: A^T lambda came from k_op_dots, which left the dots with rows idx-2..idx as per-block shares
-  int post(int idx, int pre_grid = 0) {
+  int post(int idx) {
     T* Lrow = Lambda + (int64_t)idx * ld;
-    if (!skip_step && pre_grid == 0) {
-      std::vector<StepItem> items(1);
-      if (step_item(idx, items[0])) {
-        bool done = false;
-        BL_CHECK(launch_step<T>(items, s, &done));
-        if (done) {
-          stepped(idx);
-          return BL_OK;
-        }
-      }
-    }
     Epi epi_g;  // Gamma[idx, :] and the coefficients of the back-substitution      arnoldi.py:212-218
     epi_g.mode = EPI_ADJ_GAMMA;
     epi_g.i = idx;
@@ -1631,7 +1286,8 @@ struct AdjRun {
     epi_g.coef2 = c.coefC;
     // lambda = (Pi_xi[idx] + Q gamma_row - alpha lambda + A^T lambda - Lambda beta_plus) / beta_minus
     have_reproj = false;
-    auto back_substitution_xdots = [&](bool with_pre) {
+    BL_CHECK(launch_dots<T>(g, c, rows(Q, ld, epi_g.j0, epi_g.m), z, n, epi_g, s));
+    if (banded && idx > 0) {
       // banded Gamma: the back-substitution combines nine vectors at most, and the NEXT step's re-projection dots
       // t = P lambda stream rows 0..idx once                                    arnoldi.py:202,217-219
       XDotsSpec f;
@@ -1650,18 +1306,7 @@ struct AdjRun {
       f.epi.m = idx + 1;
       f.epi.dH = dH;
       f.epi.coef = c.coefA;
-      if (with_pre) {
-        f.pre_partials = c.partials_few;
-        f.pre_count = epi_g.m;
-        f.pre_grid = pre_grid;
-        f.pre_epi = epi_g;
-      }
-      return launch_xdots<T>(c, f, s, &have_reproj);
-    };
-    if (pre_grid > 0 && banded && idx > 0) BL_CHECK(back_substitution_xdots(true));
-    if (!have_reproj) {
-      BL_CHECK(launch_dots<T>(g, c, rows(Q, ld, epi_g.j0, epi_g.m), z, n, epi_g, s));
-      if (banded && idx > 0) BL_CHECK(back_substitution_xdots(false));
+      BL_CHECK(launch_xdots<T>(c, f, s, &have_reproj));
     }
     if (!have_reproj && reortho_full && idx > 0) {
       // ... fused with the NEXT step's re-projection dots t = P lambda (rows 0..idx of Q are the
@@ -1735,36 +1380,8 @@ int arnoldi_adjoint_t(bl_operator_t* op, int dtype, int64_t n, int K, int flags,
   run.symmetric = symmetric_shortcut(flags);
   run.tridiag_cot = (flags & BL_ADJ_TRIDIAG_COTANGENT) != 0;
   BL_CHECK(run.begin());
-  StepOp sop;
-  const bool fuse = run.banded && run.defer_grad && make_step_op(op, dtype, true, false, n, ld, &sop);
   for (int idx = K - 1; idx >= 0; --idx) {
     BL_CHECK(run.pre(idx));
-    if (fuse) {  // A^T lambda + back-substitution + the next re-projection in one launch
-      std::vector<StepItem> items(1);
-      sop.wait_first = idx == K - 1;
-      if (run.fused_item(idx, &sop, items[0])) {
-        bool done = false;
-        BL_CHECK(launch_step<T>(items, s, &done));
-        if (done) {
-          run.stepped(idx);
-          continue;
-        }
-        int pre_grid = 0;  // one run alone: A^T lambda + block-local dots as one plain launch
-        BL_CHECK(launch_op_dots<T>(items, op->apply_transpose_bytes(dtype), s, &done, &pre_grid));
-        if (done) {
-          BL_CHECK(run.post(idx, pre_grid));
-          continue;
-        }
-      }
-    }
-    {  // one run alone: A^T lambda + shares of its dots with rows idx-2..idx in one plain launch
-      int pre_grid = 0;
-      BL_CHECK(run.apply_transpose_dots(idx, &pre_grid));
-      if (pre_grid > 0) {
-        BL_CHECK(run.post(idx, pre_grid));
-        continue;
-      }
-    }
     // (A^T lambda, dparams += ...) = vjp of matvec at (q_idx, params)            arnoldi.py:207-209
     {
       ProfScope prof(BL_PROF_VJP, run.defer_grad ? op->apply_transpose_bytes(dtype) : op->vjp_bytes(dtype), s);
@@ -1846,10 +1463,7 @@ int arnoldi_adjoint_batch_t(bl_operator_t* op, int dtype, int64_t n, int K, int 
         continue;
       }
     }
-    for (int p = 0; p < P; ++p) {
-      runs[p].skip_step = P > 1;
-      BL_CHECK(runs[p].post(idx));
-    }
+    for (int p = 0; p < P; ++p) BL_CHECK(runs[p].post(idx));
   }
   if (deferred) {
     ProfScope prof(BL_PROF_VJP, op->vjp_batch_bytes(dtype, P * K), s);
@@ -2018,7 +1632,7 @@ int bl_dist_set_reduce_hook(bl_allreduce_cb hook, void* user) {
 
 size_t bl_arnoldi_workspace_bytes(int64_t n, int64_t K, int dtype) {
   const size_t ld = align_up((size_t)n, 64);
-  size_t b = common_bytes(n, K);
+  size_t b = common_bytes(K);
   b += align_up((size_t)K * 8, 256);
   b += 3 * align_up((size_t)K * K * 8, 256);
   const int64_t gram_parts = gram_parts_for(n, K);
@@ -2149,7 +1763,7 @@ int bl_op_deferred_grad(bl_operator_t* op, int dtype, int* yes) {
 
 size_t bl_lanczos3_workspace_bytes(int64_t n, int64_t K, int dtype) {
   const size_t ld = align_up((size_t)n, 64);
-  return common_bytes(n, K) + 4 * align_up((ld + 64) * dtype_size(dtype), 256) + 16 * 256;
+  return common_bytes(K) + 4 * align_up((ld + 64) * dtype_size(dtype), 256) + 16 * 256;
 }
 
 int bl_lanczos3_forward(bl_operator_t* op, int dtype, int64_t n, int64_t K, const void* v, void* xs,
@@ -2188,7 +1802,7 @@ int bl_lanczos3_adjoint(bl_operator_t* op, int dtype, int64_t n, int64_t K, cons
 }
 
 // ---- small vector helpers ---------------------------------------------------------------
-size_t bl_vec_workspace_bytes(void) { return common_bytes(0, 1024) + 16 * 256; }
+size_t bl_vec_workspace_bytes(void) { return common_bytes(1024) + 16 * 256; }
 
 }  // extern "C"
 

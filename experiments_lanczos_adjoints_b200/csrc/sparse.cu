@@ -130,61 +130,13 @@ __device__ __forceinline__ double ld_stream_t(const double* p) {
   return v;
 }
 
-// y[r] = sum_k val[slot] * x[col[slot]]; one warp per slice, lane = row within the slice.
-template <typename T>
-__global__ void __launch_bounds__(256)
-k_sell_spmv(int64_t nrows, const int64_t* __restrict__ slice_ptr, const int32_t* __restrict__ col,
-            const T* __restrict__ val, const T* __restrict__ x, T* __restrict__ y) {
-  const int lane = threadIdx.x & 31;
-  const int64_t slice = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int64_t r = slice * kSlice + lane;
-  if (slice * kSlice >= nrows) return;
-  const int64_t s0 = slice_ptr[slice], s1 = slice_ptr[slice + 1];
-  T acc0 = T(0), acc1 = T(0);
-  int64_t p = s0 + lane;
-  for (; p + kSlice < s1; p += 2 * kSlice) {
-    const int c0 = ld_stream_i32(col + p), c1 = ld_stream_i32(col + p + kSlice);
-    const T v0 = ld_stream_t(val + p), v1 = ld_stream_t(val + p + kSlice);
-    acc0 = fma(v0, __ldg(x + c0), acc0);
-    acc1 = fma(v1, __ldg(x + c1), acc1);
-  }
-  if (p < s1) acc0 = fma(ld_stream_t(val + p), __ldg(x + ld_stream_i32(col + p)), acc0);
-  if (r < nrows) y[r] = acc0 + acc1;
-}
-
-// The forward Krylov step's normalisation fused into the matvec: q = v / len (true division as in
-// arnoldi.py:80, written once per row, zero padded up to n_pad) and y = A q, one pass over the vector
-// less.  The gathered entries are scaled with the reciprocal (a division per non-zero makes the kernel
-// ALU-bound): they can differ from the stored q by one ulp, the size of the matvec's own rounding.
-template <typename T>
-__global__ void __launch_bounds__(256)
-k_sell_spmv_normalised(int64_t nrows, const int64_t* __restrict__ slice_ptr, const int32_t* __restrict__ col,
-                       const T* __restrict__ val, const T* __restrict__ v, const double* __restrict__ len,
-                       T* __restrict__ q_out, int64_t n_pad, T* __restrict__ y) {
-  const int lane = threadIdx.x & 31;
-  const int64_t slice = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int64_t r = slice * kSlice + lane;
-  if (slice * kSlice >= nrows) return;
-  const T d = static_cast<T>(*len);
-  const T inv = T(1) / d;
-  if (r < n_pad) q_out[r] = r < nrows ? v[r] * T(1) / d : T(0);
-  const int64_t s0 = slice_ptr[slice], s1 = slice_ptr[slice + 1];
-  T acc0 = T(0), acc1 = T(0);
-  int64_t p = s0 + lane;
-  for (; p + kSlice < s1; p += 2 * kSlice) {
-    const int c0 = ld_stream_i32(col + p), c1 = ld_stream_i32(col + p + kSlice);
-    const T v0 = ld_stream_t(val + p), v1 = ld_stream_t(val + p + kSlice);
-    acc0 = fma(v0, __ldg(v + c0) * inv, acc0);
-    acc1 = fma(v1, __ldg(v + c1) * inv, acc1);
-  }
-  if (p < s1) acc0 = fma(ld_stream_t(val + p), __ldg(v + ld_stream_i32(col + p)) * inv, acc0);
-  if (r < nrows) y[r] = acc0 + acc1;
-}
-
 // Up to kSpmvBatch vectors per launch (lockstep Krylov runs over probes / initial conditions): the slice's values
 // and column indices -- 8 of the ~9 bytes per non-zero a single-vector SpMV moves -- are read ONCE for all of them;
-// the gathers of the P vectors are independent loads in flight together.  NORM: the forward step's fused
-// normalisation, as k_sell_spmv_normalised, with one length per run.
+// the gathers of the P vectors are independent loads in flight together.  A single vector is a batch of one.
+// NORM: the forward Krylov step's normalisation fused into the matvec, one length per run: q = v / len (true division
+// as in arnoldi.py:80, written once per row, zero padded up to n_pad) and y = A q, one pass over the vector less.  The
+// gathered entries are scaled with the reciprocal (a division per non-zero makes the kernel ALU-bound): they can
+// differ from the stored q by one ulp, the size of the matvec's own rounding.
 constexpr int kSpmvBatch = 4;
 struct MultiVec {
   const void* x[kSpmvBatch];
@@ -194,7 +146,7 @@ struct MultiVec {
 };
 
 // W slots of the row are in flight per lane: their column indices and values are loaded first, then all W x P
-// gathers are issued before the first FMA.  (The two-slots-per-iteration loop of k_sell_spmv leaves a lane with two
+// gathers are issued before the first FMA.  (A loop over two slots per iteration leaves a lane with two
 // dependent memory round trips per pair of entries: ~6 round trips for an 11-entry row, and the kernel runs at half
 // of the HBM rate for want of loads in flight.)
 template <typename T, int P, bool NORM, int W>
@@ -605,28 +557,11 @@ struct SparseOperator : bl_operator {
                            : set_params_t<double>(static_cast<const double*>(params[0]), s);
   }
 
-  static bool wide_spmv() {
-    static const bool on = [] {
-      const char* e = std::getenv("BL_SPMV_WIDE");
-      return !(e && e[0] == '0');
-    }();
-    return on;
-  }
   template <typename T>
   int matvec_t(const T* x, T* y, cudaStream_t s) {
-    if (wide_spmv()) {
-      const void* in[1] = {x};
-      void* out[1] = {y};
-      return spmv_multi_t<T, false>(sell, n_rows, 1, in, nullptr, nullptr, 0, out, s);
-    }
-    const int64_t threads = sell.nslices * kSlice;
-    const int blocks = (int)((threads + 255) / 256);
-    if (blocks > 0) {
-      k_sell_spmv<T><<<blocks, 256, 0, s>>>(n_rows, sell.slice_ptr.as<int64_t>(), sell.col.as<int32_t>(),
-                                            sell.val.as<T>(), x, y);
-      BL_LAUNCHED();
-    }
-    return BL_OK;
+    const void* in[1] = {x};
+    void* out[1] = {y};
+    return spmv_multi_t<T, false>(sell, n_rows, 1, in, nullptr, nullptr, 0, out, s);
   }
 
   int matvec(int dtype, const void* x, void* y, cudaStream_t s) override {
@@ -637,19 +572,11 @@ struct SparseOperator : bl_operator {
 
   template <typename T>
   int matvec_normalised_t(const T* v, const double* len, T* q_out, int64_t n_pad, T* y, cudaStream_t s) {
-    if (wide_spmv()) {
-      const void* in[1] = {v};
-      const double* lens[1] = {len};
-      void* q[1] = {q_out};
-      void* out[1] = {y};
-      return spmv_multi_t<T, true>(sell, n_rows, 1, in, lens, q, n_pad, out, s);
-    }
-    const int64_t threads = sell.nslices * kSlice;
-    const int blocks = (int)((threads + 255) / 256);
-    k_sell_spmv_normalised<T><<<blocks, 256, 0, s>>>(n_rows, sell.slice_ptr.as<int64_t>(), sell.col.as<int32_t>(),
-                                                     sell.val.as<T>(), v, len, q_out, n_pad, y);
-    BL_LAUNCHED();
-    return BL_OK;
+    const void* in[1] = {v};
+    const double* lens[1] = {len};
+    void* q[1] = {q_out};
+    void* out[1] = {y};
+    return spmv_multi_t<T, true>(sell, n_rows, 1, in, lens, q, n_pad, out, s);
   }
   int matvec_normalised(int dtype, const void* v, const double* len, void* q_out, int64_t n_pad, void* y,
                         cudaStream_t s) override {
@@ -682,24 +609,11 @@ struct SparseOperator : bl_operator {
       const int64_t* sp = m.slice_ptr.as<int64_t>();
       const int32_t* cl = m.col.as<int32_t>();
       const T* vl = m.val.as<T>();
-      static const int wide = [] {  // BL_SPMV_W=12: the whole row of an 11-entry-per-row operand in one chunk (P <= 2)
-        const char* e = std::getenv("BL_SPMV_W");
-        return e ? std::atoi(e) : 0;
-      }();
       switch (P) {
-        case 1:
-          if (wide == 12) k_sell_spmv_multi<T, 1, NORM, 12><<<blocks, 256, 0, s>>>(rows, sp, cl, vl, mv, n_pad);
-          else k_sell_spmv_multi<T, 1, NORM, 6><<<blocks, 256, 0, s>>>(rows, sp, cl, vl, mv, n_pad);
-          break;
-        case 2:
-          if (wide == 12) k_sell_spmv_multi<T, 2, NORM, 12><<<blocks, 256, 0, s>>>(rows, sp, cl, vl, mv, n_pad);
-          else k_sell_spmv_multi<T, 2, NORM, 6><<<blocks, 256, 0, s>>>(rows, sp, cl, vl, mv, n_pad);
-          break;
+        case 1: k_sell_spmv_multi<T, 1, NORM, 6><<<blocks, 256, 0, s>>>(rows, sp, cl, vl, mv, n_pad); break;
+        case 2: k_sell_spmv_multi<T, 2, NORM, 6><<<blocks, 256, 0, s>>>(rows, sp, cl, vl, mv, n_pad); break;
         case 3: k_sell_spmv_multi<T, 3, NORM, 4><<<blocks, 256, 0, s>>>(rows, sp, cl, vl, mv, n_pad); break;
-        default:
-          if (wide == 6 || wide == 12) k_sell_spmv_multi<T, 4, NORM, 6><<<blocks, 256, 0, s>>>(rows, sp, cl, vl, mv, n_pad);
-          else k_sell_spmv_multi<T, 4, NORM, 4><<<blocks, 256, 0, s>>>(rows, sp, cl, vl, mv, n_pad);
-          break;
+        default: k_sell_spmv_multi<T, 4, NORM, 4><<<blocks, 256, 0, s>>>(rows, sp, cl, vl, mv, n_pad); break;
       }
       BL_LAUNCHED();
     }
@@ -749,14 +663,8 @@ struct SparseOperator : bl_operator {
 
   // Deferred cotangent (square operands): inside the adjoint loop only z = A^T lam (an SpMV with the SELL of
   // A^T: 92 MB per step instead of the 175 MB of the matvec-VJP at C2), then one batched pass over the K
-  // (lambda, q) pairs.  BL_SPARSE_DEFER=0 keeps the per-step cotangent.
-  bool deferred_grad(int dtype) const override {
-    static const bool enabled = [] {
-      const char* e = std::getenv("BL_SPARSE_DEFER");
-      return !(e && e[0] == '0');
-    }();
-    return enabled && dtype == bound_dtype && n_rows == n_cols && n_rows > 0;
-  }
+  // (lambda, q) pairs.
+  bool deferred_grad(int dtype) const override { return dtype == bound_dtype && n_rows == n_cols && n_rows > 0; }
   double apply_transpose_bytes(int dtype) const override { return matvec_bytes(dtype); }
   double vjp_batch_bytes(int dtype, int count) const override {  // Q and Lambda once, col, grad read + write
     const double w = dtype == BL_F32 ? 4 : 8;
@@ -764,19 +672,9 @@ struct SparseOperator : bl_operator {
   }
   template <typename T>
   int apply_transpose_t(const T* lam, T* z, cudaStream_t s) {
-    if (wide_spmv()) {
-      const void* in[1] = {lam};
-      void* out[1] = {z};
-      return spmv_multi_t<T, false>(sell_t, n_cols, 1, in, nullptr, nullptr, 0, out, s);
-    }
-    const int64_t threads = sell_t.nslices * kSlice;
-    const int blocks = (int)((threads + 255) / 256);
-    if (blocks > 0) {
-      k_sell_spmv<T><<<blocks, 256, 0, s>>>(n_cols, sell_t.slice_ptr.as<int64_t>(), sell_t.col.as<int32_t>(),
-                                            sell_t.val.as<T>(), lam, z);
-      BL_LAUNCHED();
-    }
-    return BL_OK;
+    const void* in[1] = {lam};
+    void* out[1] = {z};
+    return spmv_multi_t<T, false>(sell_t, n_cols, 1, in, nullptr, nullptr, 0, out, s);
   }
   int apply_transpose(int dtype, const void* lam, void* z, cudaStream_t s) override {
     BL_REQUIRE(dtype == bound_dtype, "set_params must be called with the same dtype first");
@@ -816,20 +714,10 @@ struct SparseOperator : bl_operator {
     const int64_t threads = sell.nslices * kSlice;
     const int blocks = (int)((threads + 255) / 256);
     if (blocks > 0 && count > 0) {
-      static const int rounds = [] {  // BL_GRAD_U: pairs per round of k_sell_grad_batch (1, 2 or 4)
-        const char* e = std::getenv("BL_GRAD_U");
-        return e ? std::atoi(e) : (sizeof(T) == 8 ? 4 : 2);  // fp64: 6.57 -> 4.0 (2) -> 2.63 ms (4) for 400 pairs at C2
-      }();
-      auto launch = [&](auto kern) {
-        kern<<<blocks, 256, 0, s>>>(n_rows, sell.slice_ptr.as<int64_t>(), sell.col.as<int32_t>(), grad.as<T>(), Q, ldq, Lam,
-                                    ldl, count);
-      };
-      if (rounds >= 4)
-        launch(k_sell_grad_batch<T, 12, 4>);
-      else if (rounds == 2)
-        launch(k_sell_grad_batch<T, 12, 2>);
-      else
-        launch(k_sell_grad_batch<T, 12, 1>);
+      // pairs per round: fp64 6.57 (1) -> 4.0 (2) -> 2.63 ms (4) for 400 pairs at C2
+      constexpr int U = sizeof(T) == 8 ? 4 : 2;
+      k_sell_grad_batch<T, 12, U><<<blocks, 256, 0, s>>>(n_rows, sell.slice_ptr.as<int64_t>(), sell.col.as<int32_t>(),
+                                                         grad.as<T>(), Q, ldq, Lam, ldl, count);
       BL_LAUNCHED();
     }
     return BL_OK;

@@ -50,8 +50,6 @@ struct StepOp {  // the step's operator call, shared by the runs of a launch (ph
   long long n_pad = 0;  // norm: op_q is written up to n_pad entries (zero padding beyond nrows)
   int norm = 0;         // forward step: q = op_x / *op_len (true division, arnoldi.py:80-81), few_x = A q
   int wait_first = 0;   // the operand's values may be the predecessor's output: dependency wait before the first copy
-  int l2_hints = 0;     // bit 0: basis rows are copied with L2 evict_first, bit 1: the operand with evict_last
-  int depth = 8;        // fine stages of phase S's ring in use (<= kOpStages): what the producer keeps in flight
 };
 
 struct StepArgs {
@@ -256,7 +254,8 @@ __device__ __forceinline__ void grid_reduce(const StepBatch& B, double* acc_base
 // of their own and the ring holds twice as many slices.
 constexpr int kOpStageBytes = 8192;
 constexpr int kOpStages = kStages * kGroup * kConsumerThreads * 16 / kOpStageBytes;  // the ring: 96 KB = 12 fine stages
-constexpr int kOpHold = kOpStages / 2 - 1;  // stages a warp may span with the slices it has in flight
+constexpr int kOpDepth = 8;                  // fine stages in use: what the producer keeps in flight
+constexpr int kOpHold = kOpDepth / 2 - 1;    // stages a warp may span with the slices it has in flight
 constexpr int kOpRing = kOpStages * kOpStageBytes / 4;  // slots in the ring
 // The head of the stage in ring slot 0 is copied a second time behind the ring's end (into the x-tile buffer), so a
 // chunk of up to kOpOverflow slots that starts in the last ring slot reads on linearly instead of wrapping.
@@ -304,8 +303,8 @@ __device__ __forceinline__ OpRange op_range(const StepOp& op, const ColumnRange&
 
 // Loads of what a PREDECESSOR kernel wrote (x here, the vectors of phase 0) go through L2 (`ld.global.cg`): in a chain of
 // programmatic dependent launches this kernel's lifetime overlaps the predecessor's, which is outside what `ld.global.nc`
-// promises, and L1 buys nothing measurable here (BL_STEP_L2 bit 6 switches the gathers back to `ld.global.nc`: 5558 vs
-// 5532 Krylov steps/s, within the noise).
+// promises, and L1 buys nothing measurable here (gathers through `ld.global.nc` measured 5558 vs 5532 Krylov steps/s,
+// within the noise).
 // Consumer side: warp w takes the block's slices w, w + 8, ...; lane = row within the slice.  Summation order as in
 // k_sell_spmv_multi (entries k of even / odd position in two accumulators, added at the end): bit-identical results.
 // U slices of the warp are in flight together (their W x P gathers each are issued before the first FMA): with 16
@@ -328,13 +327,13 @@ __device__ __forceinline__ void op_phase(const StepBatch& B, const OpRange& o, c
   }
   const T* valp = static_cast<const T*>(op.val) + o.a0 + lane;  // this lane's values of the block's slots
   const int* colp = reinterpret_cast<const int*>(stages_raw) + lane;
-  const int depth = op.depth, ring_slots = op.depth * SLOTS, hold = op.depth / 2 - 1;
+  constexpr int ring_slots = kOpDepth * SLOTS;
   int lo = 0, hi = -1;  // stages [lo, hi] of the operand stream are held by this warp
   int hi_ring = -1, lo_ring = 0, hi_par = 0;
   auto need = [&](int st) {
     while (hi < st) {
       ++hi;
-      if (++hi_ring == depth) {
+      if (++hi_ring == kOpDepth) {
         hi_ring = 0;
         hi_par ^= hi > 0;
       }
@@ -347,12 +346,11 @@ __device__ __forceinline__ void op_phase(const StepBatch& B, const OpRange& o, c
       __syncwarp();
       if (lane == 0) tma::mbar_arrive(empty + lo_ring);
       ++lo;
-      lo_ring = lo_ring + 1 == depth ? 0 : lo_ring + 1;
+      lo_ring = lo_ring + 1 == kOpDepth ? 0 : lo_ring + 1;
     }
   };
   const long long first = o.s_lo + warp;
-  int nmine = o.s_hi > first ? (int)((o.s_hi - first + kConsumerWarps - 1) / kConsumerWarps) : 0;
-  if (op.l2_hints & 256) nmine = 0;  // timing experiment: the ring's protocol alone (every warp passes every stage)
+  const int nmine = o.s_hi > first ? (int)((o.s_hi - first + kConsumerWarps - 1) / kConsumerWarps) : 0;
   BL_CYC_DECL
   for (int base = 0; base < nmine; base += 32) {
     // lane l fetches the slot range of the warp's (base + l)-th slice (relative to the block's first slot: 32 bits)
@@ -377,7 +375,7 @@ __device__ __forceinline__ void op_phase(const StepBatch& B, const OpRange& o, c
           const int a = __shfl_sync(0xffffffffu, sp0, (i + u) & 31), b = __shfl_sync(0xffffffffu, sp1, (i + u) & 31);
           const int last = b - 32 > a ? b - 32 : a;  // last slot row of the slice
           if (u == 0) head_st = a / SLOTS;
-          if (u == 0 || (nu == u && last / SLOTS - head_st <= hold)) {
+          if (u == 0 || (nu == u && last / SLOTS - head_st <= kOpHold)) {
             rel[u] = a;
             width[u] = (b - a) / 32;
             r[u] = (first + (long long)(base + i + u) * kConsumerWarps) * 32 + lane;
@@ -425,7 +423,7 @@ __device__ __forceinline__ void op_phase(const StepBatch& B, const OpRange& o, c
             v[u][j] = T(0);
             if (j < rows[u]) {
               c[u][j] = cs[j * 32];
-              v[u][j] = (op.l2_hints & 32) ? T(1) : ld_stream(vs + j * 32);
+              v[u][j] = ld_stream(vs + j * 32);
             }
           }
         }
@@ -446,7 +444,7 @@ __device__ __forceinline__ void op_phase(const StepBatch& B, const OpRange& o, c
           for (int j = 0; j < W; ++j)
 #pragma unroll
             for (int p = 0; p < P; ++p) {  // through L2 (see the note above)
-              g[u][j][p] = (op.l2_hints & 16) ? T(c[u][j]) : ((op.l2_hints & 64) ? __ldg(x[p] + c[u][j]) : __ldcg(x[p] + c[u][j]));
+              g[u][j][p] = __ldcg(x[p] + c[u][j]);
               BL_DBG(dbg_bad(g[u][j][p]), 2, p, B.a[p].epi0.i, c[u][j], (double)g[u][j][p], (double)inv[p]);
             }
 #pragma unroll
@@ -636,8 +634,7 @@ k_step_tma(const __grid_constant__ StepBatch B) {
 
   if (warp == kConsumerWarps) {
     if (lane == 0) {  // ---- producer: the rows of phase 1 of every run, then the rows of phase 2, one ring ----
-      const uint64_t pol_first = tma::policy_evict_first(), pol_last = tma::policy_evict_last();
-      const bool rows_first = (B.op.l2_hints & 1) != 0;
+      const uint64_t pol_first = tma::policy_evict_first();
       bool waited = false;
       bool gated = !with_op;  // with the operator in the launch the ring belongs to phase S first
       int it = 0;
@@ -647,7 +644,6 @@ k_step_tma(const __grid_constant__ StepBatch B) {
           tma::griddep_wait();
           waited = true;
         }
-        const int depth = B.op.depth;
         for (int k = 0, s = 0, par = 1; k < orng.nstages; ++k) {
           const long long pos = orng.a0 + (long long)k * SLOTS;
           const uint32_t cnt = (uint32_t)((orng.a1 - pos) < SLOTS ? (orng.a1 - pos) : SLOTS);
@@ -655,17 +651,10 @@ k_step_tma(const __grid_constant__ StepBatch B) {
           const uint32_t over = s == 0 && k > 0 ? (cnt < (uint32_t)step::kOpOverflow ? cnt : (uint32_t)step::kOpOverflow) : 0u;
           tma::mbar_arrive_expect_tx(op_full + s, (cnt + over) * 4u);
           unsigned char* dst = smem_raw + (size_t)s * step::kOpStageBytes;
-          if (B.op.l2_hints & 2)
-            tma::bulk_g2s_hint(dst, B.op.col + pos, cnt * 4u, op_full + s, pol_last);
-          else
-            tma::bulk_g2s(dst, B.op.col + pos, cnt * 4u, op_full + s);
+          tma::bulk_g2s(dst, B.op.col + pos, cnt * 4u, op_full + s);
           if (over)  // the ring's end reads on linearly
-            tma::bulk_g2s(smem_raw + (size_t)depth * step::kOpStageBytes, B.op.col + pos, over * 4u, op_full + s);
-          if (B.op.l2_hints & 4)  // the values of these slots: on their way into L2 when the consumers load them
-            asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(static_cast<const T*>(B.op.val) + pos),
-                         "r"(cnt * (uint32_t)sizeof(T))
-                         : "memory");
-          if (++s == depth) {
+            tma::bulk_g2s(smem_raw + (size_t)step::kOpDepth * step::kOpStageBytes, B.op.col + pos, over * 4u, op_full + s);
+          if (++s == step::kOpDepth) {
             s = 0;
             par ^= 1;
           }
@@ -699,15 +688,9 @@ k_step_tma(const __grid_constant__ StepBatch B) {
               tma::mbar_wait(empty + s, ((it / kStages) & 1) ^ 1);
               tma::mbar_arrive_expect_tx(full + s, bytes * rows_here);
               T* dst = stages + (size_t)s * kGroup * TILE;
-              if (rows_first) {
-                for (int r = 0; r < rows_here; ++r)
-                  tma::bulk_g2s_hint(dst + (size_t)r * TILE, src.row(g * kGroup + r) + tc0 * (long long)sizeof(T), bytes,
-                                     full + s, pol_first);
-              } else {
-                for (int r = 0; r < rows_here; ++r)
-                  tma::bulk_g2s(dst + (size_t)r * TILE, src.row(g * kGroup + r) + tc0 * (long long)sizeof(T), bytes,
-                                full + s);
-              }
+              for (int r = 0; r < rows_here; ++r)
+                tma::bulk_g2s_hint(dst + (size_t)r * TILE, src.row(g * kGroup + r) + tc0 * (long long)sizeof(T), bytes,
+                                   full + s, pol_first);
             }
           }
         }
@@ -727,7 +710,6 @@ k_step_tma(const __grid_constant__ StepBatch B) {
         step::op_phase_dispatch<T, true>(B, orng, smem_raw, op_full, op_empty, warp, lane);
       else
         step::op_phase_dispatch<T, false>(B, orng, smem_raw, op_full, op_empty, warp, lane);
-      if (B.trace_slot >= 0 && (B.op.l2_hints & 8)) step::stamp(B.trace_slot, 2, tid);  // debugging: S alone
       // the producer copies this block's columns of the rows written above (generic -> async proxy), the dots
       // below read them back
       asm volatile("fence.proxy.async;" ::: "memory");
@@ -740,7 +722,7 @@ k_step_tma(const __grid_constant__ StepBatch B) {
     for (int p = 0; p < P; ++p) any_few = any_few || B.a[p].few_n > 0;
     if (any_few) {
       step::few_dots_local<T, TILE>(B, cr, n, acc_s, tid, warp, lane, csync);
-      if (!(with_op && (B.op.l2_hints & 8))) step::stamp(B.trace_slot, 2, tid);
+      step::stamp(B.trace_slot, 2, tid);
       step::grid_reduce<0>(B, acc_s, kFewMax * kConsumerWarps, tid);
       for (int p = 0; p < P; ++p) {
         if (B.a[p].few_n <= 0) continue;
@@ -756,8 +738,8 @@ k_step_tma(const __grid_constant__ StepBatch B) {
       csync();
       step::stamp(B.trace_slot, 3, tid);
     }
-    // every block is past phase S (phase 0's barrier); BL_STEP_L2 bit 7: no early trigger (debugging)
-    if (with_op && !(B.op.l2_hints & 128)) tma::griddep_launch_dependents();
+    // every block is past phase S (phase 0's barrier)
+    if (with_op) tma::griddep_launch_dependents();
 
     // ================= phase 1: out1 = (sum of terms) / div, red1[j] = <row_j, out1>, every run =================
     int it = it0, xt = 0;
@@ -1014,67 +996,6 @@ k_step_tma(const __grid_constant__ StepBatch B) {
     run_epilogue<T>(B.a[p].epi2);
     __syncthreads();
   }
-}
-
-// The operator call of ONE run's step together with the block-local part of the neighbouring-row dots, as a PLAIN
-// launch (the separate streaming kernels that follow prefetch basis rows before their dependency wait: the newest row
-// must be complete when they are scheduled).  Phase S as in k_step_tma; the block's shares of <few_j, A x> go to
-// partials[j * gridDim.x + block] and the NEXT kernel (k_xdots_tma, XDotsArgs::pre_*) adds them up in every block and
-// runs the epilogue itself -- no k_dots_few launch, no last-block pass, no grid barrier.
-template <typename T, int TILE>
-__global__ void __launch_bounds__(kStreamThreads, 2)
-k_op_dots(const __grid_constant__ StepBatch B) {
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  T* stages = reinterpret_cast<T*>(smem_raw);
-  T* xs = stages + (size_t)kStages * kGroup * TILE;
-  uint64_t* op_full = reinterpret_cast<uint64_t*>(xs + 2 * TILE) + 2 * kStages + 2;  // the layout of k_step_tma
-  uint64_t* op_empty = op_full + step::kOpStages;
-  double* acc_s = reinterpret_cast<double*>(op_empty + step::kOpStages);
-  const long long n = B.a[0].n;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < step::kOpStages; ++s) {
-      tma::mbar_init(op_full + s, 1);
-      tma::mbar_init(op_empty + s, kConsumerWarps);
-    }
-    tma::fence_barrier_init();
-  }
-  for (int j = threadIdx.x; j < B.count * B.acc_stride; j += blockDim.x) acc_s[j] = 0.0;
-  __syncthreads();
-  const ColumnRange cr = block_columns<T>(n, TILE);
-  const step::OpRange orng = step::op_range<T>(B.op, cr, n);
-  if (warp == kConsumerWarps) {
-    if (lane == 0 && orng.nstages > 0) {
-      constexpr int SLOTS = step::op_stage_slots<T>();
-      const int depth = B.op.depth;
-      for (int k = 0, s = 0, par = 1; k < orng.nstages; ++k) {
-        const long long pos = orng.a0 + (long long)k * SLOTS;
-        const uint32_t cnt = (uint32_t)((orng.a1 - pos) < SLOTS ? (orng.a1 - pos) : SLOTS);
-        tma::mbar_wait(op_empty + s, par);
-        const uint32_t over = s == 0 && k > 0 ? (cnt < (uint32_t)step::kOpOverflow ? cnt : (uint32_t)step::kOpOverflow) : 0u;
-        tma::mbar_arrive_expect_tx(op_full + s, (cnt + over) * 4u);
-        tma::bulk_g2s(smem_raw + (size_t)s * step::kOpStageBytes, B.op.col + pos, cnt * 4u, op_full + s);
-        if (over) tma::bulk_g2s(smem_raw + (size_t)depth * step::kOpStageBytes, B.op.col + pos, over * 4u, op_full + s);
-        if (++s == depth) {
-          s = 0;
-          par ^= 1;
-        }
-      }
-    }
-    return;
-  }
-  const int tid = threadIdx.x;
-  step::ConsumerSync csync;
-  if (B.op.norm)
-    step::op_phase_dispatch<T, true>(B, orng, smem_raw, op_full, op_empty, warp, lane);
-  else
-    step::op_phase_dispatch<T, false>(B, orng, smem_raw, op_full, op_empty, warp, lane);
-  csync();  // the rows written above are read back below (same block)
-  step::few_dots_local<T, TILE>(B, cr, n, acc_s, tid, warp, lane, csync);
-  for (int p = 0; p < B.count; ++p)
-    if (tid < B.a[p].few_n)
-      __stcg(B.a[p].partials + (size_t)tid * gridDim.x + blockIdx.x,
-             acc_s[(size_t)p * B.acc_stride + kFewMax * kConsumerWarps + tid]);
 }
 
 }  // namespace bl

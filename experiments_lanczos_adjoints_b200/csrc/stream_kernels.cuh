@@ -28,15 +28,16 @@ constexpr int kStreamThreads = kConsumerThreads + 32;  // + producer warp
 constexpr int kStages = 3;
 constexpr int kBoxesPerBarrier = 4;  // fused kernel: resident boxes ([8 x TILE]) that share one mbarrier
 
-struct RowSource {  // rows [0, n0) from block 0, [n0, n0 + n1) from block 1
+// Rows [0, n0) from block 0, [n0, n0 + n1) from block 1.  The kernels copy them with the L2 evict_first policy: a
+// stream that is larger than L2 does not push the vectors (and the operand) out, which every step reads again
+// (measured +4 % for one run alone).
+struct RowSource {
   const char* base0 = nullptr;
   long long ldb0 = 0;  // bytes
   int n0 = 0;
   const char* base1 = nullptr;
   long long ldb1 = 0;
   int n1 = 0;
-  int evict_first = 0;  // copy the rows with the L2 evict_first policy: a stream that is larger than L2 does not push the
-                        // vectors (and the operand) out, which every step reads again
   __device__ __forceinline__ const char* row(int j) const {
     return j < n0 ? base0 + (long long)j * ldb0 : base1 + (long long)(j - n0) * ldb1;
   }
@@ -182,8 +183,8 @@ k_dots_tma(RowSource src, int nrows, const T* __restrict__ x, long long n, doubl
         tma::mbar_arrive_expect_tx(full + s, bytes * rows_here);
         T* dst = stages + (size_t)s * kGroup * TILE;
         for (int r = 0; r < rows_here; ++r)
-          tma::bulk_g2s_opt(dst + (size_t)r * TILE, src.row(g * kGroup + r) + tc0 * (long long)sizeof(T), bytes, full + s,
-                            src.evict_first);
+          tma::bulk_g2s_hint(dst + (size_t)r * TILE, src.row(g * kGroup + r) + tc0 * (long long)sizeof(T), bytes, full + s,
+                             tma::policy_evict_first());
       }
       if (!waited && total > 0) {
         tma::griddep_wait();
@@ -308,12 +309,6 @@ struct XDotsArgs {
   unsigned int* counter = nullptr;
   Epi epi;
   int reverse = 0;
-  // Optional: the predecessor (k_op_dots) left per-block shares of `pre_count` dot products in
-  // pre_partials[j * pre_grid + block]; every block adds them up in a fixed order and runs `pre_epi` on the sums
-  // (identical numbers, idempotent writes) before it reads the coefficients that epilogue produces.
-  const double* pre_partials = nullptr;
-  int pre_count = 0, pre_grid = 0;
-  Epi pre_epi;
 };
 
 template <typename T, int TILE>
@@ -363,56 +358,13 @@ k_xdots_tma(const __grid_constant__ XDotsArgs a) {
         tma::mbar_arrive_expect_tx(full + s, bytes * rows_here);
         T* dst = stages + (size_t)s * kGroup * TILE;
         for (int r = 0; r < rows_here; ++r)
-          tma::bulk_g2s_opt(dst + (size_t)r * TILE, a.src.row(g * kGroup + r) + tc0 * (long long)sizeof(T), bytes, full + s,
-                            a.src.evict_first);
+          tma::bulk_g2s_hint(dst + (size_t)r * TILE, a.src.row(g * kGroup + r) + tc0 * (long long)sizeof(T), bytes,
+                             full + s, tma::policy_evict_first());
       }
     }
   } else {
     const int tid = threadIdx.x;  // 0..255: column vector tid of every tile
     tma::griddep_wait();          // the terms and their coefficients are the predecessor's output
-    if (a.pre_count > 0) {
-      __shared__ double pre_s[8];
-      if (a.pre_grid <= 320) {
-        if (warp < a.pre_count) {
-          const double sum = step::row_sum(a.pre_partials + (size_t)warp * a.pre_grid, a.pre_grid, lane);
-          if (lane == 0) pre_s[warp] = sum;
-        }
-      } else {
-        // thousands of shares per value (k_sell_spmv_dots: one per SpMV block): all consumer threads add them up,
-        // thread t the shares t, t + 256, ... (eight loads in flight), then lanes, then warps -- a fixed order
-        __shared__ double pre_w[8][kConsumerWarps];
-        for (int j = 0; j < a.pre_count; ++j) {
-          const double* p = a.pre_partials + (size_t)j * a.pre_grid;
-          double s = 0.0;
-          for (int k0 = tid; k0 < a.pre_grid; k0 += 8 * kConsumerThreads) {
-            double v[8];
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-              const int k = k0 + u * kConsumerThreads;
-              v[u] = k < a.pre_grid ? __ldcg(p + k) : 0.0;
-            }
-#pragma unroll
-            for (int u = 0; u < 8; ++u) s += v[u];
-          }
-          s = warp_sum(s);
-          if (lane == 0) pre_w[j][warp] = s;
-        }
-        tma::named_bar_sync(1, kConsumerThreads);
-        if (tid < a.pre_count) {
-          double s = 0.0;
-#pragma unroll
-          for (int w = 0; w < kConsumerWarps; ++w) s += pre_w[tid][w];
-          pre_s[tid] = s;
-        }
-      }
-      tma::named_bar_sync(1, kConsumerThreads);
-      struct PreSync {
-        __device__ __forceinline__ void operator()() const { tma::named_bar_sync(1, kConsumerThreads); }
-      };
-      run_epilogue_impl<T>(a.pre_epi, pre_s, tid, kConsumerThreads, PreSync());
-      __threadfence();  // the coefficients go through global memory (every block writes the same values)
-      tma::named_bar_sync(1, kConsumerThreads);
-    }
     T cv[kXTerms];
 #pragma unroll
     for (int v = 0; v < kXTerms; ++v)
@@ -607,8 +559,8 @@ k_combine_tma(CombineTmaArgs a) {
             const int rows_here = nbasis - g * kGroup < kGroup ? nbasis - g * kGroup : kGroup;
             tma::mbar_arrive_expect_tx(full + s, bytes * rows_here);
             for (int r = 0; r < rows_here; ++r)
-              tma::bulk_g2s_opt(dst + (size_t)r * TILE, a.src.row(g * kGroup + r) + tc0 * (long long)sizeof(T), bytes,
-                                full + s, a.src.evict_first);
+              tma::bulk_g2s_hint(dst + (size_t)r * TILE, a.src.row(g * kGroup + r) + tc0 * (long long)sizeof(T), bytes,
+                                 full + s, tma::policy_evict_first());
           }
         }
       }

@@ -73,19 +73,6 @@ __device__ __forceinline__ uint64_t policy_evict_first() {
   asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
   return p;
 }
-__device__ __forceinline__ uint64_t policy_evict_last() {
-  uint64_t p;
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
-
-// bulk copy with the evict_first policy when `first` is set (streams larger than L2)
-__device__ __forceinline__ void bulk_g2s_opt(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* bar, int first) {
-  if (first)
-    bulk_g2s_hint(dst_smem, src_gmem, bytes, bar, policy_evict_first());
-  else
-    bulk_g2s(dst_smem, src_gmem, bytes, bar);
-}
 
 // 2-D tiled TMA load through a tensor map (`cp.async.bulk.tensor`, SASS UTMALDG): one
 // instruction moves a [box_rows x box_cols] box; elements outside the tensor are zero-filled

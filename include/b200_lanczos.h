@@ -257,8 +257,7 @@ size_t bl_arnoldi_workspace_bytes(int64_t n, int64_t krylov_depth, int dtype);
                               * the first pass (arnoldi.py:87-88) takes h = Q^H v with rows i-1, i only -- the
                               * other entries are O(eps |A|) and H[j < i-1, i] is stored as zero; the second
                               * pass still projects against every row, so Q stays orthonormal to rounding.
-                              * The basis is read twice per step instead of three times.
-                              * BL_SYMMETRIC_FORWARD=0 in the environment ignores the bit. */
+                              * The basis is read twice per step instead of three times. */
 
 /* arnoldi._forward (arnoldi.py:57-101).  second_pass & BL_FWD_SECOND_PASS performs the second
  * Gram-Schmidt pass (`reortho_ != "none"`, arnoldi.py:91; the reference's default always
@@ -273,8 +272,7 @@ int bl_arnoldi_forward(bl_operator_t* op, int dtype, int64_t n, int64_t krylov_d
                                * lanczos.tridiag(reortho="full") guarantees, lanczos.py:152-169): H is
                                * tridiagonal up to rounding, and `Lambda beta_plus` (arnoldi.py:218) keeps
                                * only its O(1) term H[idx, idx+1] Lambda[idx+1].  Results change by
-                               * O(eps K |Lambda|); K^2/2 fewer basis rows are read per sweep.
-                               * BL_SYMMETRIC_ADJOINT=0 in the environment ignores the bit. */
+                               * O(eps K |Lambda|); K^2/2 fewer basis rows are read per sweep. */
 #define BL_ADJ_TRIDIAG_COTANGENT 4 /* with BL_ADJ_SYMMETRIC | BL_ADJ_REORTHO_FULL and dQ == NULL: dH is
                                * tridiagonal (the cotangent of lanczos.tridiag's (alpha, beta), lanczos.py:162-164).
                                * Gamma (arnoldi.py:213) is then banded up to rounding, because the re-projected

@@ -1,5 +1,6 @@
 """Where the time of a k_step_tma launch goes: block 0's time stamps (bl_step_trace_*) over one forward + adjoint
-of the headline workload (n = 1M, depth 100, fp32), summarised per phase."""
+of a lockstep batch of TRACE_PROBES runs (default 4) of the headline workload (n = 1M, depth 100, fp32), summarised
+per phase."""
 import ctypes as C
 import json
 import sys
@@ -15,18 +16,14 @@ row, col, data, dalpha, dbeta = bench.build_workload()
 n, K, dtype = bench.N_ROWS, bench.DEPTH, np.float32
 import os
 
-P = int(os.environ.get("TRACE_PROBES", 1))  # > 1: a lockstep batch (BatchedTridiagAdjointPlan)
+P = int(os.environ.get("TRACE_PROBES", 4))  # runs of the lockstep batch (BatchedTridiagAdjointPlan)
+if P < 2:
+    sys.exit(f"TRACE_PROBES={P}: k_step_tma runs for lockstep batches of two or more runs only")
 op = bl.operators.SparseOperator(row, col, (n, n))
-if P > 1:
-    pl = bl_plan.BatchedTridiagAdjointPlan(op, K, dtype, P)
-    pl.set_vectors(np.random.default_rng(0).standard_normal((P, n)).astype(dtype))
-    pl.set_params(data.astype(dtype))
-    pl.set_cotangents(np.stack([synthetic.slq_cotangent_dH(dalpha, dbeta, dtype)] * P))
-else:
-    pl = bl_plan.TridiagAdjointPlan(op, K, dtype)
-    pl.set_vector(np.random.default_rng(0).standard_normal(n).astype(dtype))
-    pl.set_params(data.astype(dtype))
-    pl.set_cotangent(synthetic.slq_cotangent_dH(dalpha, dbeta, dtype))
+pl = bl_plan.BatchedTridiagAdjointPlan(op, K, dtype, P)
+pl.set_vectors(np.random.default_rng(0).standard_normal((P, n)).astype(dtype))
+pl.set_params(data.astype(dtype))
+pl.set_cotangents(np.stack([synthetic.slq_cotangent_dH(dalpha, dbeta, dtype)] * P))
 for _ in range(3):
     pl.run()
 bl.synchronize()

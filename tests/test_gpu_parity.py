@@ -600,12 +600,6 @@ def test_staged_cotangent_pass_is_bit_identical_to_the_gather_pass():
     assert out.count("bit-identical True") == 4, out
 
 
-def test_operator_call_with_neighbouring_row_dots_matches_the_separate_launches():
-    """`k_sell_spmv_dots` + shares finished by `k_xdots_tma` (one run alone) against `k_dots_few` (BL_SPMV_DOTS=0): fewer
-    launches, H / dv / dparams equal to rounding (fp32 2e-5, fp64 1e-11; the dots are added up in another order)."""
-    _run_check_script("check_spmv_dots.py")
-
-
 @pytest.mark.parametrize("dtype", [np.float32, np.float64])
 def test_two_lockstep_lanes_in_flight_reproduce_their_solo_runs_bit_for_bit(dtype):
     """The bench configuration: two lockstep batches of four runs on two streams, one block per SM and kernel, so a
