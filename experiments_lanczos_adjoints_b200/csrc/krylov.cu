@@ -159,27 +159,6 @@ int sharded_sum(double* values, int count, cudaStream_t s) {
   return BL_OK;
 }
 
-// Peer-memory route: the cross-rank sum rides in the last block of the streaming kernel itself (its
-// epilogue carries the peer view), so a sharded reduction costs no extra launch.  Returns true when the
-// epilogue was armed; the NCCL-hook route still splits the kernel (EPI_NONE + finish_sharded).
-bool arm_peer_epilogue(Epi& epi, int count, int* rc) {
-  *rc = BL_OK;
-  if (!dist::active()) return false;
-  if (count > dist::kRedSlots) {
-    set_error("reduction too large for the peer mailbox");
-    *rc = BL_EINVAL;
-    return true;
-  }
-  dist::PeerView pv;
-  *rc = dist::next_reduce(&pv);
-  if (pv.world > 1) {  // one rank: the local sums are the global sums
-    epi.peer_mail = pv.mail[pv.rank];
-    epi.peer_seq = pv.seq;
-    epi.peer_count = count;
-  }
-  return true;
-}
-
 template <typename T>
 int finish_sharded(const Common& c, Epi epi, int count, cudaStream_t s) {
   epi.red = c.red;
@@ -200,6 +179,48 @@ int finish_sharded(const Common& c, Epi epi, int count, cudaStream_t s) {
   BL_LAUNCHED();
   return BL_OK;
 }
+
+// The epilogue of a streaming kernel's reduction, row sharding included: arm() before the launch, finish() after it.
+// Peer-memory route: the cross-rank sum rides in the last block of the kernel itself (its epilogue carries the peer
+// view), so a sharded reduction costs no extra launch.  All-reduce-hook route: the kernel runs with EPI_NONE and
+// leaves its local sums in red[0..count); finish() runs the hook and then the epilogue as a launch of its own.
+struct ShardedEpi {
+  const Common* c = nullptr;
+  Epi full;  // the epilogue as the caller built it
+  int count = 0;
+  bool split = false;  // hook route: finish() runs `full`
+
+  // Points `epi` at the run's reduction buffers and, under row sharding, arms or splits it for `n` reduced values.
+  int arm(const Common& common, Epi& epi, int n) {
+    c = &common;
+    epi.red = common.red;
+    epi.scal = common.scal;
+    full = epi;
+    count = n;
+    if (!dist::active()) {
+      split = is_sharded();
+      if (split) epi.mode = EPI_NONE;
+      return BL_OK;
+    }
+    if (n > dist::kRedSlots) {
+      set_error("reduction too large for the peer mailbox");
+      return BL_EINVAL;
+    }
+    dist::PeerView pv;
+    const int rc = dist::next_reduce(&pv);
+    if (pv.world > 1) {  // one rank: the local sums are the global sums
+      epi.peer_mail = pv.mail[pv.rank];
+      epi.peer_seq = pv.seq;
+      epi.peer_count = n;
+    }
+    return rc;
+  }
+
+  template <typename T>
+  int finish(cudaStream_t s) const {
+    return split ? finish_sharded<T>(*c, full, count, s) : BL_OK;
+  }
+};
 
 // L2 "snake" order: consecutive streaming kernels walk the basis in
 // opposite directions, so a kernel starts on the tiles its predecessor read last — the part of
@@ -257,14 +278,8 @@ RowSource row_source(const RowBlock& b0, const RowBlock* b1, size_t w) {
 
 template <typename T>
 int launch_dots(const Grid& g, const Common& c, RowBlock blk, const T* x, int64_t n, Epi epi, cudaStream_t s) {
-  epi.red = c.red;
-  epi.scal = c.scal;
-  const Epi full_epi = epi;
-  int prc = BL_OK;
-  const bool peer = arm_peer_epilogue(epi, blk.nrows, &prc);
-  BL_CHECK(prc);
-  const bool sharded = !peer && is_sharded();
-  if (sharded) epi.mode = EPI_NONE;
+  ShardedEpi se;
+  BL_CHECK(se.arm(c, epi, blk.nrows));
   {
   ProfScope prof(BL_PROF_DOTS, (double)(blk.nrows + 1) * n * sizeof(T), s);
   if (use_tma(n) && blk.nrows <= 4) {
@@ -295,8 +310,7 @@ int launch_dots(const Grid& g, const Common& c, RowBlock blk, const T* x, int64_
   }
   BL_LAUNCHED();
   }
-  if (sharded) return finish_sharded<T>(c, full_epi, blk.nrows, s);
-  return BL_OK;
+  return se.finish<T>(s);
 }
 
 template <typename T>
@@ -305,12 +319,8 @@ int launch_combine(const Grid& g, const Common& c, CombineArgs a, bool norm, cud
   a.counter = c.counters + 1;
   a.epi.red = c.red;
   a.epi.scal = c.scal;
-  const Epi full_epi = a.epi;
-  int prc = BL_OK;
-  const bool peer = norm && arm_peer_epilogue(a.epi, 1, &prc);
-  BL_CHECK(prc);
-  const bool sharded = norm && !peer && is_sharded();
-  if (sharded) a.epi.mode = EPI_NONE;
+  ShardedEpi se;  // the reduction of ||out||^2 only
+  if (norm) BL_CHECK(se.arm(c, a.epi, 1));
   const int nrows = a.blk[0].nrows + a.blk[1].nrows;
   {
   ProfScope prof(BL_PROF_COMBINE, (double)(nrows + a.nvec + 1 + (a.out2 ? 1 : 0)) * a.n * sizeof(T), s);
@@ -352,8 +362,7 @@ int launch_combine(const Grid& g, const Common& c, CombineArgs a, bool norm, cud
   }
   BL_LAUNCHED();
   }
-  if (sharded) return finish_sharded<T>(c, full_epi, 1, s);
-  return BL_OK;
+  return se.finish<T>(s);
 }
 
 // ---- tensor maps (cuTensorMapEncodeTiled through the runtime's driver entry point) --------
@@ -442,14 +451,8 @@ int launch_fused_tile(const Common& c, const FusedSpec& f, int dtype, int sr, cu
   a.partials = c.partials_dots;
   a.counter = c.counters + 0;
   a.epi = f.epi;
-  a.epi.red = c.red;
-  a.epi.scal = c.scal;
-  const Epi full_epi = a.epi;
-  int prc = BL_OK;
-  const bool peer = arm_peer_epilogue(a.epi, f.res.nrows, &prc);
-  BL_CHECK(prc);
-  const bool sharded = !peer && is_sharded();
-  if (sharded) a.epi.mode = EPI_NONE;
+  ShardedEpi se;
+  BL_CHECK(se.arm(c, a.epi, f.res.nrows));
   a.reverse = next_direction();
   const int nrows = f.res.nrows + f.str0.nrows + f.str1.nrows;
   {
@@ -457,8 +460,7 @@ int launch_fused_tile(const Common& c, const FusedSpec& f, int dtype, int sr, cu
     BL_CUDA(launch_pdl(k_fused_tma<T, TILE>, tma_grid<T>(f.n, TILE), kStreamThreads, L.total_bytes, s, a));
     BL_LAUNCHED();
   }
-  if (sharded) return finish_sharded<T>(c, full_epi, f.res.nrows, s);
-  return BL_OK;
+  return se.finish<T>(s);
 }
 
 // `*fused` is false on return when no tile shape fits shared memory or n is below the TMA threshold;
@@ -493,55 +495,38 @@ int launch_fused(const Common& c, const FusedSpec& f, int dtype, cudaStream_t s,
   return BL_OK;
 }
 
-// out = (sum of <= kXTerms vector terms) / div and red[j] = <row_j, out> over a block of basis rows: the symmetric
-// loops' replacement for the fused kernel (k_xdots_tma, stream_kernels.cuh).  `*done` stays false when n is
-// below the TMA threshold or the shape does not fit; the caller then runs its general kernels.
-struct XDotsSpec {
-  int64_t n = 0;
-  void* out = nullptr;
-  int nvec = 0;
-  VecTerm vec[kXTerms];
-  RowBlock rows;
-  const double* out_div_ptr = nullptr;
-  Epi epi;
-};
-
+// Phase 1 of a symmetric-loop step (StepArgs below) as a launch of its own: out1 = (sum of <= kXTerms vector
+// terms) / div and red[j] = <row_j, out1> over the rows of src1 (k_xdots_tma, stream_kernels.cuh).  `*done` stays
+// false when n is below the TMA threshold or the shape does not fit; the caller then runs its general kernels.
 template <typename T>
-int launch_xdots(const Common& c, const XDotsSpec& f, cudaStream_t s, bool* done) {
+int launch_xdots(const Common& c, const StepArgs& f, cudaStream_t s, bool* done) {
   *done = false;
   constexpr int TILE = kConsumerThreads * Vec<T>::N;  // 4 KB row segments
   const size_t smem = (size_t)(kStages * kGroup + 2) * TILE * sizeof(T) + (2 * kStages + 4) * 8 +
-                      (size_t)f.rows.nrows * 8 + 16;
-  if (!use_tma(f.n) || f.nvec > kXTerms || f.rows.nrows < 1 || smem > 112 * 1024) return BL_OK;
+                      (size_t)f.nrows1 * 8 + 16;
+  if (!use_tma(f.n) || f.nvec > kXTerms || f.nrows1 < 1 || smem > 112 * 1024) return BL_OK;
   *done = true;
   XDotsArgs a;
-  a.src = row_source(f.rows, nullptr, sizeof(T));
-  a.nrows = f.rows.nrows;
+  a.src = f.src1;
+  a.nrows = f.nrows1;
   a.n = f.n;
-  a.out = f.out;
+  a.out = f.out1;
   a.nvec = f.nvec;
   for (int k = 0; k < f.nvec; ++k) a.vec[k] = f.vec[k];
   a.out_div_ptr = f.out_div_ptr;
   a.partials = c.partials_dots;
   a.counter = c.counters + 0;
-  a.epi = f.epi;
-  a.epi.red = c.red;
-  a.epi.scal = c.scal;
-  const Epi full_epi = a.epi;
-  int prc = BL_OK;
-  const bool peer = arm_peer_epilogue(a.epi, f.rows.nrows, &prc);
-  BL_CHECK(prc);
-  const bool sharded = !peer && is_sharded();
-  if (sharded) a.epi.mode = EPI_NONE;
+  a.epi = f.epi1;
+  ShardedEpi se;
+  BL_CHECK(se.arm(c, a.epi, f.nrows1));
   a.reverse = next_direction();
   BL_CHECK(set_smem(k_xdots_tma<T, TILE>, 112 * 1024));
   {
-    ProfScope prof(BL_PROF_FUSED, (double)(f.rows.nrows + f.nvec + 1) * f.n * sizeof(T), s);
+    ProfScope prof(BL_PROF_FUSED, (double)(f.nrows1 + f.nvec + 1) * f.n * sizeof(T), s);
     BL_CUDA(launch_pdl(k_xdots_tma<T, TILE>, tma_grid<T>(f.n, TILE), kStreamThreads, smem, s, a));
     BL_LAUNCHED();
   }
-  if (sharded) return finish_sharded<T>(c, full_epi, f.rows.nrows, s);
-  return BL_OK;
+  return se.finish<T>(s);
 }
 
 // One launch for the three basis-streaming phases of a symmetric-loop step (k_step_tma, step_kernel.cuh).  The kernel's
@@ -745,8 +730,8 @@ bool symmetric_forward(int flags) {
 
 // ---------------------------------------------------------------------------------------
 // One Arnoldi forward run, split at the matvec so that several runs (probes) can advance in lockstep
-// and share ONE batched matvec per step (arnoldi_forward_batch_t): begin(), then per step
-// pre(i) -> [r = A q_i] -> post(i).
+// and share ONE batched matvec per step (arnoldi_forward_t): begin(), then per step
+// [q_i = v / length, v = A q_i] -> post(i), or the whole step in one k_step_tma launch (step_item).
 template <typename T>
 struct FwdRun {
   bl_operator_t* op;
@@ -775,21 +760,6 @@ struct FwdRun {
 
   T* q_row(int i) const { return Q + (int64_t)i * ld; }
 
-  // q_i = v / length, v = A q_i                                               arnoldi.py:80-84
-  int advance(int i) {
-    {
-      ProfScope prof(BL_PROF_MATVEC, op->matvec_bytes(dtype) + 2.0 * n * sizeof(T), s);
-      const int rc = op->matvec_normalised(dtype, r, c.scal + S_LEN, q_row(i), ld, alt, s);
-      if (rc == BL_OK) {
-        std::swap(r, alt);
-        return BL_OK;
-      }
-      if (rc != -1) return rc;
-    }
-    BL_CHECK(pre(i));
-    ProfScope prof(BL_PROF_MATVEC, op->matvec_bytes(dtype), s);
-    return op->matvec(dtype, q_row(i), r, s);
-  }
   int finish() {
     if (r != r_out) {
       BL_CUDA(cudaMemcpyAsync(r_out, r, (size_t)n * sizeof(T), cudaMemcpyDeviceToDevice, s));
@@ -819,6 +789,18 @@ struct FwdRun {
   }
     return BL_OK;
   }
+  // epilogue of the first pass's dots: h = Q^H v over the active rows        arnoldi.py:87
+  Epi pass_a_epi(int i) const {
+    Epi e;
+    e.mode = EPI_FWD_A;
+    e.i = i;
+    e.K = K;
+    e.j0 = first_lo(i);
+    e.m = i + 1 - e.j0;
+    e.H = H;
+    e.coef = c.coefA;
+    return e;
+  }
   // epilogue of the second pass's dots: coefB = Q^H v'; with the local first pass also H[j < i-1, i]
   Epi pass_b_epi(int i) const {
     Epi e;
@@ -831,33 +813,35 @@ struct FwdRun {
     e.H = local_first ? H : nullptr;
     return e;
   }
+  // epilogue of the last combine: length = sqrt(v . v); h[i+1] = length       arnoldi.py:95-98
+  Epi norm_epi(int i) const {
+    Epi e;
+    e.mode = EPI_FWD_NORM;
+    e.i = i;
+    e.K = K;
+    e.H = H;
+    return e;
+  }
   int pre(int i) {
     T* qi = Q + (int64_t)i * ld;
     // v /= length; Q[:, i] = v                                                 arnoldi.py:80-81
     BL_CHECK(launch_scale_copy<T>(n, r, 1.0, c.scal + S_LEN, qi, ld, s));
     return BL_OK;
   }
-  // symmetric loop, ONE launch: h = (q_{i-1}, q_i)^H v | v' = v - h_{i-1} q_{i-1} - h_i q_i, h2 = Q^H v' |
-  // v'' = v' - Q h2, ||v''||                                                     arnoldi.py:87-98
-  bool step_item(int i, StepItem& item) const {
-    if (!(second_pass && local_first)) return false;
+  // symmetric loop (local_first), step i as ONE k_step_tma item on x = A q_i, updated in place:
+  // h = (q_{i-1}, q_i)^H x | x' = x - h_{i-1} q_{i-1} - h_i q_i, h2 = Q^H x' | x'' = x' - Q h2, ||x''||   arnoldi.py:87-98
+  StepItem step_item(int i, T* x) const {
     const int m = i + 1, j0 = first_lo(i);
+    StepItem item{};
     item.c = &c;
     StepArgs& a = item.a;
-    a = StepArgs();
     a.n = n;
     a.few_n = m - j0;
     for (int j = j0; j < m; ++j) a.few_row[j - j0] = q_row(j);
-    a.few_x = r;
-    a.epi0.mode = EPI_FWD_A;
-    a.epi0.i = i;
-    a.epi0.K = K;
-    a.epi0.j0 = j0;
-    a.epi0.m = m - j0;
-    a.epi0.H = H;
-    a.epi0.coef = c.coefA;
-    a.out1 = r;
-    a.vec[a.nvec++] = term(r);
+    a.few_x = x;
+    a.epi0 = pass_a_epi(i);
+    a.out1 = x;
+    a.vec[a.nvec++] = term(x);
     for (int j = j0; j < m; ++j) a.vec[a.nvec++] = term(q_row(j), -1.0, c.coefA + j);
     a.src1 = row_source(rows(Q, ld, 0, m), nullptr, sizeof(T));
     a.nrows1 = m;
@@ -866,74 +850,48 @@ struct FwdRun {
     a.nrows2 = m;
     a.coef2 = c.coefB;
     a.sign2 = -1.0;
-    a.out2 = r;
+    a.out2 = x;
     a.norm = 1;
-    a.epi2.mode = EPI_FWD_NORM;  // length = sqrt(v . v); h[i+1] = length        arnoldi.py:95-98
-    a.epi2.i = i;
-    a.epi2.K = K;
-    a.epi2.H = H;
+    a.epi2 = norm_epi(i);
     a.wait_row = i;  // row i is the operator kernel's output (fused normalise + matvec)
     item.bytes = (double)((m - j0 + 1) + (m + a.nvec + 1) + (m + 2)) * n * sizeof(T);
-    return true;
+    return item;
   }
-  // The same with the operator call in the launch (phase S): q_i = v / length, v = A q_i, then the step.  The
-  // current vector moves to the spare buffer first (the gathers of phase S read the whole input while other blocks
-  // write the output); `unfuse` undoes that when the launch did not happen.               arnoldi.py:80-98
-  bool fused_item(int i, const StepOp* sop, StepItem& item) {
-    std::swap(r, alt);
-    if (!step_item(i, item)) {
-      std::swap(r, alt);
-      return false;
-    }
+  // The same with the operator call in the launch (phase S): q_i = v / length, x = A q_i, then the step.  x is the
+  // spare buffer (the gathers of phase S read the whole input while other blocks write the output): after the
+  // launch the caller swaps `r` and `alt`.                                                  arnoldi.py:80-98
+  StepItem fused_item(int i, const StepOp* sop) const {
+    StepItem item = step_item(i, alt);
     item.op = sop;
-    item.a.op_x = alt;
+    item.a.op_x = r;
     item.a.op_q = q_row(i);
     item.a.op_len = c.scal + S_LEN;
     item.a.wait_row = std::max(0, i - 1);  // rows i-1 (the predecessor's phase S) and i (this launch's)
     item.bytes += op->matvec_bytes(dtype) + 1.0 * n * sizeof(T);
-    return true;
+    return item;
   }
-  void unfuse() { std::swap(r, alt); }
+  // Step i as separate launches: the general loop, which for the symmetric loop is step_item(i) lowered -- phase 0
+  // is the first dots launch, phase 1 k_xdots_tma (n below the TMA threshold: the general kernels), phase 2 the
+  // second pass's combine.
   int post(int i) {
-    const int m = i + 1;
-    Epi epi_a;  // h = Q^H v (active columns only)                              arnoldi.py:87
-    epi_a.mode = EPI_FWD_A;
-    epi_a.i = i;
-    epi_a.K = K;
-    epi_a.j0 = first_lo(i);
-    epi_a.m = m - epi_a.j0;
-    epi_a.H = H;
-    epi_a.coef = c.coefA;
-    Epi norm_epi;  // length = sqrt(v . v); h[i+1] = length                      arnoldi.py:95-98
-    norm_epi.mode = EPI_FWD_NORM;
-    norm_epi.i = i;
-    norm_epi.K = K;
-    norm_epi.H = H;
-    BL_CHECK(launch_dots<T>(g, c, rows(Q, ld, epi_a.j0, epi_a.m), r, n, epi_a, s));
+    const int m = i + 1, j0 = first_lo(i);
+    BL_CHECK(launch_dots<T>(g, c, rows(Q, ld, j0, m - j0), r, n, pass_a_epi(i), s));
     bool fused = false;
-    if (second_pass && local_first) {
-      // symmetric loop: v = v - h_{i-1} q_{i-1} - h_i q_i is a three-vector combination, and h2 = Q^H v streams
-      // every active row once (no row is needed twice: nothing stays resident)   arnoldi.py:88,92
-      XDotsSpec f;
-      f.n = n;
-      f.out = r;
-      f.vec[f.nvec++] = term(r);
-      for (int j = first_lo(i); j < m; ++j) f.vec[f.nvec++] = term(q_row(j), -1.0, c.coefA + j);
-      f.rows = rows(Q, ld, 0, m);
-      f.epi = pass_b_epi(i);
-      BL_CHECK(launch_xdots<T>(c, f, s, &fused));
+    if (local_first) {
+      // v = v - h_{i-1} q_{i-1} - h_i q_i is a three-vector combination, and h2 = Q^H v streams every active row
+      // once (no row is needed twice: nothing stays resident)                 arnoldi.py:88,92
+      BL_CHECK(launch_xdots<T>(c, step_item(i, r).a, s, &fused));
     }
     if (second_pass && !fused) {
       // v = v - Q h and, from the same read of Q, h2 = Q^H v (the second pass's coefficients;
       // h itself is not updated, arnoldi.py:92)
-      Epi e = pass_b_epi(i);
       FusedSpec f;
       f.n = n;
       f.out = r;
       f.nvec = 1;
       f.vec[0] = term(r);
       f.res = rows(Q, ld, 0, m, c.coefA, -1.0);
-      f.epi = e;
+      f.epi = pass_b_epi(i);
       BL_CHECK(launch_fused<T>(c, f, dtype, s, &fused));
     }
     if (!fused) {  // v = v - Q h                                               arnoldi.py:88
@@ -942,8 +900,8 @@ struct FwdRun {
       a.out = r;
       a.nvec = 1;
       a.vec[0] = term(r);
-      a.blk[0] = rows(Q, ld, first_lo(i), m - first_lo(i), c.coefA, -1.0, first_lo(i));
-      a.epi = norm_epi;
+      a.blk[0] = rows(Q, ld, j0, m - j0, c.coefA, -1.0, j0);
+      a.epi = norm_epi(i);
       BL_CHECK(launch_combine<T>(g, c, a, !second_pass, s));
       if (second_pass) {
         BL_CHECK(launch_dots<T>(g, c, rows(Q, ld, 0, m), r, n, pass_b_epi(i), s));
@@ -956,62 +914,48 @@ struct FwdRun {
       a.nvec = 1;
       a.vec[0] = term(r);
       a.blk[0] = rows(Q, ld, 0, m, c.coefB, -1.0);
-      a.epi = norm_epi;
+      a.epi = norm_epi(i);
       BL_CHECK(launch_combine<T>(g, c, a, true, s));
     }
     return BL_OK;
   }
 };
 
+// P independent runs in lockstep (P = 1: bl_arnoldi_forward): per step one batched matvec for all of them, and
+// for the symmetric loop the Gram-Schmidt step of all of them in one launch per kStepBatch runs.  Each run owns
+// `per` bytes of the workspace.
 template <typename T>
-int arnoldi_forward_t(bl_operator_t* op, int dtype, int64_t n, int K, int flags, const T* v, T* Q,
-                      int64_t ld, T* H, T* r, T* c_out, void* workspace, size_t wbytes, cudaStream_t s) {
-  FwdRun<T> run{op, dtype, n, K, (flags & BL_FWD_SECOND_PASS) != 0, v, Q, ld, H, r, c_out, workspace, wbytes, s, {}, {}};
-  run.local_first = symmetric_forward(flags);
-  BL_CHECK(run.begin());
-  for (int i = 0; i < K; ++i) {
-    BL_CHECK(run.advance(i));
-    BL_CHECK(run.post(i));
-  }
-  return run.finish();
-}
-
-// P independent runs in lockstep: per step one batched matvec for all of them.
-template <typename T>
-int arnoldi_forward_batch_t(bl_operator_t* op, int dtype, int64_t n, int K, int flags, int P, const T* v,
-                            int64_t ldv, T* Q, int64_t ld, T* H, T* r, T* c_out, void* workspace, size_t wbytes,
-                            cudaStream_t s) {
-  const size_t per = bl_arnoldi_workspace_bytes(n, K, dtype);
-  BL_REQUIRE(wbytes >= per * (size_t)P, "workspace too small (P * bl_arnoldi_workspace_bytes)");
+int arnoldi_forward_t(bl_operator_t* op, int dtype, int64_t n, int K, int flags, int P, const void* v_, int64_t ldv,
+                      void* Q_, int64_t ld, void* H_, void* r_, void* c_, void* workspace, size_t per, cudaStream_t s) {
+  const T* v = static_cast<const T*>(v_);
+  T *Q = static_cast<T*>(Q_), *H = static_cast<T*>(H_), *r = static_cast<T*>(r_), *c_out = static_cast<T*>(c_);
+  const bool symmetric = symmetric_forward(flags);
   std::vector<FwdRun<T>> runs;
-  std::vector<const void*> in(P);
-  std::vector<void*> out(P);
   for (int p = 0; p < P; ++p) {
     runs.push_back(FwdRun<T>{op, dtype, n, K, (flags & BL_FWD_SECOND_PASS) != 0, v + (int64_t)p * ldv, Q + (int64_t)p * K * ld, ld,
                              H + (int64_t)p * K * K, r + (int64_t)p * ld, c_out + p,
                              static_cast<char*>(workspace) + per * p, per, s, {}, {}});
-    runs.back().local_first = symmetric_forward(flags);
+    runs.back().local_first = symmetric;
     BL_CHECK(runs.back().begin());
-    out[p] = runs[p].r;
   }
+  std::vector<const void*> in(P);
+  std::vector<void*> out(P);
   std::vector<const double*> lens(P);
   std::vector<void*> qout(P);
+  std::vector<StepItem> items(P);
   StepOp sop;
-  const bool fuse = (flags & BL_FWD_SECOND_PASS) != 0 && symmetric_forward(flags) &&
-                    make_step_op(op, dtype, false, true, n, ld, &sop);
+  const bool fuse = symmetric && make_step_op(op, dtype, false, true, n, ld, &sop);
   for (int i = 0; i < K; ++i) {
+    bool stepped = false;
     if (fuse) {  // operator call + Gram-Schmidt step of all runs in one launch per kStepBatch runs
-      std::vector<StepItem> items(P);
       sop.wait_first = i == 0;
-      int built = 0;
-      while (built < P && runs[built].fused_item(i, &sop, items[built])) ++built;
-      bool stepped = false;
-      if (built == P) {
-        for (StepItem& it : items) it.bytes += (op->matvec_batch_bytes(dtype, P) - P * op->matvec_bytes(dtype)) / P;
-        BL_CHECK(launch_step<T>(items, s, &stepped));
+      for (int p = 0; p < P; ++p) items[p] = runs[p].fused_item(i, &sop);
+      for (StepItem& it : items) it.bytes += (op->matvec_batch_bytes(dtype, P) - P * op->matvec_bytes(dtype)) / P;
+      BL_CHECK(launch_step<T>(items, s, &stepped));
+      if (stepped) {
+        for (FwdRun<T>& run : runs) std::swap(run.r, run.alt);
+        continue;
       }
-      if (stepped) continue;
-      for (int p = 0; p < built; ++p) runs[p].unfuse();
     }
     int rc = -1;
     {  // q_i = v / length and v = A q_i of every run in one batched operator call     arnoldi.py:80-84
@@ -1037,11 +981,9 @@ int arnoldi_forward_batch_t(bl_operator_t* op, int dtype, int64_t n, int K, int 
     } else {
       return rc;
     }
-    {  // the Gram-Schmidt step of all runs in one launch per kStepBatch runs (k_step_tma)
-      std::vector<StepItem> items(P);
-      bool eligible = true, stepped = false;
-      for (int p = 0; p < P && eligible; ++p) eligible = runs[p].step_item(i, items[p]);
-      if (eligible) BL_CHECK(launch_step<T>(items, s, &stepped));
+    if (symmetric) {  // the Gram-Schmidt step of all runs in one launch per kStepBatch runs (k_step_tma)
+      for (int p = 0; p < P; ++p) items[p] = runs[p].step_item(i, runs[p].r);
+      BL_CHECK(launch_step<T>(items, s, &stepped));
       if (stepped) continue;
     }
     for (int p = 0; p < P; ++p) BL_CHECK(runs[p].post(i));
@@ -1082,7 +1024,7 @@ struct AdjRun {
   double *eta = nullptr, *Gamma = nullptr, *PiGamma = nullptr, *Gmat = nullptr, *gram_partial = nullptr;
   int gram_parts = 0;
   T *z = nullptr, *lam = nullptr;
-  bool defer_grad = false, have_reproj = false;
+  bool defer_grad = false;
   // BL_ADJ_SYMMETRIC: the operand is symmetric, so H is tridiagonal up to rounding (full
   // re-orthogonalisation keeps |H[idx, j]| = O(eps |A|) for j > idx+1) and `Lambda beta_plus`
   // (arnoldi.py:218) reduces to its one O(1) term, -H[idx, idx+1] Lambda[idx+1]: K-idx-2 basis rows
@@ -1102,10 +1044,48 @@ struct AdjRun {
   T* lam_row(int idx) const { return Lambda + (int64_t)idx * ld; }
   // terms of `- Lambda beta_plus`: every later row of Lambda, or (symmetric) row idx+1 as a vector term
   int lam_rows_streamed(int idx) const { return symmetric ? 0 : K - idx - 1; }
-  template <typename Terms>
-  void add_symmetric_term(int idx, Terms& vec, int& nv) const {
+  // Vector terms of the back-substitution (its basis rows follow): dQ[idx] when given, eta[idx] r, -alpha Lambda[idx],
+  // A^T lambda and, for a symmetric operand, -beta_plus Lambda[idx+1].  Returns their count.   arnoldi.py:212-218
+  int back_terms(int idx, VecTerm* vec) const {
+    int nv = 0;
+    if (dQ) vec[nv++] = term(dQ + (int64_t)idx * ld);
+    vec[nv++] = term(r, 1.0, c.scal + S_ETA_IDX);
+    vec[nv++] = term(lam_row(idx), 1.0, c.scal + S_NEG_ALPHA);
+    vec[nv++] = term(z);
     if (symmetric && idx + 1 < K) vec[nv++] = term(lam_row(idx + 1), 1.0, c.coefC + idx + 1);
+    return nv;
   }
+  // epilogue of the dots with A^T lambda: Gamma[idx, :] and the coefficients of the back-substitution   arnoldi.py:212-218
+  Epi gamma_epi(int idx) const {
+    Epi e;
+    e.mode = EPI_ADJ_GAMMA;
+    e.i = idx;
+    e.K = K;
+    e.j0 = band_lo(idx);
+    e.m = idx + 1 - e.j0;
+    e.Hc = H;
+    e.Gamma = Gamma;
+    e.PiGamma = PiGamma;
+    e.eta = eta;
+    e.coef = c.coefB;
+    e.coef2 = c.coefC;
+    return e;
+  }
+  // epilogue of the re-projection dots t = P lambda, rows <= idx+1 of P = Q^T: coefA = p - t   arnoldi.py:201-204
+  Epi reproj_epi(int idx) const {
+    Epi e;
+    e.mode = EPI_ADJ_REPROJ;
+    e.i = idx;
+    e.K = K;
+    e.m = std::min(idx + 2, K);
+    e.dH = dH;
+    e.coef = c.coefA;
+    return e;
+  }
+  // What the step of idx+1 already did of pre(idx): k_step_tma wrote Lambda[idx] (its phase 2), or the separate
+  // launches computed the re-projection coefficients (phase 1); otherwise pre(idx) runs both launches.
+  enum Ahead { kNothing, kReproj, kLambdaRow };
+  Ahead ahead = kNothing;
 
   int begin() {
   Workspace w(workspace, wbytes);
@@ -1178,26 +1158,16 @@ struct AdjRun {
     BL_LAUNCHED();
   }
 
-    have_reproj = false;  // coefA already holds p - P lambda for this idx (fused into the previous step)
     return BL_OK;
   }
-  int pre_done = -1;  // the step kernel of idx+1 already wrote Lambda[idx] (its phase 2)
+  // Lambda[idx] = lambda + Q (p - P lambda): phase 2 of the step of idx+1        arnoldi.py:201-204, 216
   int pre(int idx) {
     T* Lrow = Lambda + (int64_t)idx * ld;
-    if (pre_done == idx) return BL_OK;
+    if (ahead == kLambdaRow) return BL_OK;
     if (reortho_full) {
       // lambda -= P^T (P lambda) - P^T p, rows <= idx+1 of P = Q^T              arnoldi.py:201-204
       const int mact = std::min(idx + 2, K);
-      if (!have_reproj) {
-        Epi e;
-        e.mode = EPI_ADJ_REPROJ;
-        e.i = idx;
-        e.K = K;
-        e.m = mact;
-        e.dH = dH;
-        e.coef = c.coefA;
-        BL_CHECK(launch_dots<T>(g, c, rows(Q, ld, 0, mact), lam, n, e, s));
-      }
+      if (ahead != kReproj) BL_CHECK(launch_dots<T>(g, c, rows(Q, ld, 0, mact), lam, n, reproj_epi(idx), s));
       CombineArgs a;
       a.n = n;
       a.out = Lrow;  // Lambda[:, idx] = lambda                                   arnoldi.py:216
@@ -1210,117 +1180,61 @@ struct AdjRun {
     }
     return BL_OK;
   }
-  // banded Gamma, ONE launch: Gamma row from the dots of z with rows idx-2..idx | back-substitution and the
-  // next step's re-projection dots | Lambda[idx-1] = lambda + Q (p - P lambda)   arnoldi.py:212-219, 201-204, 216
-  bool step_item(int idx, StepItem& item) const {
-    if (!(banded && idx > 0 && reortho_full)) return false;
-    T* Lrow = Lambda + (int64_t)idx * ld;
+  // banded Gamma (idx > 0), step idx as ONE k_step_tma item: Gamma row from the dots of z with rows idx-2..idx |
+  // back-substitution and the next step's re-projection dots | Lambda[idx-1] = lambda + Q (p - P lambda)
+  //                                                                             arnoldi.py:212-219, 201-204, 216
+  StepItem step_item(int idx) const {
+    const int j0 = band_lo(idx);
+    StepItem item{};
     item.c = &c;
     StepArgs& a = item.a;
-    a = StepArgs();
     a.n = n;
-    const int j0 = band_lo(idx);
     a.few_n = idx + 1 - j0;
     for (int j = j0; j <= idx; ++j) a.few_row[j - j0] = q_row(j);
     a.few_x = z;
-    a.epi0.mode = EPI_ADJ_GAMMA;
-    a.epi0.i = idx;
-    a.epi0.K = K;
-    a.epi0.j0 = j0;
-    a.epi0.m = idx + 1 - j0;
-    a.epi0.Hc = H;
-    a.epi0.Gamma = Gamma;
-    a.epi0.PiGamma = PiGamma;
-    a.epi0.eta = eta;
-    a.epi0.coef = c.coefB;
-    a.epi0.coef2 = c.coefC;
+    a.epi0 = gamma_epi(idx);
     a.out1 = lam;
-    a.vec[a.nvec++] = term(r, 1.0, c.scal + S_ETA_IDX);
-    a.vec[a.nvec++] = term(Lrow, 1.0, c.scal + S_NEG_ALPHA);
-    a.vec[a.nvec++] = term(z);
-    add_symmetric_term(idx, a.vec, a.nvec);
-    for (int j = band_lo(idx); j < band_hi(idx); ++j) a.vec[a.nvec++] = term(q_row(j), 1.0, c.coefB + j);
+    a.nvec = back_terms(idx, a.vec);
+    for (int j = j0; j < band_hi(idx); ++j) a.vec[a.nvec++] = term(q_row(j), 1.0, c.coefB + j);
     a.out_div_ptr = c.scal + S_BETA_MINUS;
     a.src1 = row_source(rows(Q, ld, 0, idx + 1), nullptr, sizeof(T));
     a.nrows1 = idx + 1;
-    a.epi1.mode = EPI_ADJ_REPROJ;
-    a.epi1.i = idx - 1;
-    a.epi1.K = K;
-    a.epi1.m = idx + 1;
-    a.epi1.dH = dH;
-    a.epi1.coef = c.coefA;
+    a.epi1 = reproj_epi(idx - 1);
     a.src2 = a.src1;  // rows <= (idx-1)+1 of P = Q^T
     a.nrows2 = idx + 1;
     a.coef2 = c.coefA;
     a.sign2 = 1.0;
-    a.out2 = Lambda + (int64_t)(idx - 1) * ld;
+    a.out2 = lam_row(idx - 1);
     a.norm = 0;
     item.bytes = (double)((a.few_n + 1) + (idx + 1 + a.nvec + 1) + (idx + 1 + 2)) * n * sizeof(T);
-    return true;
+    return item;
   }
   // The same with z = A^T Lambda[idx] in the launch (phase S; deferred parameter cotangent only).
-  bool fused_item(int idx, const StepOp* sop, StepItem& item) const {
-    if (!defer_grad || !step_item(idx, item)) return false;
+  StepItem fused_item(int idx, const StepOp* sop) const {
+    StepItem item = step_item(idx);
     item.op = sop;
     item.a.op_x = lam_row(idx);
     item.bytes += op->apply_transpose_bytes(dtype);
-    return true;
+    return item;
   }
-  void stepped(int idx) {  // the step kernel of idx also did pre(idx - 1)
-    pre_done = idx - 1;
-    have_reproj = false;
-  }
+  // Step idx as separate launches: the general loop, which for banded Gamma is step_item(idx) lowered -- phase 0 is
+  // the Gamma dots, phase 1 k_xdots_tma (n below the TMA threshold: the general kernels), phase 2 pre(idx - 1).
   int post(int idx) {
-    T* Lrow = Lambda + (int64_t)idx * ld;
-    Epi epi_g;  // Gamma[idx, :] and the coefficients of the back-substitution      arnoldi.py:212-218
-    epi_g.mode = EPI_ADJ_GAMMA;
-    epi_g.i = idx;
-    epi_g.K = K;
-    epi_g.j0 = band_lo(idx);
-    epi_g.m = idx + 1 - epi_g.j0;
-    epi_g.Hc = H;
-    epi_g.Gamma = Gamma;
-    epi_g.PiGamma = PiGamma;
-    epi_g.eta = eta;
-    epi_g.coef = c.coefB;
-    epi_g.coef2 = c.coefC;
     // lambda = (Pi_xi[idx] + Q gamma_row - alpha lambda + A^T lambda - Lambda beta_plus) / beta_minus
-    have_reproj = false;
-    BL_CHECK(launch_dots<T>(g, c, rows(Q, ld, epi_g.j0, epi_g.m), z, n, epi_g, s));
+    BL_CHECK(launch_dots<T>(g, c, rows(Q, ld, band_lo(idx), idx + 1 - band_lo(idx)), z, n, gamma_epi(idx), s));
+    bool reproj = false;
     if (banded && idx > 0) {
       // banded Gamma: the back-substitution combines nine vectors at most, and the NEXT step's re-projection dots
       // t = P lambda stream rows 0..idx once                                    arnoldi.py:202,217-219
-      XDotsSpec f;
-      f.n = n;
-      f.out = lam;
-      f.vec[f.nvec++] = term(r, 1.0, c.scal + S_ETA_IDX);
-      f.vec[f.nvec++] = term(Lrow, 1.0, c.scal + S_NEG_ALPHA);
-      f.vec[f.nvec++] = term(z);
-      add_symmetric_term(idx, f.vec, f.nvec);
-      for (int j = band_lo(idx); j < band_hi(idx); ++j) f.vec[f.nvec++] = term(q_row(j), 1.0, c.coefB + j);
-      f.rows = rows(Q, ld, 0, idx + 1);
-      f.out_div_ptr = c.scal + S_BETA_MINUS;
-      f.epi.mode = EPI_ADJ_REPROJ;
-      f.epi.i = idx - 1;
-      f.epi.K = K;
-      f.epi.m = idx + 1;
-      f.epi.dH = dH;
-      f.epi.coef = c.coefA;
-      BL_CHECK(launch_xdots<T>(c, f, s, &have_reproj));
+      BL_CHECK(launch_xdots<T>(c, step_item(idx).a, s, &reproj));
     }
-    if (!have_reproj && reortho_full && idx > 0) {
+    if (!reproj && reortho_full && idx > 0) {
       // ... fused with the NEXT step's re-projection dots t = P lambda (rows 0..idx of Q are the
       // active rows of P at idx-1): one read of those rows serves both          arnoldi.py:202,217-219
       FusedSpec f;
       f.n = n;
       f.out = lam;
-      int nv = 0;
-      if (dQ) f.vec[nv++] = term(dQ + (int64_t)idx * ld);
-      f.vec[nv++] = term(r, 1.0, c.scal + S_ETA_IDX);
-      f.vec[nv++] = term(Lrow, 1.0, c.scal + S_NEG_ALPHA);
-      f.vec[nv++] = term(z);
-      add_symmetric_term(idx, f.vec, nv);
-      f.nvec = nv;
+      f.nvec = back_terms(idx, f.vec);
       // banded: rows idx+1, idx+2 ride as resident rows (their two extra dots are not read by the epilogue)
       const int nres = banded ? band_hi(idx) : idx + 1;
       f.res = rows(Q, ld, 0, nres, c.coefB, 1.0);
@@ -1329,30 +1243,20 @@ struct AdjRun {
       f.rows_total0 = K;
       f.rows_total1 = K;
       f.out_div_ptr = c.scal + S_BETA_MINUS;
-      f.epi.mode = EPI_ADJ_REPROJ;
-      f.epi.i = idx - 1;
-      f.epi.K = K;
-      f.epi.m = idx + 1;
-      f.epi.dH = dH;
-      f.epi.coef = c.coefA;
-      BL_CHECK(launch_fused<T>(c, f, dtype, s, &have_reproj));
+      f.epi = reproj_epi(idx - 1);
+      BL_CHECK(launch_fused<T>(c, f, dtype, s, &reproj));
     }
-    if (!have_reproj) {
+    if (!reproj) {
       CombineArgs a;
       a.n = n;
       a.out = lam;
-      int nv = 0;
-      if (dQ) a.vec[nv++] = term(dQ + (int64_t)idx * ld);
-      a.vec[nv++] = term(r, 1.0, c.scal + S_ETA_IDX);
-      a.vec[nv++] = term(Lrow, 1.0, c.scal + S_NEG_ALPHA);
-      a.vec[nv++] = term(z);
-      add_symmetric_term(idx, a.vec, nv);
-      a.nvec = nv;
+      a.nvec = back_terms(idx, a.vec);
       a.blk[0] = rows(Q, ld, band_lo(idx), band_hi(idx) - band_lo(idx), c.coefB, 1.0, band_lo(idx));
       a.blk[1] = rows(Lambda, ld, idx + 1, lam_rows_streamed(idx), c.coefC, 1.0, idx + 1);
       a.out_div_ptr = c.scal + S_BETA_MINUS;
       BL_CHECK(launch_combine<T>(g, c, a, false, s));
     }
+    ahead = reproj ? kReproj : kNothing;
     return BL_OK;
   }
   int end() {
@@ -1371,43 +1275,18 @@ struct AdjRun {
   }
 };
 
+// P independent adjoint runs in lockstep (P = 1: bl_arnoldi_adjoint; the bases of P forward runs are contiguous:
+// Q[p][K][ld]): one batched A^T Lambda per step, and ONE batched parameter-cotangent pass over all P*K
+// (lambda, q) pairs.  Each run owns `per` bytes of the workspace.
 template <typename T>
-int arnoldi_adjoint_t(bl_operator_t* op, int dtype, int64_t n, int K, int flags, const T* Q,
-                      int64_t ld, const T* H, const T* r, const T* c_in, const T* dQ, const T* dH,
-                      const T* dr, const T* dc, T* dv, T* Lambda, void* workspace, size_t wbytes,
+int arnoldi_adjoint_t(bl_operator_t* op, int dtype, int64_t n, int K, int flags, int P, const void* Q_, int64_t ld,
+                      const void* H_, const void* r_, const void* c_, const void* dQ_, const void* dH_, const void* dr_,
+                      const void* dc_, void* dv_, int64_t lddv, void* Lambda_, void* workspace, size_t per,
                       cudaStream_t s) {
-  AdjRun<T> run{op, dtype, n, K, (flags & BL_ADJ_REORTHO_FULL) != 0, Q, ld, H, r, c_in, dQ, dH, dr, dc, dv, Lambda, workspace, wbytes, s, {}, {}};
-  run.symmetric = symmetric_shortcut(flags);
-  run.tridiag_cot = (flags & BL_ADJ_TRIDIAG_COTANGENT) != 0;
-  BL_CHECK(run.begin());
-  for (int idx = K - 1; idx >= 0; --idx) {
-    BL_CHECK(run.pre(idx));
-    // (A^T lambda, dparams += ...) = vjp of matvec at (q_idx, params)            arnoldi.py:207-209
-    {
-      ProfScope prof(BL_PROF_VJP, run.defer_grad ? op->apply_transpose_bytes(dtype) : op->vjp_bytes(dtype), s);
-      if (run.defer_grad)  // A^T lambda only; the parameter cotangent of all K steps follows in one batched pass
-        BL_CHECK(op->apply_transpose(dtype, run.lam_row(idx), run.z, s));
-      else
-        BL_CHECK(op->vjp(dtype, run.q_row(idx), run.lam_row(idx), run.z, s));
-    }
-    BL_CHECK(run.post(idx));
-  }
-  if (run.defer_grad) {  // dparams = sum_idx d<Lambda[idx], A(Q[idx]; params)>/dparams   arnoldi.py:207-209, 168
-    ProfScope prof(BL_PROF_VJP, op->vjp_batch_bytes(dtype, K), s);
-    BL_CHECK(op->vjp_batch(dtype, Q, ld, Lambda, ld, K, s));
-  }
-  return run.end();
-}
-
-// P independent adjoint runs in lockstep (bases of the P forward runs are contiguous: Q[p][K][ld]): one
-// batched A^T Lambda per step, and ONE batched parameter-cotangent pass over all P*K (lambda, q) pairs.
-template <typename T>
-int arnoldi_adjoint_batch_t(bl_operator_t* op, int dtype, int64_t n, int K, int flags, int P, const T* Q,
-                            int64_t ld, const T* H, const T* r, const T* c_in, const T* dQ, const T* dH, const T* dr,
-                            const T* dc, T* dv, int64_t lddv, T* Lambda, void* workspace, size_t wbytes,
-                            cudaStream_t s) {
-  const size_t per = bl_arnoldi_workspace_bytes(n, K, dtype);
-  BL_REQUIRE(wbytes >= per * (size_t)P, "workspace too small (P * bl_arnoldi_workspace_bytes)");
+  const T *Q = static_cast<const T*>(Q_), *H = static_cast<const T*>(H_), *r = static_cast<const T*>(r_);
+  const T *c_in = static_cast<const T*>(c_), *dQ = static_cast<const T*>(dQ_), *dH = static_cast<const T*>(dH_);
+  const T *dr = static_cast<const T*>(dr_), *dc = static_cast<const T*>(dc_);
+  T *dv = static_cast<T*>(dv_), *Lambda = static_cast<T*>(Lambda_);
   const bool deferred = op->deferred_grad(dtype);
   std::vector<AdjRun<T>> runs;
   std::vector<const void*> in(P);
@@ -1423,6 +1302,7 @@ int arnoldi_adjoint_batch_t(bl_operator_t* op, int dtype, int64_t n, int K, int 
     BL_CHECK(runs.back().begin());
     out[p] = runs[p].z;
   }
+  std::vector<StepItem> items(P);
   StepOp sop;
   const bool fuse = deferred && runs[0].banded && make_step_op(op, dtype, true, false, n, ld, &sop);
   for (int idx = K - 1; idx >= 0; --idx) {
@@ -1430,42 +1310,36 @@ int arnoldi_adjoint_batch_t(bl_operator_t* op, int dtype, int64_t n, int K, int 
       BL_CHECK(runs[p].pre(idx));
       in[p] = runs[p].lam_row(idx);
     }
-    if (fuse) {  // A^T lambda + back-substitution + the next re-projection of all runs in one launch
-      std::vector<StepItem> items(P);
+    const bool banded_step = runs[0].banded && idx > 0;  // the step has a k_step_tma form (AdjRun::step_item)
+    bool stepped = false;
+    if (fuse && banded_step) {  // A^T lambda + back-substitution + the next re-projection of all runs in one launch
       sop.wait_first = idx == K - 1;
-      int built = 0;
-      while (built < P && runs[built].fused_item(idx, &sop, items[built])) ++built;
-      bool done = false;
-      if (built == P) {
-        for (StepItem& it : items) it.bytes += (op->matvec_batch_bytes(dtype, P) - P * op->matvec_bytes(dtype)) / P;
-        BL_CHECK(launch_step<T>(items, s, &done));
+      for (int p = 0; p < P; ++p) items[p] = runs[p].fused_item(idx, &sop);
+      for (StepItem& it : items) it.bytes += (op->matvec_batch_bytes(dtype, P) - P * op->matvec_bytes(dtype)) / P;
+      BL_CHECK(launch_step<T>(items, s, &stepped));
+    }
+    if (!stepped) {
+      {  // (A^T lambda, dparams += ...) = vjp of matvec at (q_idx, params)          arnoldi.py:207-209
+        ProfScope prof(BL_PROF_VJP, deferred ? op->matvec_batch_bytes(dtype, P) : op->vjp_bytes(dtype) * P, s);
+        if (deferred) {  // A^T lambda only; the parameter cotangent of all steps follows in one batched pass
+          BL_CHECK(op->apply_transpose_batch(dtype, P, in.data(), out.data(), s));
+        } else {  // the parameter cotangent accumulates in the operator over steps and runs (a sum over the batch)
+          for (int p = 0; p < P; ++p) BL_CHECK(op->vjp(dtype, runs[p].q_row(idx), in[p], out[p], s));
+        }
       }
-      if (done) {
-        for (int p = 0; p < P; ++p) runs[p].stepped(idx);
-        continue;
+      if (banded_step) {  // back-substitution, re-projection dots and the next Lambda row of all runs in one launch
+        for (int p = 0; p < P; ++p) items[p] = runs[p].step_item(idx);
+        BL_CHECK(launch_step<T>(items, s, &stepped));
       }
     }
-    {
-      ProfScope prof(BL_PROF_VJP, deferred ? op->matvec_batch_bytes(dtype, P) : op->vjp_bytes(dtype) * P, s);
-      if (deferred) {
-        BL_CHECK(op->apply_transpose_batch(dtype, P, in.data(), out.data(), s));
-      } else {  // the parameter cotangent accumulates in the operator over steps and runs (a sum over the batch)
-        for (int p = 0; p < P; ++p) BL_CHECK(op->vjp(dtype, runs[p].q_row(idx), in[p], out[p], s));
-      }
+    for (AdjRun<T>& run : runs) {
+      if (stepped)
+        run.ahead = AdjRun<T>::kLambdaRow;  // the launch also wrote Lambda[idx - 1] (its phase 2)
+      else
+        BL_CHECK(run.post(idx));
     }
-    {  // back-substitution, re-projection dots and the next Lambda row of all runs in one launch (k_step_tma)
-      std::vector<StepItem> items(P);
-      bool eligible = true, done = false;
-      for (int p = 0; p < P && eligible; ++p) eligible = runs[p].step_item(idx, items[p]);
-      if (eligible) BL_CHECK(launch_step<T>(items, s, &done));
-      if (done) {
-        for (int p = 0; p < P; ++p) runs[p].stepped(idx);
-        continue;
-      }
-    }
-    for (int p = 0; p < P; ++p) BL_CHECK(runs[p].post(idx));
   }
-  if (deferred) {
+  if (deferred) {  // dparams = sum_idx d<Lambda[idx], A(Q[idx]; params)>/dparams   arnoldi.py:207-209, 168
     ProfScope prof(BL_PROF_VJP, op->vjp_batch_bytes(dtype, P * K), s);
     BL_CHECK(op->vjp_batch(dtype, Q, ld, Lambda, ld, P * K, s));
   }
@@ -1641,18 +1515,16 @@ size_t bl_arnoldi_workspace_bytes(int64_t n, int64_t K, int dtype) {
   return b + 16 * 256;
 }
 
+// One run is a lockstep batch of one whose slice is the caller's whole workspace (AdjRun / FwdRun::begin refuse a
+// workspace that is too small before anything is launched).
 int bl_arnoldi_forward(bl_operator_t* op, int dtype, int64_t n, int64_t K, int second_pass, const void* v,
                        void* Q, int64_t ld, void* H, void* r, void* c, void* workspace,
                        size_t workspace_bytes, void* stream) {
   BL_REQUIRE(op && v && Q && H && r && c && workspace, "NULL argument");
   BL_CHECK(check_basis(dtype, n, K, ld, Q));
   BL_REQUIRE(op->n == n, "operator size does not match n");
-  cudaStream_t s = as_stream(stream);
-  if (dtype == BL_F32)
-    return arnoldi_forward_t<float>(op, dtype, n, (int)K, second_pass, (const float*)v, (float*)Q, ld,
-                                    (float*)H, (float*)r, (float*)c, workspace, workspace_bytes, s);
-  return arnoldi_forward_t<double>(op, dtype, n, (int)K, second_pass, (const double*)v, (double*)Q, ld,
-                                   (double*)H, (double*)r, (double*)c, workspace, workspace_bytes, s);
+  const auto run = dtype == BL_F32 ? arnoldi_forward_t<float> : arnoldi_forward_t<double>;
+  return run(op, dtype, n, (int)K, second_pass, 1, v, n, Q, ld, H, r, c, workspace, workspace_bytes, as_stream(stream));
 }
 
 int bl_arnoldi_adjoint(bl_operator_t* op, int dtype, int64_t n, int64_t K, int reortho_full, const void* Q,
@@ -1665,16 +1537,9 @@ int bl_arnoldi_adjoint(bl_operator_t* op, int dtype, int64_t n, int64_t K, int r
   BL_REQUIRE(dQ == nullptr || reinterpret_cast<uintptr_t>(dQ) % 16 == 0, "dQ must be 16-byte aligned");
   BL_REQUIRE(op->n == n, "operator size does not match n");
   BL_REQUIRE(ld <= (int64_t)align_up((size_t)n, 64), "ld must be at most n rounded up to 64");
-  cudaStream_t s = as_stream(stream);
-  if (dtype == BL_F32)
-    return arnoldi_adjoint_t<float>(op, dtype, n, (int)K, reortho_full, (const float*)Q, ld, (const float*)H,
-                                    (const float*)r, (const float*)c, (const float*)dQ, (const float*)dH,
-                                    (const float*)dr, (const float*)dc, (float*)dv, (float*)Lambda, workspace,
-                                    workspace_bytes, s);
-  return arnoldi_adjoint_t<double>(op, dtype, n, (int)K, reortho_full, (const double*)Q, ld, (const double*)H,
-                                   (const double*)r, (const double*)c, (const double*)dQ, (const double*)dH,
-                                   (const double*)dr, (const double*)dc, (double*)dv, (double*)Lambda, workspace,
-                                   workspace_bytes, s);
+  const auto run = dtype == BL_F32 ? arnoldi_adjoint_t<float> : arnoldi_adjoint_t<double>;
+  return run(op, dtype, n, (int)K, reortho_full, 1, Q, ld, H, r, c, dQ, dH, dr, dc, dv, n, Lambda, workspace,
+             workspace_bytes, as_stream(stream));
 }
 
 int bl_arnoldi_forward_batch(bl_operator_t* op, int dtype, int64_t n, int64_t K, int second_pass, int64_t count,
@@ -1683,12 +1548,10 @@ int bl_arnoldi_forward_batch(bl_operator_t* op, int dtype, int64_t n, int64_t K,
   BL_REQUIRE(op && v && Q && H && r && c && workspace && count >= 1 && count <= 4096 && ldv >= n, "bad batch arguments");
   BL_CHECK(check_basis(dtype, n, K, ld, Q));
   BL_REQUIRE(op->n == n, "operator size does not match n");
-  cudaStream_t s = as_stream(stream);
-  if (dtype == BL_F32)
-    return arnoldi_forward_batch_t<float>(op, dtype, n, (int)K, second_pass, (int)count, (const float*)v, ldv,
-                                          (float*)Q, ld, (float*)H, (float*)r, (float*)c, workspace, workspace_bytes, s);
-  return arnoldi_forward_batch_t<double>(op, dtype, n, (int)K, second_pass, (int)count, (const double*)v, ldv,
-                                         (double*)Q, ld, (double*)H, (double*)r, (double*)c, workspace, workspace_bytes, s);
+  const size_t per = bl_arnoldi_workspace_bytes(n, K, dtype);
+  BL_REQUIRE(workspace_bytes >= per * (size_t)count, "workspace too small (P * bl_arnoldi_workspace_bytes)");
+  const auto run = dtype == BL_F32 ? arnoldi_forward_t<float> : arnoldi_forward_t<double>;
+  return run(op, dtype, n, (int)K, second_pass, (int)count, v, ldv, Q, ld, H, r, c, workspace, per, as_stream(stream));
 }
 
 int bl_arnoldi_adjoint_batch(bl_operator_t* op, int dtype, int64_t n, int64_t K, int reortho_full, int64_t count,
@@ -1702,16 +1565,11 @@ int bl_arnoldi_adjoint_batch(bl_operator_t* op, int dtype, int64_t n, int64_t K,
   BL_REQUIRE(dQ == nullptr || reinterpret_cast<uintptr_t>(dQ) % 16 == 0, "dQ must be 16-byte aligned");
   BL_REQUIRE(op->n == n, "operator size does not match n");
   BL_REQUIRE(ld <= (int64_t)align_up((size_t)n, 64), "ld must be at most n rounded up to 64");
-  cudaStream_t s = as_stream(stream);
-  if (dtype == BL_F32)
-    return arnoldi_adjoint_batch_t<float>(op, dtype, n, (int)K, reortho_full, (int)count, (const float*)Q, ld,
-                                          (const float*)H, (const float*)r, (const float*)c, (const float*)dQ,
-                                          (const float*)dH, (const float*)dr, (const float*)dc, (float*)dv, lddv,
-                                          (float*)Lambda, workspace, workspace_bytes, s);
-  return arnoldi_adjoint_batch_t<double>(op, dtype, n, (int)K, reortho_full, (int)count, (const double*)Q, ld,
-                                         (const double*)H, (const double*)r, (const double*)c, (const double*)dQ,
-                                         (const double*)dH, (const double*)dr, (const double*)dc, (double*)dv, lddv,
-                                         (double*)Lambda, workspace, workspace_bytes, s);
+  const size_t per = bl_arnoldi_workspace_bytes(n, K, dtype);
+  BL_REQUIRE(workspace_bytes >= per * (size_t)count, "workspace too small (P * bl_arnoldi_workspace_bytes)");
+  const auto run = dtype == BL_F32 ? arnoldi_adjoint_t<float> : arnoldi_adjoint_t<double>;
+  return run(op, dtype, n, (int)K, reortho_full, (int)count, Q, ld, H, r, c, dQ, dH, dr, dc, dv, lddv, Lambda,
+             workspace, per, as_stream(stream));
 }
 
 #if defined(BL_STEP_DEBUG) || defined(BL_STEP_CYCLES)

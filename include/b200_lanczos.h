@@ -261,7 +261,9 @@ size_t bl_arnoldi_workspace_bytes(int64_t n, int64_t krylov_depth, int dtype);
 
 /* arnoldi._forward (arnoldi.py:57-101).  second_pass & BL_FWD_SECOND_PASS performs the second
  * Gram-Schmidt pass (`reortho_ != "none"`, arnoldi.py:91; the reference's default always
- * does, arnoldi.py:26).  Outputs: Q (K rows, ld), H (K x K), r (n), c (1 element = 1/||v||). */
+ * does, arnoldi.py:26).  Outputs: Q (K rows, ld), H (K x K), r (n), c (1 element = 1/||v||).
+ * Runs as bl_arnoldi_forward_batch with count = 1 and ldv = n; the workspace may be as small as what one run
+ * uses (bl_arnoldi_workspace_bytes is always enough). */
 int bl_arnoldi_forward(bl_operator_t* op, int dtype, int64_t n, int64_t krylov_depth, int second_pass,
                        const void* v, void* Q, int64_t ld, void* H, void* r, void* c,
                        void* workspace, size_t workspace_bytes, void* stream);
@@ -282,7 +284,8 @@ int bl_arnoldi_forward(bl_operator_t* op, int dtype, int64_t n, int64_t krylov_d
 /* arnoldi._adjoint (arnoldi.py:104-220).  reortho_full & BL_ADJ_REORTHO_FULL re-projects lambda
  * (`reortho == "full"`, arnoldi.py:201-204).  dQ (K rows, ld), dr, dc may be NULL (= zero
  * cotangent, the SLQ case of SURVEY 3.3).  Lambda is a K x ld scratch basis supplied by the
- * caller.  Output dv (n); parameter gradients accumulate in `op`. */
+ * caller.  Output dv (n); parameter gradients accumulate in `op`.  Runs as bl_arnoldi_adjoint_batch with
+ * count = 1 and lddv = n (same workspace rule as bl_arnoldi_forward). */
 int bl_arnoldi_adjoint(bl_operator_t* op, int dtype, int64_t n, int64_t krylov_depth, int reortho_full,
                        const void* Q, int64_t ld, const void* H, const void* r, const void* c,
                        const void* dQ, const void* dH, const void* dr, const void* dc, void* dv,
