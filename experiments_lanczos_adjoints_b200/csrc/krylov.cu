@@ -496,7 +496,7 @@ int launch_fused(const Common& c, const FusedSpec& f, int dtype, cudaStream_t s,
 }
 
 // Phase 1 of a symmetric-loop step (StepArgs below) as a launch of its own: out1 = (sum of <= kXTerms vector
-// terms) / div and red[j] = <row_j, out1> over the rows of src1 (k_xdots_tma, stream_kernels.cuh).  `*done` stays
+// terms) / div and red[j] = <row_j, out1> over the rows of src1 (k_xdots_tma, step_kernel.cuh).  `*done` stays
 // false when n is below the TMA threshold or the shape does not fit; the caller then runs its general kernels.
 template <typename T>
 int launch_xdots(const Common& c, const StepArgs& f, cudaStream_t s, bool* done) {
@@ -506,24 +506,16 @@ int launch_xdots(const Common& c, const StepArgs& f, cudaStream_t s, bool* done)
                       (size_t)f.nrows1 * 8 + 16;
   if (!use_tma(f.n) || f.nvec > kXTerms || f.nrows1 < 1 || smem > 112 * 1024) return BL_OK;
   *done = true;
-  XDotsArgs a;
-  a.src = f.src1;
-  a.nrows = f.nrows1;
-  a.n = f.n;
-  a.out = f.out1;
-  a.nvec = f.nvec;
-  for (int k = 0; k < f.nvec; ++k) a.vec[k] = f.vec[k];
-  a.out_div_ptr = f.out_div_ptr;
+  StepArgs a = f;
   a.partials = c.partials_dots;
-  a.counter = c.counters + 0;
-  a.epi = f.epi1;
   ShardedEpi se;
-  BL_CHECK(se.arm(c, a.epi, f.nrows1));
-  a.reverse = next_direction();
+  BL_CHECK(se.arm(c, a.epi1, f.nrows1));
+  const int reverse = next_direction();
   BL_CHECK(set_smem(k_xdots_tma<T, TILE>, 112 * 1024));
   {
     ProfScope prof(BL_PROF_FUSED, (double)(f.nrows1 + f.nvec + 1) * f.n * sizeof(T), s);
-    BL_CUDA(launch_pdl(k_xdots_tma<T, TILE>, tma_grid<T>(f.n, TILE), kStreamThreads, smem, s, a));
+    BL_CUDA(launch_pdl(k_xdots_tma<T, TILE>, tma_grid<T>(f.n, TILE), kStreamThreads, smem, s, a, c.counters + 0,
+                       reverse));
     BL_LAUNCHED();
   }
   return se.finish<T>(s);

@@ -8,12 +8,14 @@
 //   phase 2   out2 = out1 + sum_j c_j row_j  (+ ||out2||^2)             over the active rows      (k_combine_tma)
 //
 // with a grid-wide reduction between the phases whose result (Gram-Schmidt coefficients) the next phase needs.
-// As separate launches every reduction costs a kernel boundary (ramp, last-block pass, drain, launch: 8 us
-// against 2-60 us of streaming), and a run is a chain of 800 of them.  Here the phases run in one cooperative grid:
-// blocks meet at a counter in L2, every block (few values) or block j (value j, many values) reduces the per-block
-// partials in a fixed order, and EVERY block runs the epilogue on identical numbers (its global writes are
-// redundant and identical).  The TMA producer thread takes no part in the barriers: while the consumers wait it
-// fills the 96 KB ring with the next phase's rows.
+// Phases 1 and 2 run the same device code as k_xdots_tma and k_combine_tma: phase 1 of a run is step::xdots_run,
+// the body of k_xdots_tma (defined below), and phase 2 folds the staged groups in with fma_group and writes out2
+// with store_colvec, as k_combine_tma does.  As separate launches every reduction costs a kernel boundary (ramp,
+// last-block pass, drain, launch: 8 us against 2-60 us of streaming), and a run is a chain of 800 of them.  Here
+// the phases run in one cooperative grid: blocks meet at a counter in L2, every block (few values) or block j
+// (value j, many values) reduces the per-block partials in a fixed order, and EVERY block runs the epilogue on
+// identical numbers (its global writes are redundant and identical).  The TMA producer thread takes no part in the
+// barriers: while the consumers wait it fills the 96 KB ring with the next phase's rows.
 //
 // Measured (block 0's time stamps, bl_step_trace_*), an in-kernel reduction costs ~6 us -- no less than a kernel
 // boundary with programmatic dependent launch.  What pays is the BATCH: the lockstep drivers
@@ -39,6 +41,7 @@
 namespace bl {
 
 constexpr int kFewMax = 4;
+constexpr int kXTerms = 10;
 constexpr int kStepBatch = 4;
 constexpr int kFewSlots = kFewMax * kConsumerWarps + 8;  // per-run scratch of phase 0: warp partials, then block values
 
@@ -580,15 +583,183 @@ __device__ __forceinline__ void few_dots_local(const StepBatch& B, const ColumnR
   csync();
 }
 
+// Phase 1 of one run, consumer side: out1 = (sum of the terms) / div, written to out1 and to the x tile, and
+// acc[j] += <row j of src1, out1> over the block's tiles.  Thread t holds column vector t of every term, loaded a
+// tile ahead; the rows come through the ring from the producer.  `it` (ring position) and `xt` (x-tile buffer) run
+// on across runs.  IN_STEP: inside k_step_tma, where blocks of the same launch wrote the coefficients, so they are
+// read through L2, and where the debug hooks record; p is the run's index there.
+template <typename T, int TILE, bool IN_STEP>
+__device__ __forceinline__ void xdots_run(const StepArgs& a, const ColumnRange& cr, int reverse, const T* stages,
+                                          T* xs, uint64_t* full, uint64_t* empty, int& it, int& xt, double* acc_p,
+                                          int p) {
+  using V = typename Vec<T>::type;
+  constexpr int VN = Vec<T>::N;
+  constexpr int XV = TILE / (32 * VN);  // x vectors per lane
+  static_assert(TILE == kConsumerThreads * VN, "one 16-byte column vector per consumer thread");
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const long long n = a.n;
+  const int nrows1 = a.nrows1;
+  const int ngroups1 = (nrows1 + kGroup - 1) / kGroup;
+  T cv[kXTerms];
+#pragma unroll
+  for (int v = 0; v < kXTerms; ++v) {
+    const double* cp = a.vec[v].coef_ptr;
+    cv[v] = v < a.nvec ? static_cast<T>(a.vec[v].coef_imm * (cp ? (IN_STEP ? __ldcg(cp) : *cp) : 1.0)) : T(0);
+  }
+  const T oscale = a.out_div_ptr ? static_cast<T>(IN_STEP ? __ldcg(a.out_div_ptr) : *a.out_div_ptr) : T(1);
+#ifdef BL_STEP_DEBUG
+#pragma unroll
+  for (int v = 0; v < kXTerms; ++v) BL_DBG(IN_STEP && tid == 0 && dbg_bad(cv[v]), 7, p, a.epi0.i, v, (double)cv[v], (double)oscale);
+  BL_DBG(IN_STEP && tid == 0 && (dbg_bad(oscale) || oscale == T(0)), 7, p, a.epi0.i, 99, (double)oscale, 0.0);
+#endif
+  V term[kXTerms];
+  auto load_terms = [&](int tt) {
+    const int t = reverse ? cr.ntiles - 1 - tt : tt;
+    const long long c = cr.c0 + (long long)t * TILE + (long long)tid * VN;
+    const bool live = tt < cr.ntiles && c < cr.c1;
+#pragma unroll
+    for (int v = 0; v < kXTerms; ++v)
+      term[v] = load_colvec(static_cast<const T*>(a.vec[v].ptr), c, n, live && v < a.nvec);
+  };
+  load_terms(0);
+  for (int tt = 0; tt < cr.ntiles; ++tt, ++xt) {
+    const int t = reverse ? cr.ntiles - 1 - tt : tt;
+    const long long tc0 = cr.c0 + (long long)t * TILE;
+    const int len = (int)((cr.c1 - tc0) < TILE ? (cr.c1 - tc0) : TILE);
+    const bool live = tid * VN < len;
+    T* x = xs + (size_t)(xt & 1) * TILE;
+    {  // ---- build this thread's vector of the x tile ----
+      T acc[VN];
+#pragma unroll
+      for (int k = 0; k < VN; ++k) acc[k] = T(0);
+#pragma unroll
+      for (int v = 0; v < kXTerms; ++v) {
+        if (v < a.nvec) {
+          T e[VN];
+          vec_unpack(term[v], e);
+#pragma unroll
+          for (int k = 0; k < VN; ++k) {
+            BL_DBG(IN_STEP && dbg_bad(e[k]), 8, p, a.epi0.i, v * 100000000ll + tc0 + tid * VN + k, (double)e[k], (double)cv[v]);
+            acc[k] = fma(cv[v], e[k], acc[k]);
+          }
+        }
+      }
+      const long long c = tc0 + (long long)tid * VN;
+#pragma unroll
+      for (int k = 0; k < VN; ++k) acc[k] = live && c + k < n ? acc[k] / oscale : T(0);
+      reinterpret_cast<V*>(x)[tid] = vec_pack(acc);
+      if (live) store_colvec(static_cast<T*>(a.out1), c, n, acc);
+    }
+    load_terms(tt + 1);  // in flight while this tile's rows are consumed (in place: own columns only)
+    tma::named_bar_sync(1, kConsumerThreads);
+    V xr[XV];
+#pragma unroll
+    for (int u = 0; u < XV; ++u) xr[u] = reinterpret_cast<const V*>(x)[lane + 32 * u];
+    for (int gg = 0; gg < ngroups1; ++gg, ++it) {
+      const int g = reverse ? ngroups1 - 1 - gg : gg;
+      const int s = it % kStages;
+      tma::mbar_wait(full + s, (it / kStages) & 1);
+      const int j = g * kGroup + warp;
+      if (j < nrows1) {
+        const V* row = reinterpret_cast<const V*>(stages + ((size_t)s * kGroup + warp) * TILE);
+        T a0 = T(0), a1 = T(0);
+#pragma unroll
+        for (int u = 0; u < XV; ++u) {
+          if ((lane + 32 * u) * VN < len) {
+            T q[VN], xx[VN];
+            vec_unpack(row[lane + 32 * u], q);
+            vec_unpack(xr[u], xx);
+#ifdef BL_STEP_DEBUG
+#pragma unroll
+            for (int k = 0; k < VN; ++k) {
+              BL_DBG(IN_STEP && dbg_bad(q[k]), 9, p, a.epi0.i, j * 100000000ll + tc0 + (lane + 32 * u) * VN + k, (double)q[k], (double)s);
+              BL_DBG(IN_STEP && dbg_bad(xx[k]), 10, p, a.epi0.i, j * 100000000ll + tc0 + (lane + 32 * u) * VN + k, (double)xx[k], 0.0);
+            }
+#endif
+#pragma unroll
+            for (int k = 0; k < VN; ++k) {
+              if (u & 1)
+                a1 = fma(q[k], xx[k], a1);
+              else
+                a0 = fma(q[k], xx[k], a0);
+            }
+          }
+        }
+        __syncwarp();
+        if (lane == 0) tma::mbar_arrive(empty + s);
+        double sacc = warp_sum(static_cast<double>(a0) + static_cast<double>(a1));
+        if (lane == 0) acc_p[j] += sacc;  // row j is always handled by this warp: no race
+      } else {
+        __syncwarp();
+        if (lane == 0) tma::mbar_arrive(empty + s);
+      }
+    }
+  }
+}
+
 }  // namespace step
+
+// ---------------------------------------------------------------------------------------------
+// Phase 1 of a step as a launch of its own: out1 = (sum_k a_k vec_k) / div  AND  red[j] = <row_j, out1>.  k_dots_tma
+// whose x tile is BUILT by the consumers instead of loaded.  The symmetric Krylov loops combine a handful of vectors
+// (<= kXTerms: the iterate, two to five neighbouring basis rows, r, z, two rows of Lambda) and then need the dots of
+// the result with every active basis row -- no row is used twice, so nothing has to stay resident (k_fused_tma's
+// double-buffered [rows x 128] tiles and its two-sweep hand-over per tile go away) and the rows stream through the
+// same 4 KB x 8 x 3 ring as in k_dots_tma.  Only the phase-1 fields of `a` are read; a.partials is the [nrows1][grid]
+// area of the block shares.
+template <typename T, int TILE>
+__global__ void __launch_bounds__(kStreamThreads, 2)
+k_xdots_tma(const __grid_constant__ StepArgs a, unsigned int* counter, int reverse) {
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  T* stages = reinterpret_cast<T*>(smem_raw);                       // [kStages][kGroup][TILE]
+  T* xs = stages + (size_t)kStages * kGroup * TILE;                 // [2][TILE]
+  uint64_t* full = reinterpret_cast<uint64_t*>(xs + 2 * TILE);
+  uint64_t* empty = full + kStages;
+  double* acc_s = reinterpret_cast<double*>(empty + kStages + 2);   // [nrows1]
+
+  const int nrows = a.nrows1;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < kStages; ++s) {
+      tma::mbar_init(full + s, 1);
+      tma::mbar_init(empty + s, kConsumerWarps);
+    }
+    tma::fence_barrier_init();
+  }
+  for (int j = threadIdx.x; j < nrows; j += blockDim.x) acc_s[j] = 0.0;
+  __syncthreads();
+  tma::griddep_launch_dependents();
+
+  const ColumnRange cr = block_columns<T>(a.n, TILE);
+  const int ngroups = (nrows + kGroup - 1) / kGroup;
+
+  if (warp == kConsumerWarps) {
+    if (lane == 0) {  // ---- producer: basis rows only (older than the predecessor: no griddepcontrol.wait) ----
+      const int total = cr.ntiles * ngroups;
+      for (int it = 0; it < total; ++it) {
+        const int tt = it / ngroups, gg = it - tt * ngroups;
+        const int t = reverse ? cr.ntiles - 1 - tt : tt;
+        const long long tc0 = cr.c0 + (long long)t * TILE;
+        const int len = (int)((cr.c1 - tc0) < TILE ? (cr.c1 - tc0) : TILE);
+        stage_rows<T, TILE>(stages, full, empty, it, a.src1, reverse ? ngroups - 1 - gg : gg, nrows, tc0, len);
+      }
+    }
+  } else {
+    tma::griddep_wait();  // the terms and their coefficients are the predecessor's output
+    int it = 0, xt = 0;
+    step::xdots_run<T, TILE, false>(a, cr, reverse, stages, xs, full, empty, it, xt, acc_s, 0);
+  }
+  __syncthreads();
+  for (int j = threadIdx.x; j < nrows; j += blockDim.x) a.partials[(size_t)j * gridDim.x + blockIdx.x] = acc_s[j];
+  if (!last_block_done(counter)) return;
+  reduce_partials_and_epilogue<T>(nrows, a.partials, a.epi1);
+}
 
 template <typename T, int TILE>
 __global__ void __launch_bounds__(kStreamThreads, 2)
 k_step_tma(const __grid_constant__ StepBatch B) {
   using V = typename Vec<T>::type;
   constexpr int VN = Vec<T>::N;
-  constexpr int XV = TILE / (32 * VN);  // x vectors per lane
-  static_assert(TILE == kConsumerThreads * VN, "one 16-byte column vector per consumer thread");
   extern __shared__ __align__(128) unsigned char smem_raw[];
   T* stages = reinterpret_cast<T*>(smem_raw);                       // [kStages][kGroup][TILE]
   T* xs = stages + (size_t)kStages * kGroup * TILE;                 // [2][TILE]
@@ -634,7 +805,6 @@ k_step_tma(const __grid_constant__ StepBatch B) {
 
   if (warp == kConsumerWarps) {
     if (lane == 0) {  // ---- producer: the rows of phase 1 of every run, then the rows of phase 2, one ring ----
-      const uint64_t pol_first = tma::policy_evict_first();
       bool waited = false;
       bool gated = !with_op;  // with the operator in the launch the ring belongs to phase S first
       int it = 0;
@@ -672,7 +842,6 @@ k_step_tma(const __grid_constant__ StepBatch B) {
             const int t = dir ? cr.ntiles - 1 - tt : tt;
             const long long tc0 = cr.c0 + (long long)t * TILE;
             const int len = (int)((cr.c1 - tc0) < TILE ? (cr.c1 - tc0) : TILE);
-            const uint32_t bytes = (uint32_t)len * sizeof(T);
             for (int gg = 0; gg < ngroups; ++gg, ++it) {
               const int g = dir ? ngroups - 1 - gg : gg;
               const int rows_here = nrows - g * kGroup < kGroup ? nrows - g * kGroup : kGroup;
@@ -684,13 +853,7 @@ k_step_tma(const __grid_constant__ StepBatch B) {
                 tma::griddep_wait();
                 waited = true;
               }
-              const int s = it % kStages;
-              tma::mbar_wait(empty + s, ((it / kStages) & 1) ^ 1);
-              tma::mbar_arrive_expect_tx(full + s, bytes * rows_here);
-              T* dst = stages + (size_t)s * kGroup * TILE;
-              for (int r = 0; r < rows_here; ++r)
-                tma::bulk_g2s_hint(dst + (size_t)r * TILE, src.row(g * kGroup + r) + tc0 * (long long)sizeof(T), bytes,
-                                   full + s, pol_first);
+              stage_rows<T, TILE>(stages, full, empty, it, src, g, nrows, tc0, len);
             }
           }
         }
@@ -704,7 +867,6 @@ k_step_tma(const __grid_constant__ StepBatch B) {
     step::stamp(B.trace_slot, 1, tid);
 
     // ================= phase S: x0 = A x, every run (the operator call of the step) =================
-    int it0 = 0;
     if (with_op) {
       if (B.op.norm)
         step::op_phase_dispatch<T, true>(B, orng, smem_raw, op_full, op_empty, warp, lane);
@@ -742,131 +904,9 @@ k_step_tma(const __grid_constant__ StepBatch B) {
     if (with_op) tma::griddep_launch_dependents();
 
     // ================= phase 1: out1 = (sum of terms) / div, red1[j] = <row_j, out1>, every run =================
-    int it = it0, xt = 0;
-    for (int p = 0; p < P; ++p) {
-      const StepArgs& a = B.a[p];
-      const int nrows1 = a.nrows1;
-      const int ngroups1 = (nrows1 + kGroup - 1) / kGroup;
-      double* acc_p = acc_s + (size_t)p * B.acc_stride;
-      T cv[kXTerms];
-#pragma unroll
-      for (int v = 0; v < kXTerms; ++v)
-        cv[v] = v < a.nvec ? static_cast<T>(a.vec[v].coef_imm * (a.vec[v].coef_ptr ? __ldcg(a.vec[v].coef_ptr) : 1.0)) : T(0);
-      const T oscale = a.out_div_ptr ? static_cast<T>(__ldcg(a.out_div_ptr)) : T(1);
-#ifdef BL_STEP_DEBUG
-#pragma unroll
-      for (int v = 0; v < kXTerms; ++v) BL_DBG(tid == 0 && dbg_bad(cv[v]), 7, p, a.epi0.i, v, (double)cv[v], (double)oscale);
-      BL_DBG(tid == 0 && (dbg_bad(oscale) || oscale == T(0)), 7, p, a.epi0.i, 99, (double)oscale, 0.0);
-#endif
-      V term[kXTerms];
-      auto load_terms = [&](int tt) {  // this thread's vector of every term, tile tt (columns past n read as zero)
-        const int t = dir1 ? cr.ntiles - 1 - tt : tt;
-        const long long c = cr.c0 + (long long)t * TILE + (long long)tid * VN;
-        const bool inside = tt < cr.ntiles && c < cr.c1 && c + VN <= n;
-#pragma unroll
-        for (int v = 0; v < kXTerms; ++v) {
-          T z[VN];
-#pragma unroll
-          for (int k = 0; k < VN; ++k) z[k] = T(0);
-          if (v < a.nvec) {
-            const T* ptr = static_cast<const T*>(a.vec[v].ptr) + c;
-            if (inside) {
-              term[v] = *reinterpret_cast<const V*>(ptr);
-              continue;
-            }
-            if (tt < cr.ntiles && c < cr.c1)  // the vector that straddles n
-#pragma unroll
-              for (int k = 0; k < VN; ++k)
-                if (c + k < n) z[k] = ptr[k];
-          }
-          term[v] = vec_pack(z);
-        }
-      };
-      load_terms(0);
-      for (int tt = 0; tt < cr.ntiles; ++tt, ++xt) {
-        const int t = dir1 ? cr.ntiles - 1 - tt : tt;
-        const long long tc0 = cr.c0 + (long long)t * TILE;
-        const int len = (int)((cr.c1 - tc0) < TILE ? (cr.c1 - tc0) : TILE);
-        const int b = xt & 1;
-        {  // ---- build this thread's vector of the x tile ----
-          T acc[VN];
-#pragma unroll
-          for (int k = 0; k < VN; ++k) acc[k] = T(0);
-#pragma unroll
-          for (int v = 0; v < kXTerms; ++v) {
-            if (v < a.nvec) {
-              T e[VN];
-              vec_unpack(term[v], e);
-#pragma unroll
-              for (int k = 0; k < VN; ++k) {
-                BL_DBG(dbg_bad(e[k]), 8, p, a.epi0.i, v * 100000000ll + tc0 + tid * VN + k, (double)e[k], (double)cv[v]);
-                acc[k] = fma(cv[v], e[k], acc[k]);
-              }
-            }
-          }
-          const long long c = tc0 + (long long)tid * VN;
-          bool all_ok = true;
-#pragma unroll
-          for (int k = 0; k < VN; ++k) {
-            const bool ok = tid * VN + k < len && c + k < n;
-            acc[k] = ok ? acc[k] / oscale : T(0);
-            all_ok = all_ok && ok;
-          }
-          reinterpret_cast<V*>(xs + (size_t)b * TILE)[tid] = vec_pack(acc);
-          if (all_ok) {
-            *reinterpret_cast<V*>(static_cast<T*>(a.out1) + c) = vec_pack(acc);
-          } else {
-#pragma unroll
-            for (int k = 0; k < VN; ++k)
-              if (tid * VN + k < len && c + k < n) static_cast<T*>(a.out1)[c + k] = acc[k];
-          }
-        }
-        load_terms(tt + 1);  // in flight while this tile's rows are consumed (in place: own columns only)
-        csync();
-        V xr[XV];
-#pragma unroll
-        for (int u = 0; u < XV; ++u) xr[u] = reinterpret_cast<const V*>(xs + (size_t)b * TILE)[lane + 32 * u];
-        for (int gg = 0; gg < ngroups1; ++gg, ++it) {
-          const int g = dir1 ? ngroups1 - 1 - gg : gg;
-          const int s = it % kStages;
-          tma::mbar_wait(full + s, (it / kStages) & 1);
-          const int j = g * kGroup + warp;
-          if (j < nrows1) {
-            const V* row = reinterpret_cast<const V*>(stages + ((size_t)s * kGroup + warp) * TILE);
-            T a0 = T(0), a1 = T(0);
-#pragma unroll
-            for (int u = 0; u < XV; ++u) {
-              if ((lane + 32 * u) * VN < len) {
-                T q[VN], xx[VN];
-                vec_unpack(row[lane + 32 * u], q);
-                vec_unpack(xr[u], xx);
-#ifdef BL_STEP_DEBUG
-#pragma unroll
-                for (int k = 0; k < VN; ++k) {
-                  BL_DBG(dbg_bad(q[k]), 9, p, a.epi0.i, j * 100000000ll + tc0 + (lane + 32 * u) * VN + k, (double)q[k], (double)s);
-                  BL_DBG(dbg_bad(xx[k]), 10, p, a.epi0.i, j * 100000000ll + tc0 + (lane + 32 * u) * VN + k, (double)xx[k], 0.0);
-                }
-#endif
-#pragma unroll
-                for (int k = 0; k < VN; ++k) {
-                  if (u & 1)
-                    a1 = fma(q[k], xx[k], a1);
-                  else
-                    a0 = fma(q[k], xx[k], a0);
-                }
-              }
-            }
-            __syncwarp();
-            if (lane == 0) tma::mbar_arrive(empty + s);
-            double sacc = warp_sum(static_cast<double>(a0) + static_cast<double>(a1));
-            if (lane == 0) acc_p[j] += sacc;  // row j is always handled by this warp: no race
-          } else {
-            __syncwarp();
-            if (lane == 0) tma::mbar_arrive(empty + s);
-          }
-        }
-      }
-    }
+    int it = 0, xt = 0;
+    for (int p = 0; p < P; ++p)
+      step::xdots_run<T, TILE, true>(B.a[p], cr, dir1, stages, xs, full, empty, it, xt, acc_s + (size_t)p * B.acc_stride, p);
     csync();
     step::stamp(B.trace_slot, 4, tid);
     step::grid_reduce<1>(B, acc_s, 0, tid);
@@ -895,20 +935,10 @@ k_step_tma(const __grid_constant__ StepBatch B) {
       const int nrows2 = a.nrows2;
       const int ngroups2 = (nrows2 + kGroup - 1) / kGroup;
       const T* coef_p = coef_s + (size_t)p * B.coef_stride;
-      auto load_x = [&](int tt) -> V {  // out1 as this very thread wrote it in phase 1
-        T z[VN];
-#pragma unroll
-        for (int k = 0; k < VN; ++k) z[k] = T(0);
-        if (tt < cr.ntiles) {
-          const int t = dir2 ? cr.ntiles - 1 - tt : tt;
-          const long long c = cr.c0 + (long long)t * TILE + (long long)tid * VN;
-          if (c < cr.c1 && c + VN <= n) return *reinterpret_cast<const V*>(static_cast<const T*>(a.out1) + c);
-          if (c < cr.c1)
-#pragma unroll
-            for (int k = 0; k < VN; ++k)
-              if (c + k < n) z[k] = static_cast<const T*>(a.out1)[c + k];
-        }
-        return vec_pack(z);
+      auto load_x = [&](int tt) {  // out1 as this very thread wrote it in phase 1
+        const int t = dir2 ? cr.ntiles - 1 - tt : tt;
+        const long long c = cr.c0 + (long long)t * TILE + (long long)tid * VN;
+        return load_colvec(static_cast<const T*>(a.out1), c, n, tt < cr.ntiles && c < cr.c1);
       };
       V xnext = load_x(0);
       for (int tt = 0; tt < cr.ntiles; ++tt) {
@@ -917,7 +947,6 @@ k_step_tma(const __grid_constant__ StepBatch B) {
         const int len = (int)((cr.c1 - tc0) < TILE ? (cr.c1 - tc0) : TILE);
         const long long col = tc0 + (long long)tid * VN;
         const bool live = tid * VN < len;
-        const bool fullvec = live && col + VN <= n;
         T acc[VN];
         vec_unpack(xnext, acc);
         xnext = load_x(tt + 1);
@@ -926,29 +955,9 @@ k_step_tma(const __grid_constant__ StepBatch B) {
           const int s = it % kStages;
           tma::mbar_wait(full + s, (it / kStages) & 1);
           const int rows_here = nrows2 - g * kGroup < kGroup ? nrows2 - g * kGroup : kGroup;
-          if (live) {
-            const V* st = reinterpret_cast<const V*>(stages + (size_t)s * kGroup * TILE) + tid;
-            const T* cf = coef_p + g * kGroup;
-            if (rows_here == kGroup) {
-              V q[kGroup];
-#pragma unroll
-              for (int r = 0; r < kGroup; ++r) q[r] = st[(size_t)r * (TILE / VN)];
-#pragma unroll
-              for (int r = 0; r < kGroup; ++r) {
-                T e[VN];
-                vec_unpack(q[r], e);
-#pragma unroll
-                for (int k = 0; k < VN; ++k) acc[k] = fma(cf[r], e[k], acc[k]);
-              }
-            } else {
-              for (int r = 0; r < rows_here; ++r) {
-                T e[VN];
-                vec_unpack(st[(size_t)r * (TILE / VN)], e);
-#pragma unroll
-                for (int k = 0; k < VN; ++k) acc[k] = fma(cf[r], e[k], acc[k]);
-              }
-            }
-          }
+          if (live)
+            fma_group<T, TILE>(reinterpret_cast<const V*>(stages + (size_t)s * kGroup * TILE) + tid, coef_p + g * kGroup,
+                               rows_here, acc);
           __syncwarp();
           if (lane == 0) tma::mbar_arrive(empty + s);
         }
@@ -958,13 +967,7 @@ k_step_tma(const __grid_constant__ StepBatch B) {
             for (int k = 0; k < VN; ++k)
               if (col + k < n) ss += static_cast<double>(acc[k] * acc[k]);
           }
-          if (fullvec) {
-            *reinterpret_cast<V*>(static_cast<T*>(a.out2) + col) = vec_pack(acc);
-          } else {
-#pragma unroll
-            for (int k = 0; k < VN; ++k)
-              if (col + k < n) static_cast<T*>(a.out2)[col + k] = acc[k];
-          }
+          store_colvec(static_cast<T*>(a.out2), col, n, acc);
         }
       }
       if (a.norm) {  // acc_s is free by now: warp sums of ||out2||^2, added up at the exit

@@ -61,6 +61,79 @@ __device__ __forceinline__ ColumnRange block_columns(long long n, int tile) {
   return r;
 }
 
+// This thread's column vector of p at column c, when `live`; zero otherwise.  Vectors of length n are not zero-padded:
+// the one that straddles n is read element by element, its elements past n as zero.
+template <typename T>
+__device__ __forceinline__ typename Vec<T>::type load_colvec(const T* p, long long c, long long n, bool live) {
+  constexpr int VN = Vec<T>::N;
+  if (live && c + VN <= n) return *reinterpret_cast<const typename Vec<T>::type*>(p + c);
+  T z[VN];
+#pragma unroll
+  for (int k = 0; k < VN; ++k) z[k] = T(0);
+  if (live)
+#pragma unroll
+    for (int k = 0; k < VN; ++k)
+      if (c + k < n) z[k] = p[c + k];
+  return vec_pack(z);
+}
+
+// Stores this thread's column vector at column c of p; of the vector that straddles n, only the elements before n.
+template <typename T>
+__device__ __forceinline__ void store_colvec(T* p, long long c, long long n, const T (&v)[Vec<T>::N]) {
+  constexpr int VN = Vec<T>::N;
+  if (c + VN <= n) {
+    *reinterpret_cast<typename Vec<T>::type*>(p + c) = vec_pack(v);
+  } else {
+#pragma unroll
+    for (int k = 0; k < VN; ++k)
+      if (c + k < n) p[c + k] = v[k];
+  }
+}
+
+// Producer: group g of the rows [0, nrows) of src, columns [tc0, tc0 + len), into ring stage it % kStages once the
+// consumers have released it.
+template <typename T, int TILE>
+__device__ __forceinline__ void stage_rows(T* stages, uint64_t* full, uint64_t* empty, int it, const RowSource& src,
+                                           int g, int nrows, long long tc0, int len) {
+  const uint32_t bytes = (uint32_t)len * sizeof(T);
+  const int rows_here = nrows - g * kGroup < kGroup ? nrows - g * kGroup : kGroup;
+  const int s = it % kStages;
+  tma::mbar_wait(empty + s, ((it / kStages) & 1) ^ 1);
+  tma::mbar_arrive_expect_tx(full + s, bytes * rows_here);
+  T* dst = stages + (size_t)s * kGroup * TILE;
+  const uint64_t pol = tma::policy_evict_first();
+  for (int r = 0; r < rows_here; ++r)
+    tma::bulk_g2s_hint(dst + (size_t)r * TILE, src.row(g * kGroup + r) + tc0 * (long long)sizeof(T), bytes, full + s,
+                       pol);
+}
+
+// acc += sum_r cf[r] * (row r of a staged group) for this thread's column vector (st: its vector of row 0): a full
+// group with all loads first.
+template <typename T, int TILE>
+__device__ __forceinline__ void fma_group(const typename Vec<T>::type* st, const T* cf, int rows, T (&acc)[Vec<T>::N]) {
+  using V = typename Vec<T>::type;
+  constexpr int VN = Vec<T>::N;
+  if (rows == kGroup) {
+    V q[kGroup];
+#pragma unroll
+    for (int r = 0; r < kGroup; ++r) q[r] = st[(size_t)r * (TILE / VN)];
+#pragma unroll
+    for (int r = 0; r < kGroup; ++r) {
+      T e[VN];
+      vec_unpack(q[r], e);
+#pragma unroll
+      for (int k = 0; k < VN; ++k) acc[k] = fma(cf[r], e[k], acc[k]);
+    }
+  } else {
+    for (int r = 0; r < rows; ++r) {
+      T e[VN];
+      vec_unpack(st[(size_t)r * (TILE / VN)], e);
+#pragma unroll
+      for (int k = 0; k < VN; ++k) acc[k] = fma(cf[r], e[k], acc[k]);
+    }
+  }
+}
+
 // Fixed-order cross-block reduction + epilogue, run by the last block (all threads call it).
 // Latency-bound (one block reads gridDim.x * nrows doubles from L2), so every lane issues all of
 // its loads for two rows before the first add: <= 10 independent 16-byte loads in flight.
@@ -176,15 +249,7 @@ k_dots_tma(RowSource src, int nrows, const T* __restrict__ x, long long n, doubl
         const int g = reverse ? ngroups - 1 - gg : gg;
         const long long tc0 = cr.c0 + (long long)t * TILE;
         const int len = (int)((cr.c1 - tc0) < TILE ? (cr.c1 - tc0) : TILE);
-        const uint32_t bytes = (uint32_t)len * sizeof(T);
-        const int s = it % kStages;
-        tma::mbar_wait(empty + s, ((it / kStages) & 1) ^ 1);
-        const int rows_here = nrows - g * kGroup < kGroup ? nrows - g * kGroup : kGroup;
-        tma::mbar_arrive_expect_tx(full + s, bytes * rows_here);
-        T* dst = stages + (size_t)s * kGroup * TILE;
-        for (int r = 0; r < rows_here; ++r)
-          tma::bulk_g2s_hint(dst + (size_t)r * TILE, src.row(g * kGroup + r) + tc0 * (long long)sizeof(T), bytes, full + s,
-                             tma::policy_evict_first());
+        stage_rows<T, TILE>(stages, full, empty, it, src, g, nrows, tc0, len);
       }
       if (!waited && total > 0) {
         tma::griddep_wait();
@@ -262,15 +327,6 @@ k_dots_tma(RowSource src, int nrows, const T* __restrict__ x, long long n, doubl
   reduce_partials_and_epilogue<T>(nrows, partials, epi);
 }
 
-// ---------------------------------------------------------------------------------------------
-// out = (sum_k a_k vec_k) / div  AND  red[j] = <row_j, out>: k_dots_tma whose x tile is BUILT by the consumers
-// instead of loaded.  The symmetric Krylov loops combine a handful of vectors (<= kXTerms: the iterate, two to
-// five neighbouring basis rows, r, z, two rows of Lambda) and then need the dots of the result with every active
-// basis row -- no row is used twice, so nothing has to stay resident (k_fused_tma's double-buffered [rows x 128]
-// tiles and its two-sweep hand-over per tile go away) and the rows stream through the same 4 KB x 8 x 3 ring as
-// in k_dots_tma.  Thread t of the 256 consumers owns one 16-byte column vector of the tile: it holds that vector
-// of every term in registers (loaded one tile ahead: only tile 0's loads are exposed, and they depend on the
-// predecessor anyway), writes the combined vector to `out` and to the shared x tile.
 namespace step {
 // fixed-order sum of one row of per-block partials by one warp; all loads of a lane are issued before the adds
 __device__ __forceinline__ double row_sum(const double* __restrict__ p, int G, int lane) {
@@ -294,187 +350,6 @@ __device__ __forceinline__ double row_sum(const double* __restrict__ p, int G, i
 }
 
 }  // namespace step
-
-constexpr int kXTerms = 10;
-
-struct XDotsArgs {
-  RowSource src;
-  int nrows = 0;
-  long long n = 0;
-  void* out = nullptr;
-  int nvec = 0;
-  VecTerm vec[kXTerms];
-  const double* out_div_ptr = nullptr;
-  double* partials = nullptr;
-  unsigned int* counter = nullptr;
-  Epi epi;
-  int reverse = 0;
-};
-
-template <typename T, int TILE>
-__global__ void __launch_bounds__(kStreamThreads, 2)
-k_xdots_tma(const __grid_constant__ XDotsArgs a) {
-  using V = typename Vec<T>::type;
-  constexpr int VN = Vec<T>::N;
-  constexpr int XV = TILE / (32 * VN);  // x vectors per lane
-  static_assert(TILE == kConsumerThreads * VN, "one 16-byte column vector per consumer thread");
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  T* stages = reinterpret_cast<T*>(smem_raw);                       // [kStages][kGroup][TILE]
-  T* xs = stages + (size_t)kStages * kGroup * TILE;                 // [2][TILE]
-  uint64_t* full = reinterpret_cast<uint64_t*>(xs + 2 * TILE);
-  uint64_t* empty = full + kStages;
-  double* acc_s = reinterpret_cast<double*>(empty + kStages + 2);   // [nrows]
-
-  const int nrows = a.nrows, reverse = a.reverse;
-  const long long n = a.n;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < kStages; ++s) {
-      tma::mbar_init(full + s, 1);
-      tma::mbar_init(empty + s, kConsumerWarps);
-    }
-    tma::fence_barrier_init();
-  }
-  for (int j = threadIdx.x; j < nrows; j += blockDim.x) acc_s[j] = 0.0;
-  __syncthreads();
-  tma::griddep_launch_dependents();
-
-  const ColumnRange cr = block_columns<T>(n, TILE);
-  const int ngroups = (nrows + kGroup - 1) / kGroup;
-
-  if (warp == kConsumerWarps) {
-    if (lane == 0) {  // ---- producer: basis rows only (older than the predecessor: no griddepcontrol.wait) ----
-      const int total = cr.ntiles * ngroups;
-      for (int it = 0; it < total; ++it) {
-        const int tt = it / ngroups, gg = it - tt * ngroups;
-        const int t = reverse ? cr.ntiles - 1 - tt : tt;
-        const int g = reverse ? ngroups - 1 - gg : gg;
-        const long long tc0 = cr.c0 + (long long)t * TILE;
-        const int len = (int)((cr.c1 - tc0) < TILE ? (cr.c1 - tc0) : TILE);
-        const uint32_t bytes = (uint32_t)len * sizeof(T);
-        const int s = it % kStages;
-        tma::mbar_wait(empty + s, ((it / kStages) & 1) ^ 1);
-        const int rows_here = nrows - g * kGroup < kGroup ? nrows - g * kGroup : kGroup;
-        tma::mbar_arrive_expect_tx(full + s, bytes * rows_here);
-        T* dst = stages + (size_t)s * kGroup * TILE;
-        for (int r = 0; r < rows_here; ++r)
-          tma::bulk_g2s_hint(dst + (size_t)r * TILE, a.src.row(g * kGroup + r) + tc0 * (long long)sizeof(T), bytes,
-                             full + s, tma::policy_evict_first());
-      }
-    }
-  } else {
-    const int tid = threadIdx.x;  // 0..255: column vector tid of every tile
-    tma::griddep_wait();          // the terms and their coefficients are the predecessor's output
-    T cv[kXTerms];
-#pragma unroll
-    for (int v = 0; v < kXTerms; ++v)
-      cv[v] = v < a.nvec ? static_cast<T>(a.vec[v].coef_imm * (a.vec[v].coef_ptr ? *a.vec[v].coef_ptr : 1.0)) : T(0);
-    const T oscale = a.out_div_ptr ? static_cast<T>(*a.out_div_ptr) : T(1);
-    V term[kXTerms];
-    auto load_terms = [&](int tt) {  // this thread's vector of every term, tile tt (columns past n read as zero)
-      const int t = reverse ? cr.ntiles - 1 - tt : tt;
-      const long long c = cr.c0 + (long long)t * TILE + (long long)tid * VN;
-      const bool inside = tt < cr.ntiles && c < cr.c1 && c + VN <= n;
-#pragma unroll
-      for (int v = 0; v < kXTerms; ++v) {
-        T z[VN];
-#pragma unroll
-        for (int k = 0; k < VN; ++k) z[k] = T(0);
-        if (v < a.nvec) {
-          const T* p = static_cast<const T*>(a.vec[v].ptr) + c;
-          if (inside) {
-            term[v] = *reinterpret_cast<const V*>(p);
-            continue;
-          }
-          if (tt < cr.ntiles && c < cr.c1)  // the vector that straddles n
-#pragma unroll
-            for (int k = 0; k < VN; ++k)
-              if (c + k < n) z[k] = p[k];
-        }
-        term[v] = vec_pack(z);
-      }
-    };
-    load_terms(0);
-    int it = 0;
-    for (int tt = 0; tt < cr.ntiles; ++tt) {
-      const int t = reverse ? cr.ntiles - 1 - tt : tt;
-      const long long tc0 = cr.c0 + (long long)t * TILE;
-      const int len = (int)((cr.c1 - tc0) < TILE ? (cr.c1 - tc0) : TILE);
-      const int b = tt & 1;
-      {  // ---- build this thread's vector of the x tile ----
-        T acc[VN];
-#pragma unroll
-        for (int k = 0; k < VN; ++k) acc[k] = T(0);
-#pragma unroll
-        for (int v = 0; v < kXTerms; ++v) {
-          if (v < a.nvec) {
-            T e[VN];
-            vec_unpack(term[v], e);
-#pragma unroll
-            for (int k = 0; k < VN; ++k) acc[k] = fma(cv[v], e[k], acc[k]);
-          }
-        }
-        const long long c = tc0 + (long long)tid * VN;
-        bool all_ok = true;
-#pragma unroll
-        for (int k = 0; k < VN; ++k) {
-          const bool ok = tid * VN + k < len && c + k < n;
-          acc[k] = ok ? acc[k] / oscale : T(0);
-          all_ok = all_ok && ok;
-        }
-        reinterpret_cast<V*>(xs + (size_t)b * TILE)[tid] = vec_pack(acc);
-        if (all_ok) {
-          *reinterpret_cast<V*>(static_cast<T*>(a.out) + c) = vec_pack(acc);
-        } else {
-#pragma unroll
-          for (int k = 0; k < VN; ++k)
-            if (tid * VN + k < len && c + k < n) static_cast<T*>(a.out)[c + k] = acc[k];
-        }
-      }
-      load_terms(tt + 1);  // in flight while this tile's rows are consumed (in place: own columns only)
-      tma::named_bar_sync(1, kConsumerThreads);
-      V xr[XV];
-#pragma unroll
-      for (int u = 0; u < XV; ++u) xr[u] = reinterpret_cast<const V*>(xs + (size_t)b * TILE)[lane + 32 * u];
-      for (int gg = 0; gg < ngroups; ++gg, ++it) {
-        const int g = reverse ? ngroups - 1 - gg : gg;
-        const int s = it % kStages;
-        tma::mbar_wait(full + s, (it / kStages) & 1);
-        const int j = g * kGroup + warp;
-        if (j < nrows) {
-          const V* row = reinterpret_cast<const V*>(stages + ((size_t)s * kGroup + warp) * TILE);
-          T a0 = T(0), a1 = T(0);
-#pragma unroll
-          for (int u = 0; u < XV; ++u) {
-            if ((lane + 32 * u) * VN < len) {
-              T q[VN], xx[VN];
-              vec_unpack(row[lane + 32 * u], q);
-              vec_unpack(xr[u], xx);
-#pragma unroll
-              for (int k = 0; k < VN; ++k) {
-                if (u & 1)
-                  a1 = fma(q[k], xx[k], a1);
-                else
-                  a0 = fma(q[k], xx[k], a0);
-              }
-            }
-          }
-          __syncwarp();
-          if (lane == 0) tma::mbar_arrive(empty + s);
-          double sacc = warp_sum(static_cast<double>(a0) + static_cast<double>(a1));
-          if (lane == 0) acc_s[j] += sacc;  // row j is always handled by this warp: no race
-        } else {
-          __syncwarp();
-          if (lane == 0) tma::mbar_arrive(empty + s);
-        }
-      }
-    }
-  }
-  __syncthreads();
-  for (int j = threadIdx.x; j < nrows; j += blockDim.x) a.partials[(size_t)j * gridDim.x + blockIdx.x] = acc_s[j];
-  if (!last_block_done(a.counter)) return;
-  reduce_partials_and_epilogue<T>(nrows, a.partials, a.epi);
-}
 
 // ---------------------------------------------------------------------------------------------
 // out = s * sum_j c_j row_j (+ ||out||^2): dense vector terms are rows too (src.nv leading
@@ -540,28 +415,22 @@ k_combine_tma(CombineTmaArgs a) {
         const int t = reverse ? cr.ntiles - 1 - tt : tt;
         const long long tc0 = cr.c0 + (long long)t * TILE;
         const int len = (int)((cr.c1 - tc0) < TILE ? (cr.c1 - tc0) : TILE);
-        const uint32_t bytes = (uint32_t)len * sizeof(T);
         for (int gg = 0; gg < ngroups; ++gg, ++it) {
-          const bool vec_group = gg >= ngb;
-          const int g = vec_group ? gg : (reverse ? ngb - 1 - gg : gg);
-          const int s = it % kStages;
-          if (vec_group && !waited) {
+          if (gg < ngb) {
+            stage_rows<T, TILE>(stages, full, empty, it, a.src, reverse ? ngb - 1 - gg : gg, nbasis, tc0, len);
+            continue;
+          }
+          if (!waited) {
             tma::griddep_wait();
             waited = true;
           }
+          const uint32_t bytes = (uint32_t)len * sizeof(T);
+          const int s = it % kStages;
           tma::mbar_wait(empty + s, ((it / kStages) & 1) ^ 1);
+          tma::mbar_arrive_expect_tx(full + s, bytes * a.nvec);
           T* dst = stages + (size_t)s * kGroup * TILE;
-          if (vec_group) {
-            tma::mbar_arrive_expect_tx(full + s, bytes * a.nvec);
-            for (int r = 0; r < a.nvec; ++r)
-              tma::bulk_g2s(dst + (size_t)r * TILE, static_cast<const T*>(a.vec[r].ptr) + tc0, bytes, full + s);
-          } else {
-            const int rows_here = nbasis - g * kGroup < kGroup ? nbasis - g * kGroup : kGroup;
-            tma::mbar_arrive_expect_tx(full + s, bytes * rows_here);
-            for (int r = 0; r < rows_here; ++r)
-              tma::bulk_g2s_hint(dst + (size_t)r * TILE, a.src.row(g * kGroup + r) + tc0 * (long long)sizeof(T), bytes,
-                                 full + s, tma::policy_evict_first());
-          }
+          for (int r = 0; r < a.nvec; ++r)
+            tma::bulk_g2s(dst + (size_t)r * TILE, static_cast<const T*>(a.vec[r].ptr) + tc0, bytes, full + s);
         }
       }
     }
@@ -593,7 +462,6 @@ k_combine_tma(CombineTmaArgs a) {
       const int len = (int)((cr.c1 - tc0) < TILE ? (cr.c1 - tc0) : TILE);
       const long long col = tc0 + (long long)tid * VN;
       const bool live = tid * VN < len;
-      const bool fullvec = live && col + VN <= a.n;
       T acc[VN];
 #pragma unroll
       for (int k = 0; k < VN; ++k) acc[k] = T(0);
@@ -603,29 +471,9 @@ k_combine_tma(CombineTmaArgs a) {
         const int s = it % kStages;
         tma::mbar_wait(full + s, (it / kStages) & 1);
         const int rows_here = vec_group ? a.nvec : (nbasis - g * kGroup < kGroup ? nbasis - g * kGroup : kGroup);
-        if (live) {
-          const V* st = reinterpret_cast<const V*>(stages + (size_t)s * kGroup * TILE) + tid;
-          const T* cf = coef + g * kGroup;
-          if (rows_here == kGroup) {
-            V q[kGroup];
-#pragma unroll
-            for (int r = 0; r < kGroup; ++r) q[r] = st[(size_t)r * (TILE / VN)];
-#pragma unroll
-            for (int r = 0; r < kGroup; ++r) {
-              T e[VN];
-              vec_unpack(q[r], e);
-#pragma unroll
-              for (int k = 0; k < VN; ++k) acc[k] = fma(cf[r], e[k], acc[k]);
-            }
-          } else {
-            for (int r = 0; r < rows_here; ++r) {
-              T e[VN];
-              vec_unpack(st[(size_t)r * (TILE / VN)], e);
-#pragma unroll
-              for (int k = 0; k < VN; ++k) acc[k] = fma(cf[r], e[k], acc[k]);
-            }
-          }
-        }
+        if (live)
+          fma_group<T, TILE>(reinterpret_cast<const V*>(stages + (size_t)s * kGroup * TILE) + tid, coef + g * kGroup,
+                             rows_here, acc);
         __syncwarp();
         if (lane == 0) tma::mbar_arrive(empty + s);
       }
@@ -635,17 +483,8 @@ k_combine_tma(CombineTmaArgs a) {
           acc[k] = acc[k] * oscale[0] / oscale[1];
           if (NORM && col + k < a.n) ss += static_cast<double>(acc[k] * acc[k]);
         }
-        if (fullvec) {
-          reinterpret_cast<V*>(a.out)[col / VN] = vec_pack(acc);
-          if (a.out2) reinterpret_cast<V*>(a.out2)[col / VN] = vec_pack(acc);
-        } else {
-#pragma unroll
-          for (int k = 0; k < VN; ++k)
-            if (col + k < a.n) {
-              static_cast<T*>(a.out)[col + k] = acc[k];
-              if (a.out2) static_cast<T*>(a.out2)[col + k] = acc[k];
-            }
-        }
+        store_colvec(static_cast<T*>(a.out), col, a.n, acc);
+        if (a.out2) store_colvec(static_cast<T*>(a.out2), col, a.n, acc);
       }
     }
   }
