@@ -428,12 +428,7 @@ struct GramOperator : bl_operator {
   int tc_split = 1;
 
   bool tc_eligible(int dtype) const { return dtype == BL_F32 && d <= 20; }
-  bool use_tc(int dtype) const {
-    if (!tc_eligible(dtype) || path == 1) return false;
-    if (path == 2) return true;
-    const char* env = std::getenv("BL_GRAM_PATH");  // "alu" / "tc": A/B comparisons without recompiling
-    return !(env && std::string(env) == "alu");
-  }
+  bool use_tc(int dtype) const { return tc_eligible(dtype) && path != 1; }
   int tc_rowtiles() const { return (int)((n + gramtc::kM - 1) / gramtc::kM); }
   int tc_gparts() const { return tc_rowtiles() * tc_split; }
 

@@ -4,10 +4,11 @@ Host-side mirror of `/root/reference/src/matfree_extensions/hutchinson.py` plus 
 `matfree.hutchinson.hutchinson` / `sampler_rademacher` pair the reference imports
 (`/root/reference/src/matfree_extensions/util/gp_util.py:8,557`).  An estimator is
 `sample(key, *parameters)`; `sample_fun(key)` returns the `(num, n)` probe matrix.  Probe
-vectors are independent Lanczos runs: in lockstep batches on operators that share work between
-vectors (the Gram operator, `lanczos.probe_batch_sum`; a sparse operand, `lanczos.probe_lockstep_sum`), one
-after the other otherwise; sharded over GPUs
-by `parallel.shard_probes`.
+vectors are independent Lanczos runs, which `probe_sum` sums in one of three ways: lockstep
+batches on a sparse operand (`lanczos.probe_lockstep_sum`, at least `lanczos.LOCKSTEP_MIN_PROBES`
+probes), lockstep runs on the Gram operator, which shares work between vectors
+(`lanczos.probe_batch_sum`), and one probe after the other otherwise (`probe_loop_sum`).
+`parallel.hutchinson_sharded` shards the probes over GPUs.
 
 PRNG note: JAX's threefry stream cannot be reproduced without JAX.  `sampler_rademacher` /
 `sampler_normal` / `split` here are NumPy-based; parity tests always pass probes explicitly.
@@ -88,22 +89,24 @@ def _resident(parameters, like):
 
 
 def probe_sum(integrand_fun, samples, parameters, *, with_grad=False):
-    """Sum (not mean) of the integrand over probes; gradients stay on the device."""
-    lazy = type(samples).__name__ == "LazyProbes"  # rows drawn on demand (parallel.sharded_sampler)
-    if (isinstance(samples, np.ndarray) or lazy) and samples.ndim == 2 and len(samples) > 1 and hasattr(integrand_fun, "alg"):
-        from experiments_lanczos_adjoints_b200 import lanczos
+    """Sum (not mean) of the integrand over probes, `(total, grads, count)`; gradients stay on the device."""
+    from experiments_lanczos_adjoints_b200 import lanczos
 
-        if lanczos._pipeline_eligible(integrand_fun, samples):  # sparse operand: lockstep batches of probes
-            if lanczos._probe_mode() == "streams":  # ... or independent runs in flight on separate streams
-                return lanczos.probe_pipelined_sum(integrand_fun, samples, parameters, with_grad=with_grad)
-            return lanczos.probe_lockstep_sum(integrand_fun, samples, parameters, with_grad=with_grad)
-        if lazy:
-            samples = np.asarray(samples)
-        if samples.dtype in (np.float32, np.float64) and lanczos._batch_eligible(integrand_fun, samples.dtype):
-            return lanczos.probe_batch_sum(integrand_fun, samples, parameters, with_grad=with_grad)
-    total, grads, count = 0.0, None, 0
-    if type(samples).__name__ == "LazyProbes":
+    lazy = type(samples).__name__ == "LazyProbes"  # rows drawn on demand (parallel.sharded_sampler)
+    matrix = (isinstance(samples, np.ndarray) or lazy) and samples.ndim == 2 and len(samples) > 1
+    if matrix and lanczos._lockstep_eligible(integrand_fun, samples):  # lazy probes are drawn one batch at a time
+        return lanczos.probe_lockstep_sum(integrand_fun, samples, parameters, with_grad=with_grad)
+    if lazy:
         samples = np.asarray(samples)
+    if matrix and samples.dtype in (np.float32, np.float64) and lanczos._batch_eligible(integrand_fun, samples.dtype):
+        return lanczos.probe_batch_sum(integrand_fun, samples, parameters, with_grad=with_grad)
+    return probe_loop_sum(integrand_fun, samples, parameters, with_grad=with_grad)
+
+
+def probe_loop_sum(integrand_fun, samples, parameters, *, with_grad):
+    """`probe_sum` one probe at a time (`jax.vmap(integrand)`, hutchinson.py:14): the path of every integrand the
+    batched sums do not take, and their reference in tests."""
+    total, grads, count = 0.0, None, 0
     rows = _probe_rows(samples)
     if len(rows):
         parameters = _resident(parameters, rows[0])

@@ -18,6 +18,7 @@ import numpy as np
 from experiments_lanczos_adjoints_b200 import _lib
 from experiments_lanczos_adjoints_b200 import arnoldi
 from experiments_lanczos_adjoints_b200 import device as dev
+from experiments_lanczos_adjoints_b200 import synthetic
 from experiments_lanczos_adjoints_b200.arnoldi import _cotangent_basis, _cotangent_vec, _ptr, _run, _Workspace
 
 
@@ -107,11 +108,7 @@ class _TridiagFull:
 
         def pullback(cot):
             (dQt, (dalpha, dbeta)), (dq_rem, dnorm) = cot
-            # cotangent of T = (H + H^T)/2 and its diagonals (lanczos.py:162-164)
-            dH = np.diag(np.asarray(dalpha, dtype=dtype))
-            if K > 1:
-                dbeta = np.asarray(dbeta, dtype=dtype)
-                dH = dH + 0.5 * (np.diag(dbeta, 1) + np.diag(dbeta, -1))
+            dH = synthetic.slq_cotangent_dH(dalpha, dbeta, dtype)
             # cotangent of (r/||r||, ||r||) (lanczos.py:166)
             dr = None
             dq = _cotangent_vec(dq_rem, r.size, dtype)
@@ -301,7 +298,7 @@ def _batch_eligible(integrand, dtype) -> bool:
     their parameter cotangent (the Gram operator on the tensor-core path)."""
     import ctypes as C
 
-    alg = integrand.alg
+    alg = getattr(integrand, "alg", None)
     if not isinstance(alg, _TridiagFull) or not alg.alg.custom_vjp:
         return False
     op = alg.alg.op
@@ -315,63 +312,34 @@ def _batch_eligible(integrand, dtype) -> bool:
     return bool(yes.value)
 
 
-PROBE_LANES = 4  # independent probes in flight per GPU in `probe_pipelined_sum`
-
-
-def _pipeline_eligible(integrand, probes) -> bool:
-    """Probes in flight apply to the full-reorthogonalisation adjoint path on a sparse operand (an operator that
-    can be cloned: every lane needs its own values and cotangent accumulator)."""
-    alg = getattr(integrand, "alg", None)
-    if not isinstance(alg, _TridiagFull) or not alg.alg.custom_vjp or PROBE_LANES < 2:
-        return False
-    op = alg.alg.op
-    return (type(op).__name__ == "SparseOperator" and op.shape[0] == op.shape[1] and len(probes) >= 2 * PROBE_LANES
-            and probes.dtype in (np.float32, np.float64))  # fmt: skip
-
-
-def probe_pipelined_sum(integrand, probes, parameters, *, with_grad, lanes=None):
-    """Sum over the rows of `probes (P, n)` of the SLQ integrand (and of its parameter gradient) with several
-    probes IN FLIGHT: every lane owns an operator handle, a `TridiagAdjointPlan` (basis, adjoint basis, workspace)
-    and a stream.  The forward runs of a group of probes are enqueued back to back; while the host does the
-    K x K `eigh` of one lane (`lanczos.py:48-59`), the other lanes' kernels run, and one run's per-launch fixed
-    costs are filled by the others' kernels.  The parameter cotangent accumulates inside each lane's operator over
-    all its probes and is exported once.  Same numbers as a loop of `integrand.value_and_grad`
-    (`jax.vmap(integrand)`, hutchinson.py:14) up to summation order."""
-    from experiments_lanczos_adjoints_b200 import plan as _plan
-
-    probes = np.asarray(probes)
-    P, n = probes.shape
-    dtype = probes.dtype
-    hess = integrand.alg.alg
-    K = hess.K
-    if not isinstance(K, (int, np.integer)) or K < 1 or K > n:
-        raise ValueError(f"Parameter depth {K} is outside the expected range")
-    L = max(1, min(lanes or PROBE_LANES, P))
-    cache = integrand.__dict__.setdefault("_lane_plans", {})
-    key = (L, dtype.str, n, K)
-    if key not in cache:
-        ops = [hess.op] + [hess.op.clone() for _ in range(L - 1)]
-        cache[key] = [_plan.TridiagAdjointPlan(o, K, dtype, stream=dev.Stream()) for o in ops]
-    plans = cache[key]
-    host_params = [p.numpy() if isinstance(p, dev.DeviceArray) else np.asarray(p) for p in parameters]
-    dev.synchronize()  # the lanes' streams start after whatever the caller enqueued
-    for pl in plans:
-        pl.set_params(*host_params)
-    total = 0.0
-    used = [False] * L
-    # kernels of different lanes share an SM (one block per SM and kernel), see bl_set_blocks_per_sm; the caller's own
-    # setting comes back afterwards
-    with dev.blocks_per_sm(1 if L >= 3 else dev.get_blocks_per_sm()):
-        try:
-            total = _pipelined_groups(integrand, plans, probes, L, K, dtype, with_grad, used)
-        finally:
-            for pl in plans:
-                pl.stream.synchronize()
-    return _pipelined_finish(plans, used, dtype, total, P, with_grad)
-
-
 LOCKSTEP_BATCH = 4  # runs per lockstep batch (one k_step_tma launch serves up to four runs)
 LOCKSTEP_LANES = 2  # batches in flight: the host's K x K eigh of one batch runs under the other batch's kernels
+LOCKSTEP_MIN_PROBES = 8  # two full batches, so that two are in flight; fewer probes run one at a time
+
+
+def _lockstep_eligible(integrand, probes) -> bool:
+    """Lockstep batches (`probe_lockstep_sum`) apply to the full-reorthogonalisation adjoint path on a square sparse
+    operand (an operator that can be cloned: every lane needs its own values and cotangent accumulator), for at
+    least `LOCKSTEP_MIN_PROBES` float32 or float64 probes."""
+    alg = getattr(integrand, "alg", None)
+    if not isinstance(alg, _TridiagFull) or not alg.alg.custom_vjp:
+        return False
+    op = alg.alg.op
+    return (type(op).__name__ == "SparseOperator" and op.shape[0] == op.shape[1]
+            and len(probes) >= LOCKSTEP_MIN_PROBES and probes.dtype in (np.float32, np.float64))  # fmt: skip
+
+
+def _slq_batch(integrand, coefs, scales, with_grad, total, dH):
+    """Adds `||v0||^2 e1^T f(T) e1` (`lanczos.py:25,59`) of each run of a batch to `total`, in run order, and returns
+    the sum; with `with_grad`, `dH[b]` receives run b's cotangent of `H`.  `coefs[b]` is run b's `(diag, off_diag)`,
+    `scales[b]` its `||v0||`."""
+    for b, ((diag, off), scale) in enumerate(zip(coefs, scales)):
+        g, dalpha, dbeta, _ = _quadform_and_cotangents(integrand.matfun, integrand.matfun_grad, diag, off, with_grad)
+        s2 = scale**2
+        total += s2 * g
+        if with_grad:
+            dH[b] = synthetic.slq_cotangent_dH(s2 * dalpha, s2 * dbeta, dH.dtype)
+    return total
 
 
 def probe_lockstep_sum(integrand, probes, parameters, *, with_grad, batch=None, lanes=None):
@@ -420,15 +388,7 @@ def probe_lockstep_sum(integrand, probes, parameters, *, with_grad, batch=None, 
             warnings.warn("tridiag(reortho='full'): the operand is not symmetric on this Krylov space; the adjoint "
                           "runs the general Arnoldi loops, as the reference does.", stacklevel=3)  # fmt: skip
         dH = np.zeros((B, K, K), dtype)
-        for b in range(real):
-            diag, off = coefs[b]
-            g, dalpha, dbeta, _ = _quadform_and_cotangents(integrand.matfun, integrand.matfun_grad, diag, off, with_grad)
-            s2 = scales[b] ** 2
-            total += s2 * g
-            if with_grad:
-                dH[b] = np.diag(s2 * dalpha)
-                if K > 1:
-                    dH[b] += 0.5 * (np.diag(s2 * dbeta, 1) + np.diag(s2 * dbeta, -1))
+        total = _slq_batch(integrand, coefs[:real], scales, with_grad, total, dH)
         if with_grad:
             pl.set_cotangents(dH)  # padding runs of a short last batch carry a zero cotangent: no contribution
             pl.adjoint(zero=not used[li], export=False,
@@ -462,58 +422,25 @@ def probe_lockstep_sum(integrand, probes, parameters, *, with_grad, batch=None, 
         for pl in plans:
             pl.stream.synchronize()
         bps.__exit__(None, None, None)
-    return _pipelined_finish(plans, used, dtype, total, P, with_grad)
+    return total, (_lane_grad_sum(plans, used, dtype) if with_grad else None), P
 
 
-def _probe_mode() -> str:
-    """BL_PROBE_MODE: `lockstep` (default; batched runs, `probe_lockstep_sum`) or `streams` (independent runs on
-    separate streams, `probe_pipelined_sum`) for the SLQ estimator on a sparse operand."""
-    import os
-
-    return os.environ.get("BL_PROBE_MODE", "lockstep")
-
-
-def _pipelined_groups(integrand, plans, probes, L, K, dtype, with_grad, used):
-    total = 0.0
-    P = len(probes)
-    for p0 in range(0, P, L):
-        group = probes[p0 : p0 + L]
-        scales = np.linalg.norm(group.astype(np.float64), axis=1)  # lanczos.py:25
-        for pl, v, sc in zip(plans, group, scales):
-            pl.set_vector((v / sc).astype(dtype))
-            pl.forward()
-        for li, (pl, sc) in enumerate(zip(plans, scales)):
-            diag, off = pl.coefficients()  # synchronises this lane only
-            g, dalpha, dbeta, _ = _quadform_and_cotangents(integrand.matfun, integrand.matfun_grad, diag, off, with_grad)
-            s2 = sc**2
-            total += s2 * g
-            if with_grad:
-                dH = np.diag(s2 * dalpha)
-                if K > 1:
-                    dH = dH + 0.5 * (np.diag(s2 * dbeta, 1) + np.diag(s2 * dbeta, -1))
-                pl.set_cotangent(dH.astype(dtype))
-                pl.adjoint(zero=not used[li], export=False)
-                used[li] = True
-    return total
-
-
-def _pipelined_finish(plans, used, dtype, total, P, with_grad):
-    grads = None
-    if with_grad:
-        active = [pl for pl, u in zip(plans, used) if u]
-        for pl in active:
-            pl.export_grads()
-            pl.stream.synchronize()
-        stream = dev.default_stream()
-        grads = []
-        for gi in range(len(active[0].grads)):
-            acc = dev.DeviceArray(active[0].grads[gi].shape, dtype)
-            _lib.call("bl_vec_axpby", dev.dtype_code(dtype), acc.size, 1.0, active[0].grads[gi].ptr, 0.0, None, acc.ptr, stream.ptr)
-            for pl in active[1:]:
-                _lib.call("bl_vec_axpby", dev.dtype_code(dtype), acc.size, 1.0, acc.ptr, 1.0, pl.grads[gi].ptr, acc.ptr, stream.ptr)
-            grads.append(acc)
-        stream.synchronize()
-    return total, grads, P
+def _lane_grad_sum(plans, used, dtype):
+    """Exports the parameter cotangent each used lane accumulated in its operator and returns the sum over lanes."""
+    active = [pl for pl, u in zip(plans, used) if u]
+    for pl in active:
+        pl.export_grads()
+        pl.stream.synchronize()
+    stream = dev.default_stream()
+    grads = []
+    for gi in range(len(active[0].grads)):
+        acc = dev.DeviceArray(active[0].grads[gi].shape, dtype)
+        _lib.call("bl_vec_axpby", dev.dtype_code(dtype), acc.size, 1.0, active[0].grads[gi].ptr, 0.0, None, acc.ptr, stream.ptr)
+        for pl in active[1:]:
+            _lib.call("bl_vec_axpby", dev.dtype_code(dtype), acc.size, 1.0, acc.ptr, 1.0, pl.grads[gi].ptr, acc.ptr, stream.ptr)
+        grads.append(acc)
+    stream.synchronize()
+    return grads
 
 
 def probe_batch_sum(integrand, probes, parameters, *, with_grad, stream=None, chunk=16):
@@ -549,17 +476,9 @@ def probe_batch_sum(integrand, probes, parameters, *, with_grad, stream=None, ch
         _lib.call("bl_arnoldi_forward_batch", op._handle, code, n, K, arnoldi.forward_flags(True, True), B, U.ptr, n, Q.ptr, ld, H.ptr, r.ptr, c.ptr,
                   ws.ptr, per * B, stream.ptr)  # fmt: skip
         Hh = H.numpy(stream).reshape(B, K, K)
+        coefs = [(np.diag(T, 0), np.diag(T, 1)) for T in 0.5 * (Hh + Hh.transpose(0, 2, 1))]  # lanczos.py:162
         dH = np.zeros((B, K, K), dtype=dtype)
-        for b in range(B):
-            T = 0.5 * (Hh[b] + Hh[b].T)  # lanczos.py:162
-            diag, off = np.diag(T, 0), np.diag(T, 1)
-            g, dalpha, dbeta, _ = _quadform_and_cotangents(integrand.matfun, integrand.matfun_grad, diag, off, with_grad)
-            s2 = scale[b] ** 2
-            total += s2 * g
-            if with_grad:
-                dH[b] = np.diag(s2 * dalpha)
-                if K > 1:
-                    dH[b] += 0.5 * (np.diag(s2 * dbeta, 1) + np.diag(s2 * dbeta, -1))
+        total = _slq_batch(integrand, coefs, scale, with_grad, total, dH)
         if with_grad:
             dHd = dev.asarray(dH.reshape(B, K * K))
             dv = dev.DeviceArray((B, n), dtype, ld=ld)

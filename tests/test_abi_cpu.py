@@ -197,27 +197,23 @@ def test_sparse_operator_clone_shares_the_pattern_not_the_handle():
             assert np.array_equal(a, b)
 
 
-def test_probe_pipeline_eligibility_is_host_logic():
-    """Which estimator calls keep probes in flight (`lanczos._pipeline_eligible`): full-reorthogonalisation SLQ on a
-    square sparse operand with at least two probes per lane; everything else takes the lockstep or sequential route."""
+def test_probe_lockstep_eligibility_is_host_logic():
+    """Which estimator calls run their probes in lockstep batches (`lanczos._lockstep_eligible`): full-
+    reorthogonalisation SLQ on a square sparse operand with at least 8 probes; everything else takes the Gram batch
+    or the one-probe-at-a-time route."""
     from experiments_lanczos_adjoints_b200 import lanczos
 
     n = 64
     idx = np.arange(n, dtype=np.int32)
     sparse = bl.operators.SparseOperator(idx, idx, (n, n))
-    probes = np.ones((2 * lanczos.PROBE_LANES, n), np.float32)
+    probes = np.ones((8, n), np.float32)
     full = bl.lanczos.integrand_spd(np.log, 4, sparse)
-    assert lanczos._pipeline_eligible(full, probes)
-    assert not lanczos._pipeline_eligible(full, probes[:-1])  # fewer than two probes per lane
-    assert not lanczos._pipeline_eligible(full, probes.astype(np.int32))
-    assert not lanczos._pipeline_eligible(bl.lanczos.integrand_spd(np.log, 4, sparse, reortho="none"), probes)
-    assert not lanczos._pipeline_eligible(bl.lanczos.integrand_spd(np.log, 4, bl.operators.DenseOperator(n)), probes)
+    assert lanczos._lockstep_eligible(full, probes)
+    assert not lanczos._lockstep_eligible(full, probes[:-1])  # fewer than two batches of four
+    assert not lanczos._lockstep_eligible(full, probes.astype(np.int32))
+    assert not lanczos._lockstep_eligible(bl.lanczos.integrand_spd(np.log, 4, sparse, reortho="none"), probes)
+    assert not lanczos._lockstep_eligible(bl.lanczos.integrand_spd(np.log, 4, bl.operators.DenseOperator(n)), probes)
     assert not lanczos._batch_eligible(full, np.float32)  # the sparse operand shares no work between probes
-    lanes, lanczos.PROBE_LANES = lanczos.PROBE_LANES, 1
-    try:
-        assert not lanczos._pipeline_eligible(full, probes)
-    finally:
-        lanczos.PROBE_LANES = lanes
 
 
 def test_ffi_shim_handlers_match_their_bindings(tmp_path):

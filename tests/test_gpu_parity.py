@@ -649,42 +649,35 @@ def test_two_lockstep_lanes_in_flight_reproduce_their_solo_runs_bit_for_bit(dtyp
                     assert np.array_equal(got, want), f"rep {rep} lane {li}: {name} differs from the solo run"
 
 
-@pytest.mark.parametrize("mode", ["lockstep", "streams"])
 @pytest.mark.parametrize("dtype", [np.float32, np.float64])
-def test_slq_estimator_with_probes_in_flight_matches_the_sequential_loop(dtype, mode, monkeypatch):
+def test_slq_estimator_with_probes_in_flight_matches_the_sequential_loop(dtype):
     """`hutchinson(integrand_spd(log, K, sparse_op), sampler)`: with >= 8 probes the estimator runs the probes in
     lockstep batches of four (`lanczos.probe_lockstep_sum`: multi-vector SpMV + one Gram-Schmidt step kernel per
-    batch; the default) or keeps four independent runs in flight on separate streams
-    (`lanczos.probe_pipelined_sum`, BL_PROBE_MODE=streams); value and gradient must equal the one-probe-at-a-time
-    loop (`jax.vmap(integrand)` + mean, hutchinson.py:14,54)."""
+    batch, two batches in flight); value and gradient must equal the one-probe-at-a-time loop
+    (`hutchinson.probe_loop_sum`, `jax.vmap(integrand)` + mean, hutchinson.py:14,54)."""
     from experiments_lanczos_adjoints_b200 import lanczos
-
-    monkeypatch.setattr(lanczos, "_probe_mode", lambda: mode)
 
     n, K, num = 20_003, 12, 9  # 9 = 4 + 4 + 1: the last group is ragged; n odd: rows 1..3 of a batch's (4, n) arrays are not 16-byte aligned
     row, col, data = banded_spd(n, 4, seed=31)
     probes = (np.random.default_rng(32).integers(0, 2, size=(num, n)) * 2 - 1).astype(dtype)
-    results = {}
-    for lanes in (1, 4):
-        lanczos.PROBE_LANES = lanes
-        try:
-            op = bl.operators.SparseOperator(row, col, (n, n))
-            integrand = bl.lanczos.integrand_spd(np.log, K, op)
-            estimate = bl.hutchinson.hutchinson(integrand, lambda key: probes)
-            assert lanczos._pipeline_eligible(integrand, probes) == (lanes > 1)
-            value, (grad,) = estimate.value_and_grad(None, data.astype(dtype))
-            results[lanes] = (float(value), grad.numpy(), float(estimate(None, data.astype(dtype))))
-        finally:
-            lanczos.PROBE_LANES = 4
+    integrand = bl.lanczos.integrand_spd(np.log, K, bl.operators.SparseOperator(row, col, (n, n)))
+    estimate = bl.hutchinson.hutchinson(integrand, lambda key: probes)
+    assert lanczos._lockstep_eligible(integrand, probes)
+    value, (grad,) = estimate.value_and_grad(None, data.astype(dtype))
+    lockstep = (float(value), grad.numpy(), float(estimate(None, data.astype(dtype))))
+    loop_integrand = bl.lanczos.integrand_spd(np.log, K, bl.operators.SparseOperator(row, col, (n, n)))
+    total, (grad,), count = bl.hutchinson.probe_loop_sum(loop_integrand, probes, (data.astype(dtype),), with_grad=True)
+    value_nograd = bl.hutchinson.probe_loop_sum(loop_integrand, probes, (data.astype(dtype),), with_grad=False)[0]
+    loop = (float(total) / count, grad.numpy() / count, float(value_nograd) / count)
     t_val, t_grad = (F64, F64) if dtype == np.float64 else (F32_VAL, F32_GRAD)
-    assert abs(results[4][0] - results[1][0]) < t_val * abs(results[1][0])
-    assert abs(results[4][2] - results[1][2]) < t_val * abs(results[1][2])
-    assert rel_err(results[4][1], results[1][1]) < t_grad
+    assert abs(lockstep[0] - loop[0]) < t_val * abs(loop[0])
+    assert abs(lockstep[2] - loop[2]) < t_val * abs(loop[2])
+    assert rel_err(lockstep[1], loop[1]) < t_grad
     # and against the float64 oracle on the same probes
     ref = krylov.IntegrandSPD(np.log, lambda x: 1.0 / x, K, operators.CsrFastOperator(row, col, (n, n)))
     val_ref, (grad_ref,) = krylov.hutchinson_value_and_grad(ref, probes.astype(np.float64), data)
-    assert abs(results[4][0] - val_ref) < 10 * t_val * abs(val_ref)
-    assert rel_err(results[4][1], grad_ref) < 10 * t_grad
+    assert abs(lockstep[0] - val_ref) < 10 * t_val * abs(val_ref)
+    assert rel_err(lockstep[1], grad_ref) < 10 * t_grad
 
 
 def test_peer_memory_route_two_ranks_on_one_gpu_matches_single_operator():
