@@ -89,6 +89,10 @@ SIGNATURES = {
     "bl_pcg_workspace_bytes": (C.c_size_t, [_i64, _i32]),
     "bl_pcg_solve": (_i32, [_vp, _i32, _i64, _vp, _vp, _i64, _i64, C.c_double, C.c_double, _i32, _vp, _vp,
                             C.POINTER(C.c_int64), _vp, C.c_size_t, _vp]),
+    "bl_pcg_batch_workspace_bytes": (C.c_size_t, [_i64, _i64, _i32]),
+    "bl_pcg_solve_batch": (_i32, [_vp, _i32, _i64, _i64, _vp, _i64, _vp, _i64, _i64, C.c_double, C.c_double, _i32, _vp,
+                                  _vp, C.POINTER(C.c_int64), _vp, C.c_size_t, _vp]),
+    "bl_rows_dot_pairs": (_i32, [_i32, _i64, _i64, _vp, _vp, _i64, _vp, _vp]),
     "bl_cholesky_workspace_bytes": (C.c_size_t, [_i64, _i64, _i32]),
     "bl_cholesky_partial": (_i32, [_vp, _i32, _i64, _i64, _i32, _vp, _i64, C.POINTER(C.c_int), C.POINTER(C.c_int64),
                                    _vp, C.c_size_t, _vp]),
@@ -100,6 +104,11 @@ SIGNATURES = {
     "bl_op_gram_create": (_i32, [_i64, _i64, _i32, _vp, _pvp]),
     "bl_op_gram_set_path": (_i32, [_vp, _i32]),
     "bl_op_gram_tile_distances": (_i32, [_vp, _i64, _i64, _vp, _vp]),
+    "bl_gram_cross_create": (_i32, [_vp, _i64, _vp, _pvp]),
+    "bl_gram_cross_destroy": (_i32, [_vp]),
+    "bl_gram_cross_matvec": (_i32, [_vp, _i32, _vp, _vp, _vp]),
+    "bl_gram_cross_columns": (_i32, [_vp, _i32, _i64, _i64, _vp, _i64, _vp]),
+    "bl_gram_cross_prior_diag": (_i32, [_vp, _i32, _vp, _vp]),
     "bl_op_wave_create": (_i32, [_i64, _vp, _pvp]),
     "bl_op_wave_slab_create": (_i32, [_i64, _i64, _i32, _i32, _vp, _pvp]),
     "bl_op_wave_halo": (_i32, [_vp, _i32, _pvp]),

@@ -8,6 +8,9 @@ The whole iteration runs on the device (`bl_pcg_solve`, `csrc/solve.cu`): step l
 test of `pcg_adaptive` and `_safe_divide` never touch the host; the fixed-step solver does not
 synchronise at all.  `solve.vjp(A, b, P)` is the `jax.lax.custom_linear_solve` rule of `cg.py:25-27`
 (symmetric A): `db = A^{-1} xbar`, `dtheta = -d<db, A(x; theta)>/dtheta`.
+
+`vmap_solver(solve)(A, B, P)` solves for every row of `B` in lockstep (`bl_pcg_solve_batch`): what
+`jax.vmap(solve, in_axes=(None, 0, None))` gives in the reference.
 """
 
 from __future__ import annotations
@@ -128,3 +131,56 @@ def pcg_adaptive(*, atol: float, rtol, maxiter: int, miniter: int, check_every: 
 
 def cg_adaptive(**kwargs):
     return _NoPrecond(pcg_adaptive(**kwargs))
+
+
+class _VmapSolver:
+    def __init__(self, solve):
+        if isinstance(solve, _NoPrecond):
+            self._solver, self._takes_p = solve._solver, False
+        elif isinstance(solve, _Solver):
+            self._solver, self._takes_p = solve, True
+        else:
+            raise TypeError("vmap_solver takes a solver of this module (pcg_* / cg_*)")
+        self._ws = None
+
+    def __call__(self, A, B, P=None, *, stream=None):
+        A = _as_bound(A)
+        if P is not None and not self._takes_p:
+            raise TypeError("a cg_* solver takes no preconditioner")
+        if P is not None and not hasattr(P, "_precond_handle"):
+            raise TypeError("P must be a bound low-rank preconditioner (`pre.bind(noise)`) or None")
+        stream = stream or dev.default_stream()
+        if not isinstance(B, dev.DeviceArray):
+            B = np.asarray(B)
+            if B.ndim != 2 or B.shape[1] != A.n:
+                raise ValueError(f"B must be (count, {A.n}), got shape {B.shape}")
+            B = dev.basis_from_host(B, B.dtype if B.dtype in (np.float32, np.float64) else np.float64)
+        if B.ndim != 2 or B.shape[1] != A.n:
+            raise ValueError(f"B must be (count, {A.n}), got shape {B.shape}")
+        count, n = B.shape
+        if B.is_transposed or (B.ld * B.dtype.itemsize) % 16:
+            B = dev.basis_from_host(B.numpy(), B.dtype)
+        s, dtype, ld = self._solver, B.dtype, B.ld
+        A.bind(dtype, stream)
+        nbytes = _lib.load().bl_pcg_batch_workspace_bytes(ld, count, dev.dtype_code(dtype))
+        if self._ws is None or self._ws.size * self._ws.dtype.itemsize < nbytes:
+            self._ws = dev.DeviceArray(((nbytes + 7) // 8,), np.float64)
+        X, R = dev.empty((count, n), dtype, ld=ld), dev.empty((count, n), dtype, ld=ld)
+        steps = np.zeros(count, np.int64)
+        _lib.call("bl_pcg_solve_batch", A.op._handle, dev.dtype_code(dtype), n, count, B.ptr, ld,
+                  P._precond_handle() if P is not None else None, s.max_steps, s.min_steps, s.atol, s.rtol,
+                  s.check_every, X.ptr, R.ptr, steps.ctypes.data_as(C.POINTER(C.c_int64)), self._ws.ptr, nbytes,
+                  stream.ptr)  # fmt: skip
+        info = _Info(X, residual_abs=R)
+        if s.atol >= 0.0:
+            info["num_steps"] = steps
+        return X, info
+
+
+def vmap_solver(solve, /):
+    """`jax.vmap(solve, in_axes=(None, 0, None))` for a `pcg_*` / `cg_*` solver: `vmap_solver(solve)(A, B, P=None)`
+    solves `A x = b` for every row `b` of `B` (count, n) and returns `(X (count, n), info)`; the info carries the
+    residuals row by row and, for the adaptive solvers, `num_steps` per row.  Each row follows exactly the rules
+    of `solve`; the rows share each operator sweep (the Gram operator evaluates a kernel tile once for up to 16
+    rows)."""
+    return _VmapSolver(solve)

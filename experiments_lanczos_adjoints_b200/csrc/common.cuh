@@ -133,20 +133,24 @@ __device__ __forceinline__ double block_sum(double v, double* smem) {
   return r;
 }
 
-// "Last block done" election: returns true in every thread of the block that finishes last.
-// Partials written by all blocks before the call are visible to the elected block.
-__device__ __forceinline__ bool last_block_done(unsigned int* counter) {
+// "Last block done" election among `blocks` blocks that share `counter`: returns true in every thread of the
+// block that finishes last.  Partials written by all blocks before the call are visible to the elected block.
+__device__ __forceinline__ bool last_block_done(unsigned int* counter, unsigned int blocks) {
   __shared__ bool is_last;
   __threadfence();
   __syncthreads();
   if (threadIdx.x == 0) {
     unsigned int prev = atomicAdd(counter, 1u);
-    is_last = (prev == gridDim.x * gridDim.y - 1);
+    is_last = (prev == blocks - 1);
     if (is_last) *counter = 0u;  // re-arm for the next launch on the same stream
   }
   __syncthreads();
   if (is_last) __threadfence();
   return is_last;
+}
+// ... among all blocks of the grid
+__device__ __forceinline__ bool last_block_done(unsigned int* counter) {
+  return last_block_done(counter, gridDim.x * gridDim.y);
 }
 
 }  // namespace bl

@@ -23,6 +23,7 @@
 
 #include <cstdint>
 #include <string>
+#include <vector>
 
 #include "b200_lanczos.h"
 #include "xla/ffi/api/ffi.h"
@@ -211,6 +212,40 @@ ffi::Error PcgSolve(cudaStream_t stream, ffi::AnyBuffer b, ffi::RemainingArgs pa
   return ffi::Error::Success();
 }
 
+// B, X, R (count, ld): the rows of B solved in lockstep (jax.vmap of the solve); num_steps (s64, count)
+ffi::Error PcgSolveBatch(cudaStream_t stream, ffi::AnyBuffer B, ffi::RemainingArgs params, ffi::Result<ffi::AnyBuffer> X,
+                         ffi::Result<ffi::AnyBuffer> R, ffi::Result<ffi::AnyBuffer> num_steps,
+                         ffi::Result<ffi::AnyBuffer> workspace, int64_t op_handle, int64_t precond_handle,
+                         int64_t max_steps, int64_t min_steps, double atol, double rtol, int64_t check_every) {
+  bl_operator_t* op = as_op(op_handle);
+  const int dtype = dtype_of(B.element_type());
+  const int64_t count = B.dimensions()[0], ld = B.dimensions()[1];
+  int64_t n = 0;
+  BL_FFI_TRY(to_error(bl_op_size(op, &n)));
+  BL_FFI_TRY(bind_params(op, dtype, params, stream));
+  std::vector<int64_t> steps((size_t)count);
+  BL_FFI_TRY(to_error(bl_pcg_solve_batch(op, dtype, n, count, B.untyped_data(), ld,
+                                         reinterpret_cast<bl_precond_t*>(precond_handle), max_steps, min_steps, atol,
+                                         rtol, (int)check_every, X->untyped_data(), R->untyped_data(), steps.data(),
+                                         workspace->untyped_data(), workspace->size_bytes(), stream)));
+  // `steps` lives in this frame: the copy must have completed before it returns
+  if (cudaMemcpyAsync(num_steps->untyped_data(), steps.data(), sizeof(int64_t) * steps.size(), cudaMemcpyHostToDevice,
+                      stream) != cudaSuccess ||
+      cudaStreamSynchronize(stream) != cudaSuccess)
+    return ffi::Error::Internal("copy of num_steps failed");
+  return ffi::Error::Success();
+}
+
+// y = K(X*, X) v of a bl_gram_cross_t whose parent Gram operator is bound with `params` first
+ffi::Error GramCrossMatvec(cudaStream_t stream, ffi::AnyBuffer v, ffi::RemainingArgs params,
+                           ffi::Result<ffi::AnyBuffer> y, int64_t op_handle, int64_t cross_handle) {
+  bl_operator_t* op = as_op(op_handle);
+  const int dtype = dtype_of(v.element_type());
+  BL_FFI_TRY(bind_params(op, dtype, params, stream));
+  return to_error(bl_gram_cross_matvec(reinterpret_cast<bl_gram_cross_t*>(cross_handle), dtype, v.untyped_data(),
+                                       y->untyped_data(), stream));
+}
+
 ffi::Error PrecondApply(cudaStream_t stream, ffi::AnyBuffer v, ffi::Result<ffi::AnyBuffer> out, int64_t precond_handle) {
   return to_error(bl_precond_apply(reinterpret_cast<bl_precond_t*>(precond_handle), dtype_of(v.element_type()),
                                    v.untyped_data(), out->untyped_data(), stream));
@@ -318,6 +353,28 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(bl_ffi_pcg_solve, PcgSolve,
                                   .Attr<double>("atol")
                                   .Attr<double>("rtol")
                                   .Attr<int64_t>("check_every"));
+
+XLA_FFI_DEFINE_HANDLER_SYMBOL(bl_ffi_pcg_solve_batch, PcgSolveBatch,
+                              BL_STREAM.Arg<Buf>()  // B (count, ld)
+                                  .RemainingArgs()
+                                  .Ret<Buf>()  // X
+                                  .Ret<Buf>()  // R
+                                  .Ret<Buf>()  // num_steps (s64, count)
+                                  .Ret<Buf>()  // workspace
+                                  .Attr<int64_t>("op_handle")
+                                  .Attr<int64_t>("precond_handle")
+                                  .Attr<int64_t>("max_steps")
+                                  .Attr<int64_t>("min_steps")
+                                  .Attr<double>("atol")
+                                  .Attr<double>("rtol")
+                                  .Attr<int64_t>("check_every"));
+
+XLA_FFI_DEFINE_HANDLER_SYMBOL(bl_ffi_gram_cross_matvec, GramCrossMatvec,
+                              BL_STREAM.Arg<Buf>()  // v (n)
+                                  .RemainingArgs()  // the parent's params
+                                  .Ret<Buf>()       // y (M)
+                                  .Attr<int64_t>("op_handle")
+                                  .Attr<int64_t>("cross_handle"));
 
 XLA_FFI_DEFINE_HANDLER_SYMBOL(bl_ffi_precond_apply, PrecondApply,
                               BL_STREAM.Arg<Buf>().Ret<Buf>().Attr<int64_t>("precond_handle"));

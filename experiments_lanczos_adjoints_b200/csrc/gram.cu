@@ -148,11 +148,15 @@ __device__ __forceinline__ void kernel_eval2(const P2<T>& sigma, const P2<T>& s2
 //   ADJ == false: part[split][i] = sum_{j in split} k_ij v_j
 //   ADJ == true : part[split][i] = sum_j k_ij lam_j ; block partial sums of
 //                 d_sigma = sum lam_i q_j k_ij / sigma and  d_ls[k] = sum lam_i q_j dk_ij (x_ik - x_jk)^2
-template <typename T, int DP, int RI, bool ADJ, int KIND>
+// CROSS == true: the rows are the m points (xsa, xxa) of another set (a cross-covariance K(X*, X) v,
+// part[split][m]); the columns stay the n points (xs, xx).
+template <typename T, int DP, int RI, bool ADJ, int KIND, bool CROSS = false>
 __global__ void __launch_bounds__(kTileI)
 k_gram_sweep(int64_t n, int d, const T* __restrict__ xs, const T* __restrict__ xx,
              const T* __restrict__ consts, const T* __restrict__ v, const T* __restrict__ q,
-             T* __restrict__ part, double* __restrict__ gpart /* [blocks][d+1] */) {
+             T* __restrict__ part, double* __restrict__ gpart /* [blocks][d+1] */, int64_t m,
+             const T* __restrict__ xsa, const T* __restrict__ xxa) {
+  static_assert(!(CROSS && ADJ), "the cross-covariance sweep has no adjoint");
   using V = typename Vec<T>::type;
   constexpr int VN = Vec<T>::N;
   constexpr int NV = DP / VN;
@@ -165,6 +169,9 @@ k_gram_sweep(int64_t n, int d, const T* __restrict__ xs, const T* __restrict__ x
 
   const int tid = threadIdx.x;
   const int64_t i0 = (int64_t)blockIdx.x * (kTileI * RI);
+  const int64_t rows = CROSS ? m : n;
+  const T* xsr = CROSS ? xsa : xs;
+  const T* xxr = CROSS ? xxa : xx;
   static_assert(RI % 2 == 0, "rows are processed in pairs");
   constexpr int RP = RI / 2;
   const P2<T> sigma2 = p2_splat(consts[0]);
@@ -173,12 +180,12 @@ k_gram_sweep(int64_t n, int d, const T* __restrict__ xs, const T* __restrict__ x
 #pragma unroll
   for (int p = 0; p < RP; ++p) {
     const int64_t ia = i0 + tid + (int64_t)kTileI * (2 * p), ib = ia + kTileI;
-    live[2 * p] = ia < n;
-    live[2 * p + 1] = ib < n;
+    live[2 * p] = ia < rows;
+    live[2 * p + 1] = ib < rows;
 #pragma unroll
     for (int k = 0; k < DP; ++k)
-      xi[p][k] = p2_set(live[2 * p] ? xs[ia * DP + k] : T(0), live[2 * p + 1] ? xs[ib * DP + k] : T(0));
-    xxi[p] = p2_set(live[2 * p] ? xx[ia] : T(0), live[2 * p + 1] ? xx[ib] : T(0));
+      xi[p][k] = p2_set(live[2 * p] ? xsr[ia * DP + k] : T(0), live[2 * p + 1] ? xsr[ib * DP + k] : T(0));
+    xxi[p] = p2_set(live[2 * p] ? xxr[ia] : T(0), live[2 * p + 1] ? xxr[ib] : T(0));
     lam_i[p] = p2_set((ADJ && live[2 * p]) ? v[ia] : T(0), (ADJ && live[2 * p + 1]) ? v[ib] : T(0));
   }
 
@@ -276,7 +283,7 @@ k_gram_sweep(int64_t n, int d, const T* __restrict__ xs, const T* __restrict__ x
 #pragma unroll
   for (int r = 0; r < RI; ++r) {
     const int64_t i = i0 + tid + (int64_t)kTileI * r;
-    if (live[r]) part[(int64_t)blockIdx.y * n + i] = static_cast<T>(y_acc[r]);
+    if (live[r]) part[(int64_t)blockIdx.y * rows + i] = static_cast<T>(y_acc[r]);
   }
   if (ADJ) {
     // rows that are not live carry lam_i = 0, so their sums are already zero
@@ -292,17 +299,20 @@ k_gram_sweep(int64_t n, int d, const T* __restrict__ xs, const T* __restrict__ x
   }
 }
 
-// out[j] = k(x_j, x_idx) (idx = *index) or k(x_j, x_j) (index == nullptr): the lazy kernel of
-// gp_util.py:257-258, same expanded squared distance as the sweeps
+// out[b * ldo + j] = k(x_j, z_c), c = (index ? *index : 0) + b + zstep * j, b = blockIdx.y: the lazy kernel
+// of gp_util.py:257-258, same expanded squared distance as the sweeps.  z = x with zstep 0 gives the column
+// of point *index, with zstep 1 the diagonal; z = other points with zstep 0 gives cross-covariance columns.
 template <typename T>
 __global__ void k_gram_elements(int64_t n, int dp, int kind, const T* __restrict__ xs, const T* __restrict__ xx,
-                                const T* __restrict__ consts, const int64_t* __restrict__ index, T* __restrict__ out) {
+                                const T* __restrict__ zs, const T* __restrict__ zz, int64_t zstep,
+                                const T* __restrict__ consts, const int64_t* __restrict__ index, int64_t ldo,
+                                T* __restrict__ out) {
   const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= n) return;
-  const int64_t c = index ? index[0] : j;
+  const int64_t c = (index ? index[0] : 0) + blockIdx.y + zstep * j;
   T dot = T(0);
-  for (int k = 0; k < dp; ++k) dot = fma(xs[j * dp + k], xs[c * dp + k], dot);
-  T s2 = xx[j] + xx[c] - T(2) * dot;
+  for (int k = 0; k < dp; ++k) dot = fma(xs[j * dp + k], zs[c * dp + k], dot);
+  T s2 = xx[j] + zz[c] - T(2) * dot;
   s2 = s2 > T(0) ? s2 : T(0);
   const T sigma = consts[0];
   T val;
@@ -312,17 +322,18 @@ __global__ void k_gram_elements(int64_t n, int dp, int kind, const T* __restrict
     const T s = sqrt(s2 + Eps<T>::v());
     val = kind == 0 ? sigma * (T(1) + s) * exp(-s) : sigma * exp(-s);
   }
-  out[j] = val;
+  out[(int64_t)blockIdx.y * ldo + j] = val;
 }
 
-// y[i] = sum_s part[s][i] + noise * v[i]
+// y[i] = sum_s part[s][i] + noise * v[i]   (noise == nullptr: no noise term -- a cross-covariance, whose
+// v is not indexed by the rows)
 template <typename T>
 __global__ void k_gram_finish(int64_t n, int jsplit, const T* __restrict__ part, const T* __restrict__ noise,
                               const T* __restrict__ v, T* __restrict__ y) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     T s = T(0);
     for (int sp = 0; sp < jsplit; ++sp) s += part[(int64_t)sp * n + i];
-    y[i] = fma(noise[0], v[i], s);
+    y[i] = noise ? fma(noise[0], v[i], s) : s;
   }
 }
 
@@ -411,6 +422,19 @@ __global__ void k_gram_grad_finish_batch(int d, int nblocks, const double* __res
 
 }  // namespace
 
+// Test points of a cross-covariance K(X*, X) (bl_gram_cross_t): scaled and, on the tensor-core path, packed
+// as the row operand with the kernel parameters bound to the parent operator (never its noise).  `binds`
+// records which bind of the parent they were prepared for.
+struct GramOperator;
+struct GramCross {
+  GramOperator* parent = nullptr;
+  int64_t m = 0, mpad = 0;
+  DevBuf X;  // m x d doubles
+  DevBuf xs, xx, consts, opA, part;
+  uint64_t binds = 0;
+  int split = 1;  // column splits of the sweep
+};
+
 struct GramOperator : bl_operator {
   int64_t d = 0;
   int kind = 0;
@@ -420,6 +444,7 @@ struct GramOperator : bl_operator {
   const void* raw_os = nullptr;
   const void* noise = nullptr;
   int bound_dtype = -1;
+  uint64_t binds = 0;  // set_params calls so far (cross objects re-prepare when it moves)
   int jsplit = 1;
   // tensor-core path (fp32, d <= 20): packed TF32 operands, see gram_tc.cuh
   int path = 0;  // 0 = automatic, 1 = FP32 ALU kernel, 2 = tcgen05 kernel
@@ -438,14 +463,20 @@ struct GramOperator : bl_operator {
   // padded point dimension (multiple of 4) and rows per thread
   int dp() const { return d <= 4 ? 4 : d <= 8 ? 8 : d <= 12 ? 12 : d <= 16 ? 16 : 32; }
   int ri() const { return dp() <= 16 ? 4 : 2; }
-  int nblocks_i() const { return (int)((n + (int64_t)kTileI * ri() - 1) / ((int64_t)kTileI * ri())); }
+  int nblocks_for(int64_t rows) const { return (int)((rows + (int64_t)kTileI * ri() - 1) / ((int64_t)kTileI * ri())); }
+  int nblocks_i() const { return nblocks_for(n); }
+  // column splits of the ALU sweep: about four row blocks per SM
+  int jsplit_for(int64_t rows) const {
+    const int nb = nblocks_for(rows);
+    return std::max(1, std::min<int>(64, (4 * sm_count() + nb - 1) / nb));
+  }
 
   template <typename T>
   int set_params_t(cudaStream_t s) {
     BL_CHECK(xs.ensure(((size_t)n + kTileJ) * dp() * sizeof(T)));
     BL_CHECK(xx.ensure(((size_t)n + kTileJ) * sizeof(T)));
     BL_CHECK(consts.ensure(4 * sizeof(T)));
-    jsplit = std::max(1, std::min<int>(64, (4 * sm_count() + nblocks_i() - 1) / nblocks_i()));
+    jsplit = jsplit_for(n);
     const bool tc = use_tc(sizeof(T) == 4 ? BL_F32 : BL_F64);
     if (tc) plan_tc();
     BL_CHECK(part.ensure((size_t)std::max(jsplit, tc_split) * n * sizeof(T)));
@@ -460,18 +491,23 @@ struct GramOperator : bl_operator {
   }
 
   // ---- tensor-core path ------------------------------------------------------------------
-  // column splits: balance waves of one-CTA-per-SM blocks against the per-CTA prologue (~1 tile)
-  void plan_tc() {
-    npad = (n + gramtc::kN - 1) / gramtc::kN * gramtc::kN;
+  // column splits of a sweep over `rowtiles` row tiles: balance waves of one-CTA-per-SM blocks against the
+  // per-CTA prologue (~1 tile)
+  int tc_split_for(int rowtiles) const {
     const int tiles = (int)(npad / gramtc::kN), sms = sm_count();
     double best = 1e300;
-    tc_split = 1;
+    int split = 1;
     for (int sp = 1; sp <= std::min(tiles, 64); ++sp) {
       const int per = (tiles + sp - 1) / sp;
-      const int waves = (tc_rowtiles() * sp + sms - 1) / sms;
+      const int waves = (rowtiles * sp + sms - 1) / sms;
       const double cost = (double)waves * (per + 1.0);
-      if (cost < best - 1e-9) best = cost, tc_split = sp;
+      if (cost < best - 1e-9) best = cost, split = sp;
     }
+    return split;
+  }
+  void plan_tc() {
+    npad = (n + gramtc::kN - 1) / gramtc::kN * gramtc::kN;
+    tc_split = tc_split_for(tc_rowtiles());
   }
   int pack_tc(cudaStream_t s) {
     const int slots = gramtc::slots_for((int)d);
@@ -483,11 +519,13 @@ struct GramOperator : bl_operator {
     BL_LAUNCHED();
     return BL_OK;
   }
-  template <int KIND, bool ADJ, int D>
-  int launch_tc(const float* v, const float* q, float* dbg_out, int dbg_bx, int dbg_by, cudaStream_t s) {
+  // CROSS: rows are the test points of `c`
+  template <int KIND, bool ADJ, int D, bool CROSS = false>
+  int launch_tc(const float* v, const float* q, float* dbg_out, int dbg_bx, int dbg_by, cudaStream_t s,
+                const GramCross* c = nullptr) {
     const int slots = gramtc::slots_for((int)d);
     const gramtc::Plan pl = gramtc::make_plan(slots, ADJ);
-    auto kernel = gramtc::k_gram_tc_sweep<KIND, ADJ, D>;
+    auto kernel = gramtc::k_gram_tc_sweep<KIND, ADJ, D, CROSS>;
     {
       static std::mutex mu;
       static std::map<int, bool> done;
@@ -502,10 +540,14 @@ struct GramOperator : bl_operator {
         done[dev] = true;
       }
     }
-    kernel<<<dim3(tc_rowtiles(), tc_split), gramtc::kThreads, pl.total, s>>>(
-        n, npad, (int)d, slots, opA.as<float>(), opB.as<float>(), xt.as<float>(), xx.as<float>(), consts.as<float>(), v,
-        q,
-        part.as<float>(), gpart.as<double>(), dbg_out, dbg_bx, dbg_by);
+    if (CROSS)
+      kernel<<<dim3((unsigned)(c->mpad / gramtc::kM), c->split), gramtc::kThreads, pl.total, s>>>(
+          n, npad, (int)d, slots, c->opA.as<float>(), opB.as<float>(), nullptr, c->xx.as<float>(), consts.as<float>(), v,
+          nullptr, c->part.as<float>(), nullptr, nullptr, 0, 0, c->m, c->mpad);
+    else
+      kernel<<<dim3(tc_rowtiles(), tc_split), gramtc::kThreads, pl.total, s>>>(
+          n, npad, (int)d, slots, opA.as<float>(), opB.as<float>(), xt.as<float>(), xx.as<float>(), consts.as<float>(), v,
+          q, part.as<float>(), gpart.as<double>(), dbg_out, dbg_bx, dbg_by, n, npad);
     BL_LAUNCHED();
     return BL_OK;
   }
@@ -529,11 +571,7 @@ struct GramOperator : bl_operator {
       BL_CHECK((launch_tc_d<1, ADJ>(v, q, dbg_out, bx, by, s)));
     else
       BL_CHECK((launch_tc_d<2, ADJ>(v, q, dbg_out, bx, by, s)));
-    if (y) {
-      k_gram_finish<float><<<std::min<int>(1024, (int)((n + 255) / 256)), 256, 0, s>>>(
-          n, tc_split, part.as<float>(), static_cast<const float*>(noise), v, y);
-      BL_LAUNCHED();
-    }
+    if (y) BL_CHECK(finish<float>(n, tc_split, part.as<float>(), static_cast<const float*>(noise), v, y, s));
     return BL_OK;
   }
   // ---- deferred parameter cotangent (operators.cuh) ------------------------------------------
@@ -677,15 +715,18 @@ struct GramOperator : bl_operator {
     raw_os = params[1];
     noise = params[2];
     bound_dtype = dtype;
+    ++binds;
     return dtype == BL_F32 ? set_params_t<float>(s) : set_params_t<double>(s);
   }
 
-  template <typename T, int DP, int RI, bool ADJ>
-  void launch_sweep(const T* v, const T* q, cudaStream_t s) {
-    dim3 grid(nblocks_i(), jsplit);
-#define BL_GRAM_LAUNCH(KIND)                                                                                  \
-  k_gram_sweep<T, DP, RI, ADJ, KIND><<<grid, kTileI, 0, s>>>(n, (int)d, xs.as<T>(), xx.as<T>(), consts.as<T>(), v, \
-                                                             q, part.as<T>(), gpart.as<double>())
+  // CROSS: rows are the test points of `c`
+  template <typename T, int DP, int RI, bool ADJ, bool CROSS = false>
+  void launch_sweep(const T* v, const T* q, cudaStream_t s, const GramCross* c = nullptr) {
+    dim3 grid(CROSS ? nblocks_for(c->m) : nblocks_i(), CROSS ? c->split : jsplit);
+#define BL_GRAM_LAUNCH(KIND)                                                                                        \
+  k_gram_sweep<T, DP, RI, ADJ, KIND, CROSS><<<grid, kTileI, 0, s>>>(                                                \
+      n, (int)d, xs.as<T>(), xx.as<T>(), consts.as<T>(), v, q, (CROSS ? c->part : part).template as<T>(),            \
+      gpart.as<double>(), CROSS ? c->m : n, (CROSS ? c->xs : xs).template as<T>(), (CROSS ? c->xx : xx).template as<T>())
     if (kind == 0)
       BL_GRAM_LAUNCH(0);
     else if (kind == 1)
@@ -695,21 +736,25 @@ struct GramOperator : bl_operator {
 #undef BL_GRAM_LAUNCH
   }
 
-  template <typename T, bool ADJ>
-  int sweep(const T* v, const T* q, T* y, cudaStream_t s) {
+  template <typename T, bool ADJ, bool CROSS = false>
+  int sweep(const T* v, const T* q, T* y, cudaStream_t s, const GramCross* c = nullptr) {
     switch (dp()) {
-      case 4: launch_sweep<T, 4, 4, ADJ>(v, q, s); break;
-      case 8: launch_sweep<T, 8, 4, ADJ>(v, q, s); break;
-      case 12: launch_sweep<T, 12, 4, ADJ>(v, q, s); break;
-      case 16: launch_sweep<T, 16, 4, ADJ>(v, q, s); break;
-      default: launch_sweep<T, 32, 2, ADJ>(v, q, s); break;
+      case 4: launch_sweep<T, 4, 4, ADJ, CROSS>(v, q, s, c); break;
+      case 8: launch_sweep<T, 8, 4, ADJ, CROSS>(v, q, s, c); break;
+      case 12: launch_sweep<T, 12, 4, ADJ, CROSS>(v, q, s, c); break;
+      case 16: launch_sweep<T, 16, 4, ADJ, CROSS>(v, q, s, c); break;
+      default: launch_sweep<T, 32, 2, ADJ, CROSS>(v, q, s, c); break;
     }
     BL_LAUNCHED();
-    if (y) {
-      k_gram_finish<T><<<std::min<int>(1024, (int)((n + 255) / 256)), 256, 0, s>>>(
-          n, jsplit, part.as<T>(), static_cast<const T*>(noise), v, y);
-      BL_LAUNCHED();
-    }
+    if (y) BL_CHECK(finish<T>(CROSS ? c->m : n, CROSS ? c->split : jsplit, (CROSS ? c->part : part).template as<T>(),
+                              CROSS ? nullptr : static_cast<const T*>(noise), v, y, s));
+    return BL_OK;
+  }
+  // y = sum of the column splits' partial products (+ noise v for the square operator: noise != nullptr)
+  template <typename T>
+  int finish(int64_t rows, int split, const T* partp, const T* noisep, const T* v, T* y, cudaStream_t s) {
+    k_gram_finish<T><<<std::min<int>(1024, (int)((rows + 255) / 256)), 256, 0, s>>>(rows, split, partp, noisep, v, y);
+    BL_LAUNCHED();
     return BL_OK;
   }
 
@@ -740,21 +785,91 @@ struct GramOperator : bl_operator {
                            : vjp_t<double>((const double*)q, (const double*)lam, (double*)z, s);
   }
 
-  int elements(int dtype, const int64_t* index, void* out, cudaStream_t s) {
-    BL_REQUIRE(dtype == bound_dtype, "set_params must be called with the same dtype first");
-    const int blocks = (int)((n + 255) / 256);
-    if (dtype == BL_F32)
-      k_gram_elements<float><<<blocks, 256, 0, s>>>(n, dp(), kind, xs.as<float>(), xx.as<float>(), consts.as<float>(),
-                                                    index, static_cast<float*>(out));
-    else
-      k_gram_elements<double><<<blocks, 256, 0, s>>>(n, dp(), kind, xs.as<double>(), xx.as<double>(),
-                                                     consts.as<double>(), index, static_cast<double*>(out));
+  // out[b][j] = k(x_j, z_c) for the `rows` points x, b < count (k_gram_elements)
+  template <typename T>
+  int elements_t(int64_t rows, const DevBuf& xsb, const DevBuf& xxb, const T* zs, const T* zz, int64_t zstep,
+                 const int64_t* index, int64_t count, int64_t ldo, T* out, cudaStream_t s) {
+    k_gram_elements<T><<<dim3((unsigned)((rows + 255) / 256), (unsigned)count), 256, 0, s>>>(
+        rows, dp(), kind, xsb.as<T>(), xxb.as<T>(), zs, zz, zstep, consts.as<T>(), index, ldo, out);
     BL_LAUNCHED();
     return BL_OK;
+  }
+  int elements(int dtype, const int64_t* index, void* out, cudaStream_t s) {
+    BL_REQUIRE(dtype == bound_dtype, "set_params must be called with the same dtype first");
+    const int64_t zstep = index ? 0 : 1;
+    if (dtype == BL_F32)
+      return elements_t<float>(n, xs, xx, xs.as<float>(), xx.as<float>(), zstep, index, 1, n, static_cast<float*>(out), s);
+    return elements_t<double>(n, xs, xx, xs.as<double>(), xx.as<double>(), zstep, index, 1, n, static_cast<double*>(out), s);
   }
   int element_diagonal(int dtype, void* out, cudaStream_t s) override { return elements(dtype, nullptr, out, s); }
   int element_column(int dtype, const int64_t* index, void* out, cudaStream_t s) override {
     return elements(dtype, index, out, s);
+  }
+
+  // ---- cross-covariance with the test points of a GramCross ------------------------------------
+  template <typename T>
+  int cross_prepare_t(GramCross& c, cudaStream_t s) {
+    const int64_t m = c.m;
+    BL_CHECK(c.xs.ensure((size_t)m * dp() * sizeof(T)));
+    BL_CHECK(c.xx.ensure((size_t)m * sizeof(T)));
+    BL_CHECK(c.consts.ensure(4 * sizeof(T)));  // k_gram_prepare's copy of the outputscale (the sweeps read the parent's)
+    k_gram_prepare<T><<<std::min<int>(1024, (int)((m + 255) / 256)), 256, 0, s>>>(
+        m, (int)d, dp(), kind, c.X.as<double>(), static_cast<const T*>(raw_ls), static_cast<const T*>(raw_os),
+        c.xs.as<T>(), c.xx.as<T>(), c.consts.as<T>());
+    BL_LAUNCHED();
+    if (use_tc(sizeof(T) == 4 ? BL_F32 : BL_F64)) {
+      const int slots = gramtc::slots_for((int)d);
+      c.mpad = (m + gramtc::kM - 1) / gramtc::kM * gramtc::kM;
+      c.split = tc_split_for((int)(c.mpad / gramtc::kM));
+      BL_CHECK(c.opA.ensure((size_t)c.mpad * slots * sizeof(float)));
+      gramtc::k_gram_tc_pack<<<std::min<int>(1024, (int)((c.mpad + 127) / 128)), 128, 0, s>>>(
+          m, c.mpad, (int)d, dp(), slots, c.xs.as<float>(), c.xx.as<float>(), c.opA.as<float>(), nullptr, nullptr);
+      BL_LAUNCHED();
+    } else {
+      c.split = jsplit_for(m);
+    }
+    BL_CHECK(c.part.ensure((size_t)c.split * m * sizeof(T)));
+    c.binds = binds;
+    return BL_OK;
+  }
+  int cross_prepare(GramCross& c, int dtype, cudaStream_t s) {
+    BL_REQUIRE(dtype == bound_dtype, "bind the parent gram operator with the same dtype first");
+    if (c.binds == binds) return BL_OK;
+    return dtype == BL_F32 ? cross_prepare_t<float>(c, s) : cross_prepare_t<double>(c, s);
+  }
+  // y (m) = K(X*, X) v (n): no noise term
+  int cross_matvec(GramCross& c, int dtype, const void* v, void* y, cudaStream_t s) {
+    BL_CHECK(cross_prepare(c, dtype, s));
+    if (use_tc(dtype)) {
+      const float* vf = static_cast<const float*>(v);
+      if (kind == 0)
+        BL_CHECK((launch_tc<0, false, 1, true>(vf, nullptr, nullptr, 0, 0, s, &c)));
+      else if (kind == 1)
+        BL_CHECK((launch_tc<1, false, 1, true>(vf, nullptr, nullptr, 0, 0, s, &c)));
+      else
+        BL_CHECK((launch_tc<2, false, 1, true>(vf, nullptr, nullptr, 0, 0, s, &c)));
+      return finish<float>(c.m, c.split, c.part.as<float>(), nullptr, vf, static_cast<float*>(y), s);
+    }
+    return dtype == BL_F32 ? sweep<float, false, true>((const float*)v, nullptr, (float*)y, s, &c)
+                           : sweep<double, false, true>((const double*)v, nullptr, (double*)y, s, &c);
+  }
+  // out[b][j] = k(x*_{first+b}, x_j), b < count, row stride ldo
+  int cross_columns(GramCross& c, int dtype, int64_t first, int64_t count, void* out, int64_t ldo, cudaStream_t s) {
+    BL_CHECK(cross_prepare(c, dtype, s));
+    if (dtype == BL_F32)
+      return elements_t<float>(n, xs, xx, c.xs.as<float>() + first * dp(), c.xx.as<float>() + first, 0, nullptr, count,
+                               ldo, static_cast<float*>(out), s);
+    return elements_t<double>(n, xs, xx, c.xs.as<double>() + first * dp(), c.xx.as<double>() + first, 0, nullptr, count,
+                              ldo, static_cast<double*>(out), s);
+  }
+  // out[t] = k(x*_t, x*_t): the kernel formula at s2 = 0
+  int cross_prior_diag(GramCross& c, int dtype, void* out, cudaStream_t s) {
+    BL_CHECK(cross_prepare(c, dtype, s));
+    if (dtype == BL_F32)
+      return elements_t<float>(c.m, c.xs, c.xx, c.xs.as<float>(), c.xx.as<float>(), 1, nullptr, 1, c.m,
+                               static_cast<float*>(out), s);
+    return elements_t<double>(c.m, c.xs, c.xx, c.xs.as<double>(), c.xx.as<double>(), 1, nullptr, 1, c.m,
+                              static_cast<double*>(out), s);
   }
 
   int grad_zero(int dtype, cudaStream_t s) override {
@@ -775,6 +890,10 @@ struct GramOperator : bl_operator {
 };
 
 }  // namespace bl
+
+struct bl_gram_cross {
+  bl::GramCross cross;
+};
 
 extern "C" int bl_op_gram_set_path(bl_operator_t* op, int path) {
   auto* o = dynamic_cast<bl::GramOperator*>(op);
@@ -810,4 +929,47 @@ extern "C" int bl_op_gram_create(int64_t n, int64_t d, int kind, const double* X
   }
   *op = o;
   return BL_OK;
+}
+
+extern "C" int bl_gram_cross_create(bl_operator_t* gram, int64_t m, const double* Xtest_host, bl_gram_cross_t** out) {
+  auto* g = dynamic_cast<bl::GramOperator*>(gram);
+  BL_REQUIRE(g != nullptr && out && Xtest_host && m > 0, "bad gram cross arguments (a gram operator and m >= 1 test points)");
+  auto* c = new bl_gram_cross();
+  c->cross.parent = g;
+  c->cross.m = m;
+  int rc = c->cross.X.ensure((size_t)m * g->d * sizeof(double));
+  if (rc == BL_OK &&
+      cudaMemcpy(c->cross.X.p, Xtest_host, (size_t)m * g->d * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess) {
+    bl::set_error("cudaMemcpy of the test points failed");
+    rc = BL_ECUDA;
+  }
+  if (rc != BL_OK) {
+    delete c;
+    return rc;
+  }
+  *out = c;
+  return BL_OK;
+}
+
+extern "C" int bl_gram_cross_destroy(bl_gram_cross_t* c) {
+  delete c;
+  return BL_OK;
+}
+
+extern "C" int bl_gram_cross_matvec(bl_gram_cross_t* c, int dtype, const void* v, void* y, void* stream) {
+  BL_REQUIRE(c && v && y, "bad gram cross matvec arguments");
+  return c->cross.parent->cross_matvec(c->cross, dtype, v, y, bl::as_stream(stream));
+}
+
+extern "C" int bl_gram_cross_columns(bl_gram_cross_t* c, int dtype, int64_t first, int64_t count, void* out, int64_t ld,
+                                     void* stream) {
+  BL_REQUIRE(c && out && first >= 0 && count >= 1 && first + count <= c->cross.m && count <= 65535 &&
+                 ld >= c->cross.parent->n,
+             "bad gram cross columns arguments (0 <= first, first + count <= m, count <= 65535, ld >= n)");
+  return c->cross.parent->cross_columns(c->cross, dtype, first, count, out, ld, bl::as_stream(stream));
+}
+
+extern "C" int bl_gram_cross_prior_diag(bl_gram_cross_t* c, int dtype, void* out, void* stream) {
+  BL_REQUIRE(c && out, "bad gram cross prior diagonal arguments");
+  return c->cross.parent->cross_prior_diag(c->cross, dtype, out, bl::as_stream(stream));
 }

@@ -122,6 +122,7 @@ __device__ __forceinline__ float rsqf(float x) {
 // xs [n][dp] (scaled inputs), xx [n] (squared norms, same values as the ALU kernel uses)
 //   -> opA / opB [slots/4][npad][4]   (points >= n are zero rows)
 //   -> xt [kXtRows][npad]             (transposed fp32 coordinates for the adjoint epilogue)
+// opB == nullptr: only the row operand and no xt (the test points of a cross-covariance sweep)
 __global__ void k_gram_tc_pack(int64_t n, int64_t npad, int d, int dp, int slots, const float* __restrict__ xs,
                                const float* __restrict__ xx, float* __restrict__ opA, float* __restrict__ opB,
                                float* __restrict__ xt) {
@@ -150,9 +151,10 @@ __global__ void k_gram_tc_pack(int64_t n, int64_t npad, int d, int dp, int slots
       va.x = a[4 * c], va.y = a[4 * c + 1], va.z = a[4 * c + 2], va.w = a[4 * c + 3];
       vb.x = b[4 * c], vb.y = b[4 * c + 1], vb.z = b[4 * c + 2], vb.w = b[4 * c + 3];
       reinterpret_cast<float4*>(opA)[(int64_t)c * npad + i] = va;
-      reinterpret_cast<float4*>(opB)[(int64_t)c * npad + i] = vb;
+      if (opB) reinterpret_cast<float4*>(opB)[(int64_t)c * npad + i] = vb;
     }
-    for (int k = 0; k < kXtRows; ++k) xt[(int64_t)k * npad + i] = (live && k < d) ? xs[i * dp + k] : 0.f;
+    if (opB)
+      for (int k = 0; k < kXtRows; ++k) xt[(int64_t)k * npad + i] = (live && k < d) ? xs[i * dp + k] : 0.f;
   }
 }
 
@@ -321,15 +323,16 @@ struct RaggedRow {
 };
 
 // warp 0.  Aux: `bool ragged(jt)`, `void fill(float* aux, jt, lane)`, `uint32_t bytes(jt)`,
-// `void issue(float* aux, jt, bar)` for the auxiliary rows of one stage.
+// `void issue(float* aux, jt, bar)` for the auxiliary rows of one stage.  opA has `apad` points per slot
+// chunk, opB `npad` (the same number unless the rows are another point set than the columns).
 template <class Aux>
-__device__ __forceinline__ void producer_warp(const Pipe& p, const float* __restrict__ opA,
+__device__ __forceinline__ void producer_warp(const Pipe& p, const float* __restrict__ opA, int64_t apad,
                                               const float* __restrict__ opB, int64_t npad, const Aux& aux) {
   const int lane = threadIdx.x & 31;
   if (lane == 0 && p.ntiles > 0) {
     tma::mbar_arrive_expect_tx(p.a_full, p.pl.a_bytes);
     for (int c = 0; c < 2 * p.pl.ksteps; ++c)
-      tma::bulk_g2s(p.smA + (size_t)c * kM * 16, opA + ((int64_t)c * npad + p.i0) * 4, kM * 16, p.a_full);
+      tma::bulk_g2s(p.smA + (size_t)c * kM * 16, opA + ((int64_t)c * apad + p.i0) * 4, kM * 16, p.a_full);
   }
   for (int it = 0; it < p.ntiles; ++it) {
     const Slot sl = slot_of(p, it);
@@ -408,12 +411,14 @@ __device__ __forceinline__ void epi_release(const Pipe& p, const Slot& sl) {
   }
 }
 // 32 accumulator columns (col0 ..) of this thread's row; on tiles that hold pairs with i == j the
-// diagonal entry is replaced by the value that makes s2 exactly zero
+// diagonal entry is replaced by the value that makes s2 exactly zero.  DIAG == false (rows and columns
+// are different point sets): no replacement.
+template <bool DIAG = true>
 __device__ __forceinline__ void epi_load(const Pipe& p, const EpiThread& e, const Slot& sl, int it, int col0,
                                          uint32_t (&r)[32]) {
   tmem_ld32(p.tmem_base + ((uint32_t)(e.qd * 32) << 16) + (uint32_t)(sl.b * kN + col0), r);
   const int64_t jt = (p.t0 + it) * kN;
-  if (jt < p.i0 + kM && p.i0 < jt + kN) {
+  if (DIAG && jt < p.i0 + kM && p.i0 < jt + kN) {
     const int jd = (int)(p.i0 + e.row - jt) - col0;  // column of this chunk with j == i (if any)
 #pragma unroll
     for (int c = 0; c < 32; ++c) r[c] = c == jd ? e.acc_diag : r[c];
@@ -496,22 +501,28 @@ struct RowsAux {
 //                 gpart[cta][d]  = sum lam_i q_j k_ij               (k includes sigma)
 //                 gpart[cta][k]  = sum lam_i q_j dk_ij (x_ik - x_jk)^2,  k < d
 // dbg != nullptr: CTA (dbg_bx, dbg_by) writes the raw accumulator (x.y - |y|^2/2) of its first tile to dbg[128][256].
-template <int KIND, bool ADJ, int D>
+// CROSS == true: the rows are another point set (a cross-covariance K(X*, X) v): m rows packed in opA with
+// mpad points per slot chunk, xx = their squared norms, part[split][m]; the columns stay the n points of opB.
+// Only the square sweep replaces the diagonal (it is exact only where the row and the column are one point).
+template <int KIND, bool ADJ, int D, bool CROSS = false>
 __global__ void __launch_bounds__(kThreads, 1)
 k_gram_tc_sweep(int64_t n, int64_t npad, int d, int slots, const float* __restrict__ opA,
                 const float* __restrict__ opB, const float* __restrict__ xt, const float* __restrict__ xx,
                 const float* __restrict__ consts, const float* __restrict__ v, const float* __restrict__ q,
-                float* __restrict__ part, double* __restrict__ gpart, float* __restrict__ dbg, int dbg_bx, int dbg_by) {
+                float* __restrict__ part, double* __restrict__ gpart, float* __restrict__ dbg, int dbg_bx, int dbg_by,
+                int64_t m, int64_t mpad) {
+  static_assert(!(CROSS && ADJ), "the cross-covariance sweep has no adjoint");
   extern __shared__ __align__(1024) uint8_t smem[];
   __shared__ double ycomb[kM];
+  const int64_t rows = CROSS ? m : n;
   const Pipe p = pipe_setup(smem, make_plan(slots, ADJ), n);
   const int warp = threadIdx.x >> 5;
   if (warp == 0) {
-    producer_warp(p, opA, opB, npad, SweepAux<ADJ, D>{RaggedRow{v, n}, RaggedRow{q, n}, xt, npad});
+    producer_warp(p, opA, CROSS ? mpad : npad, opB, npad, SweepAux<ADJ, D>{RaggedRow{v, n}, RaggedRow{q, n}, xt, npad});
   } else if (warp == 1) {
     mma_warp(p);
   } else {
-    const EpiThread e = epi_thread<KIND>(p, n, xx);
+    const EpiThread e = epi_thread<KIND>(p, rows, xx);
     double yacc = 0.0, uacc = 0.0, dacc[ADJ ? D : 1];
     float2 nxi[ADJ ? D : 1];  // (-x_ik, -x_ik)
 #pragma unroll
@@ -538,7 +549,7 @@ k_gram_tc_sweep(int64_t n, int64_t npad, int d, int slots, const float* __restri
 #pragma unroll
           for (int c = 0; c < 32; ++c) dbg[(size_t)e.row * kN + col0 + c] = __uint_as_float(r[c]);
         }
-        epi_load(p, e, sl, it, col0, r);
+        epi_load<!CROSS>(p, e, sl, it, col0, r);
 #pragma unroll
         for (int pp = 0; pp < 8; ++pp) {
           const float4 v4 = *reinterpret_cast<const float4*>(smV + col0 + 4 * pp);
@@ -577,7 +588,7 @@ k_gram_tc_sweep(int64_t n, int64_t npad, int d, int slots, const float* __restri
     const double sigma = (double)consts[0];
     if (e.half == 1) ycomb[e.row] = yacc;
     tma::named_bar_sync(1, kEpiWarps * 32);
-    if (e.half == 0 && e.live) part[(int64_t)blockIdx.y * n + p.i0 + e.row] = (float)((yacc + ycomb[e.row]) * sigma);
+    if (e.half == 0 && e.live) part[(int64_t)blockIdx.y * rows + p.i0 + e.row] = (float)((yacc + ycomb[e.row]) * sigma);
     if (ADJ) {
       const double li = e.live ? (double)v[p.i0 + e.row] * sigma : 0.0;
 #pragma unroll
@@ -606,7 +617,7 @@ k_gram_tc_gradbatch(int64_t n, int64_t npad, int d, int slots, const float* __re
   if (warp == 0) {
     RowsAux<D> aux{{}, M, n, xt, npad};
     for (int m = 0; m < M; ++m) aux.rows.p[m] = Qrows + (int64_t)m * ldq;
-    producer_warp(p, opA, opB, npad, aux);
+    producer_warp(p, opA, npad, opB, npad, aux);
   } else if (warp == 1) {
     mma_warp(p);
   } else {
@@ -692,7 +703,7 @@ k_gram_tc_multi(int64_t n, int64_t npad, int slots, const float* __restrict__ op
   const Pipe p = pipe_setup(smem, make_plan_multi(slots), n);
   const int warp = threadIdx.x >> 5;
   if (warp == 0) {
-    producer_warp(p, opA, opB, npad, RowsAux<1>{vecs, P, n, nullptr, npad});
+    producer_warp(p, opA, npad, opB, npad, RowsAux<1>{vecs, P, n, nullptr, npad});
   } else if (warp == 1) {
     mma_warp(p);
   } else {

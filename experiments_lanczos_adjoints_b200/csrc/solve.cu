@@ -9,9 +9,12 @@
 // Everything stays on the stream: step lengths, residual norms, the convergence flag, the pivot
 // permutation and the pivot index live in device memory; every kernel that reduces ends with the
 // deterministic "partials + last block" scheme and lets that last block update the scalars.  The
-// fixed-step solver never synchronises; the adaptive one reads ONE flag back every `check_every`
+// fixed-step solver never synchronises; the adaptive one reads the flags back every `check_every`
 // iterations (iterations after convergence are frozen on the device, so the result is the state at
-// exactly the iteration where the reference's while_loop stops).
+// exactly the iteration where the reference's while_loop stops).  Several right-hand sides run in
+// lockstep as columns of one grid (blockIdx.y = column, each with its own scalars): every column follows
+// exactly the rules of a single solve.
+#include <climits>
 #include <cmath>
 #include <vector>
 
@@ -43,13 +46,14 @@ __device__ __forceinline__ T safe_divide(T a, T b) {
 
 int grid_for(int64_t n) { return (int)std::max<int64_t>(1, std::min<int64_t>(kMaxGrid, (n + kThreads - 1) / kThreads)); }
 
-// block partial -> partials[blockIdx.x]; returns true in the last block with the total in *total
+// block partial -> partials[blockIdx.x]; returns true in the last block (of this column's gridDim.x blocks)
+// with the total in *total
 __device__ __forceinline__ bool reduce_to_last(double v, double* partials, unsigned int* counter, double* total) {
   __shared__ double red[32];
   __shared__ double tot;
   double s = block_sum(v, red);
   if (threadIdx.x == 0) partials[blockIdx.x] = s;
-  if (!last_block_done(counter)) return false;
+  if (!last_block_done(counter, gridDim.x)) return false;
   double acc = 0.0;
   for (int b = threadIdx.x; b < (int)gridDim.x; b += blockDim.x) acc += partials[b];
   acc = block_sum(acc, red);
@@ -59,21 +63,39 @@ __device__ __forceinline__ bool reduce_to_last(double v, double* partials, unsig
   return true;
 }
 
-enum DotMode { DOT_INIT = 0, DOT_PAP = 1, DOT_RZ = 2, DOT_PLAIN = 3 };
+enum DotMode { DOT_INIT = 0, DOT_PAP = 1, DOT_RZ = 2 };
+
+// Column c = blockIdx.y of a lockstep solve: its vectors start at row c (stride ld), its scalars, block
+// partials and counter are its own.
+struct Column {
+  int64_t off;
+  double* scal;
+  double* partials;
+  unsigned int* counter;
+};
+__device__ __forceinline__ Column column_of(int64_t ld, double* scal, double* partials, unsigned int* counter) {
+  const int c = blockIdx.y;
+  return Column{(int64_t)c * ld, scal + (size_t)c * S_N, partials + (size_t)c * kMaxGrid, counter + c};
+}
 
 // d = <x, y>, then (last block):
 //   DOT_INIT : rz = d                                          cg.py:31-33 (the first dot(r, z))
 //   DOT_PAP  : alpha = safe_divide(rz, d)                      cg.py:46
 //   DOT_RZ   : beta = safe_divide(d, rz); rz = d               cg.py:55
+// DOT_PAP / DOT_RZ of a frozen column are skipped: nothing reads their results any more.
 template <typename T>
-__global__ void __launch_bounds__(kThreads) k_cg_dot(int64_t n, const T* __restrict__ x, const T* __restrict__ y,
-                                                       double* partials, unsigned int* counter, double* scal, int mode,
-                                                       T* out) {
+__global__ void __launch_bounds__(kThreads) k_cg_dot(int64_t n, int64_t ld, const T* __restrict__ x,
+                                                       const T* __restrict__ y, double* partials, unsigned int* counter,
+                                                       double* scal_all, int mode) {
+  const Column col = column_of(ld, scal_all, partials, counter);
+  double* scal = col.scal;
+  if (mode != DOT_INIT && scal[S_ACTIVE] == 0.0) return;  // uniform over the column's blocks
+  x += col.off, y += col.off;
   double acc = 0.0;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
     acc += static_cast<double>(x[i]) * static_cast<double>(y[i]);
   double d;
-  if (!reduce_to_last(acc, partials, counter, &d)) return;
+  if (!reduce_to_last(acc, col.partials, col.counter, &d)) return;
   if (threadIdx.x != 0) return;
   const T dt = static_cast<T>(d);
   if (mode == DOT_INIT) {
@@ -81,11 +103,9 @@ __global__ void __launch_bounds__(kThreads) k_cg_dot(int64_t n, const T* __restr
   } else if (mode == DOT_PAP) {
     scal[S_PAP] = dt;
     scal[S_ALPHA] = safe_divide<T>(static_cast<T>(scal[S_RZ]), dt);
-  } else if (mode == DOT_RZ) {
+  } else {
     scal[S_BETA] = safe_divide<T>(dt, static_cast<T>(scal[S_RZ]));
     scal[S_RZ] = dt;
-  } else if (out) {
-    out[0] = dt;
   }
 }
 
@@ -93,9 +113,12 @@ __global__ void __launch_bounds__(kThreads) k_cg_dot(int64_t n, const T* __restr
 // frozen (no update) once the convergence flag of the previous iteration is down.
 template <typename T>
 __global__ void __launch_bounds__(kThreads)
-k_cg_update_xr(int64_t n, const T* __restrict__ p, const T* __restrict__ Ap, T* __restrict__ x, T* __restrict__ r,
-               double atol, double rtol, long long miniter, long long maxiter, double* partials, unsigned int* counter,
-               double* scal) {
+k_cg_update_xr(int64_t n, int64_t ld, const T* __restrict__ p, const T* __restrict__ Ap, T* __restrict__ x,
+               T* __restrict__ r, double atol, double rtol, long long miniter, long long maxiter, double* partials,
+               unsigned int* counter, double* scal_all) {
+  const Column col = column_of(ld, scal_all, partials, counter);
+  double* scal = col.scal;
+  p += col.off, Ap += col.off, x += col.off, r += col.off;
   const bool active = scal[S_ACTIVE] != 0.0;
   const bool adaptive = atol >= 0.0;
   if (!active) return;  // every block takes the same branch: the flag only changes in the last block below
@@ -112,7 +135,7 @@ k_cg_update_xr(int64_t n, const T* __restrict__ p, const T* __restrict__ Ap, T* 
     }
   }
   double tot;
-  if (!reduce_to_last(acc, partials, counter, &tot)) return;
+  if (!reduce_to_last(acc, col.partials, col.counter, &tot)) return;
   if (threadIdx.x != 0) return;
   const double steps = scal[S_NSTEPS] + 1.0;
   scal[S_NSTEPS] = steps;
@@ -126,8 +149,11 @@ k_cg_update_xr(int64_t n, const T* __restrict__ p, const T* __restrict__ Ap, T* 
 // the cond of the adaptive loop on the initial state x = 0, r = b            cg.py:104-113
 template <typename T>
 __global__ void __launch_bounds__(kThreads)
-k_cg_init(int64_t n, const T* __restrict__ b, T* __restrict__ x, T* __restrict__ r, double atol, long long miniter,
-          long long maxiter, double* partials, unsigned int* counter, double* scal) {
+k_cg_init(int64_t n, int64_t ld, const T* __restrict__ b, T* __restrict__ x, T* __restrict__ r, double atol,
+          long long miniter, long long maxiter, double* partials, unsigned int* counter, double* scal_all) {
+  const Column col = column_of(ld, scal_all, partials, counter);
+  double* scal = col.scal;
+  b += col.off, x += col.off, r += col.off;
   double acc = 0.0;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     x[i] = T(0);
@@ -138,7 +164,7 @@ k_cg_init(int64_t n, const T* __restrict__ b, T* __restrict__ x, T* __restrict__
     }
   }
   double tot;
-  if (!reduce_to_last(acc, partials, counter, &tot)) return;
+  if (!reduce_to_last(acc, col.partials, col.counter, &tot)) return;
   if (threadIdx.x != 0) return;
   scal[S_NSTEPS] = 0.0;
   scal[S_ERR2] = tot;
@@ -150,8 +176,11 @@ k_cg_init(int64_t n, const T* __restrict__ b, T* __restrict__ x, T* __restrict__
 
 // p = z + beta p   (beta == nullptr: p = z)                                  cg.py:56, 34
 template <typename T>
-__global__ void __launch_bounds__(kThreads) k_cg_update_p(int64_t n, const T* __restrict__ z, T* __restrict__ p,
-                                                            const double* scal, bool first) {
+__global__ void __launch_bounds__(kThreads) k_cg_update_p(int64_t n, int64_t ld, const T* __restrict__ z,
+                                                            T* __restrict__ p, const double* scal_all, bool first) {
+  const int64_t off = (int64_t)blockIdx.y * ld;
+  const double* scal = scal_all + (size_t)blockIdx.y * S_N;
+  z += off, p += off;
   if (!first && scal[S_ACTIVE] == 0.0) return;
   const T b = first ? T(0) : static_cast<T>(scal[S_BETA]);
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
@@ -159,12 +188,14 @@ __global__ void __launch_bounds__(kThreads) k_cg_update_p(int64_t n, const T* __
 }
 
 // ---- low-rank preconditioner ------------------------------------------------------------------
-// t[k] = <L_k, v>  (one block per row k; L_k = k-th column of the factor, stored as a row of length n)
+// t[k] = <L_k, v_k>  (one block per row k; L_k = k-th column of the factor, stored as a row of length n;
+// ldv = 0: one vector v for every row)
 template <typename T>
 __global__ void __launch_bounds__(kThreads) k_rows_dot(int64_t n, const T* __restrict__ L, int64_t ld,
-                                                         const T* __restrict__ v, double* __restrict__ t) {
+                                                         const T* __restrict__ v, int64_t ldv, double* __restrict__ t) {
   __shared__ double red[32];
   const T* row = L + (int64_t)blockIdx.x * ld;
+  v += (int64_t)blockIdx.x * ldv;
   double acc = 0.0;
   for (int64_t i = threadIdx.x; i < n; i += blockDim.x) acc += static_cast<double>(row[i]) * static_cast<double>(v[i]);
   acc = block_sum(acc, red);
@@ -366,7 +397,7 @@ int spd_inverse(std::vector<double>& a, int r) {
 template <typename T>
 int precond_apply_t(bl_precond* p, const T* v, T* out, cudaStream_t s) {
   const int r = (int)p->rank;
-  k_rows_dot<T><<<r, kThreads, 0, s>>>(p->n, static_cast<const T*>(p->L), p->ld, v, p->t.as<double>());
+  k_rows_dot<T><<<r, kThreads, 0, s>>>(p->n, static_cast<const T*>(p->L), p->ld, v, 0, p->t.as<double>());
   BL_LAUNCHED();
   k_small_matvec<<<1, kThreads, 0, s>>>(r, p->M.as<double>(), p->t.as<double>(), p->w.as<double>());
   BL_LAUNCHED();
@@ -376,61 +407,73 @@ int precond_apply_t(bl_precond* p, const T* v, T* out, cudaStream_t s) {
   return BL_OK;
 }
 
+// `count` columns of n values, row stride ld, in lockstep (count == 1: bl_pcg_solve)
 template <typename T>
-int pcg_t(bl_operator* op, int dtype, int64_t n, const T* b, bl_precond* pre, int64_t max_steps, int64_t min_steps,
-          double atol, double rtol, int check_every, T* x, T* r, int64_t* num_steps_host, void* workspace,
-          size_t workspace_bytes, cudaStream_t s) {
+int pcg_t(bl_operator* op, int dtype, int64_t n, int64_t count, int64_t ld, const T* b, bl_precond* pre,
+          int64_t max_steps, int64_t min_steps, double atol, double rtol, int check_every, T* x, T* r,
+          int64_t* num_steps_host, void* workspace, size_t workspace_bytes, cudaStream_t s) {
   Carve w{static_cast<char*>(workspace), workspace_bytes};
-  double* scal = static_cast<double*>(w.take(S_N * 8));
-  double* partials = static_cast<double*>(w.take(kMaxGrid * 8));
-  unsigned int* counter = static_cast<unsigned int*>(w.take(256));
-  T* p = static_cast<T*>(w.take((size_t)n * sizeof(T)));
-  T* Ap = static_cast<T*>(w.take((size_t)n * sizeof(T)));
-  T* z = pre ? static_cast<T*>(w.take((size_t)n * sizeof(T))) : nullptr;
+  double* scal = static_cast<double*>(w.take((size_t)count * S_N * 8));
+  double* partials = static_cast<double*>(w.take((size_t)count * kMaxGrid * 8));
+  unsigned int* counter = static_cast<unsigned int*>(w.take((size_t)count * 4));
+  T* p = static_cast<T*>(w.take((size_t)count * ld * sizeof(T)));
+  T* Ap = static_cast<T*>(w.take((size_t)count * ld * sizeof(T)));
+  T* z = pre ? static_cast<T*>(w.take((size_t)count * ld * sizeof(T))) : nullptr;
   BL_REQUIRE(scal && partials && counter && p && Ap && (!pre || z), "pcg workspace too small");
-  BL_CUDA(cudaMemsetAsync(workspace, 0, 256 * 3 + kMaxGrid * 8, s));
-  const int g = grid_for(n);
+  BL_CUDA(cudaMemsetAsync(workspace, 0, reinterpret_cast<char*>(p) - static_cast<char*>(workspace), s));
+  const dim3 g(grid_for(n), (unsigned)count);
   const bool adaptive = atol >= 0.0;
-  k_cg_init<T><<<g, kThreads, 0, s>>>(n, b, x, r, atol, (long long)min_steps, (long long)max_steps, partials, counter, scal);
+  std::vector<int64_t> live((size_t)count);  // columns not yet seen frozen by the host
+  for (int64_t c = 0; c < count; ++c) live[c] = c;
+  std::vector<const void*> in;
+  std::vector<void*> out;
+  k_cg_init<T><<<g, kThreads, 0, s>>>(n, ld, b, x, r, atol, (long long)min_steps, (long long)max_steps, partials,
+                                      counter, scal);
   BL_LAUNCHED();
-  auto precond = [&](const T* in) -> const T* {  // z = P(r)
-    if (!pre) return in;
-    if (precond_apply_t<T>(pre, in, z, s) != BL_OK) return nullptr;
-    return z;
+  auto precond = [&]() -> int {  // z = P(r) for the live columns
+    for (int64_t c : live) BL_CHECK(precond_apply_t<T>(pre, r + c * ld, z + c * ld, s));
+    return BL_OK;
   };
-  const T* zz = precond(r);
-  BL_REQUIRE(zz != nullptr, "preconditioner failed");
-  k_cg_update_p<T><<<g, kThreads, 0, s>>>(n, zz, p, scal, true);
+  const T* zz = pre ? z : r;
+  if (pre) BL_CHECK(precond());
+  k_cg_update_p<T><<<g, kThreads, 0, s>>>(n, ld, zz, p, scal, true);
   BL_LAUNCHED();
-  k_cg_dot<T><<<g, kThreads, 0, s>>>(n, r, zz, partials, counter, scal, DOT_INIT, nullptr);
+  k_cg_dot<T><<<g, kThreads, 0, s>>>(n, ld, r, zz, partials, counter, scal, DOT_INIT);
   BL_LAUNCHED();
-  int64_t done = 0;
+  std::vector<double> host((size_t)count * S_N);
+  bool polled = false;
   for (int64_t it = 0; it < max_steps; ++it) {
-    BL_CHECK(op->matvec(dtype, p, Ap, s));
-    k_cg_dot<T><<<g, kThreads, 0, s>>>(n, p, Ap, partials, counter, scal, DOT_PAP, nullptr);
+    if (live.size() == 1) {
+      BL_CHECK(op->matvec(dtype, p + live[0] * ld, Ap + live[0] * ld, s));
+    } else {
+      in.clear(), out.clear();
+      for (int64_t c : live) in.push_back(p + c * ld), out.push_back(Ap + c * ld);
+      BL_CHECK(op->matvec_batch(dtype, (int)live.size(), in.data(), out.data(), s));
+    }
+    k_cg_dot<T><<<g, kThreads, 0, s>>>(n, ld, p, Ap, partials, counter, scal, DOT_PAP);
     BL_LAUNCHED();
-    k_cg_update_xr<T><<<g, kThreads, 0, s>>>(n, p, Ap, x, r, atol, rtol, (long long)min_steps, (long long)max_steps,
-                                             partials, counter, scal);
+    k_cg_update_xr<T><<<g, kThreads, 0, s>>>(n, ld, p, Ap, x, r, atol, rtol, (long long)min_steps,
+                                             (long long)max_steps, partials, counter, scal);
     BL_LAUNCHED();
-    zz = precond(r);
-    BL_REQUIRE(zz != nullptr, "preconditioner failed");
-    k_cg_dot<T><<<g, kThreads, 0, s>>>(n, r, zz, partials, counter, scal, DOT_RZ, nullptr);
+    if (pre) BL_CHECK(precond());
+    k_cg_dot<T><<<g, kThreads, 0, s>>>(n, ld, r, zz, partials, counter, scal, DOT_RZ);
     BL_LAUNCHED();
-    k_cg_update_p<T><<<g, kThreads, 0, s>>>(n, zz, p, scal, false);
+    k_cg_update_p<T><<<g, kThreads, 0, s>>>(n, ld, zz, p, scal, false);
     BL_LAUNCHED();
-    done = it + 1;
     if (adaptive && ((it + 1) % check_every == 0 || it + 1 == max_steps)) {
-      double flag[2];
-      BL_CUDA(cudaMemcpyAsync(flag, scal + S_ACTIVE, 16, cudaMemcpyDeviceToHost, s));
+      BL_CUDA(cudaMemcpyAsync(host.data(), scal, host.size() * 8, cudaMemcpyDeviceToHost, s));
       BL_CUDA(cudaStreamSynchronize(s));
-      if (flag[0] == 0.0) {
-        done = (int64_t)flag[1];
-        break;
-      }
+      polled = true;
+      std::vector<int64_t> still;
+      for (int64_t c : live)
+        if (host[(size_t)c * S_N + S_ACTIVE] != 0.0) still.push_back(c);
+      live.swap(still);
+      if (live.empty()) break;
     }
   }
-  if (adaptive && max_steps == 0) done = 0;
-  if (num_steps_host) *num_steps_host = done;
+  if (num_steps_host)
+    for (int64_t c = 0; c < count; ++c)  // fixed steps: every column runs max_steps iterations
+      num_steps_host[c] = !adaptive ? max_steps : polled ? (int64_t)host[(size_t)c * S_N + S_NSTEPS] : 0;
   return BL_OK;
 }
 
@@ -480,6 +523,11 @@ size_t bl_pcg_workspace_bytes(int64_t n, int dtype) {
   return 256 * 3 + align_up(kMaxGrid * 8, 256) + 3 * align_up((size_t)n * dtype_size(dtype), 256) + 1024;
 }
 
+size_t bl_pcg_batch_workspace_bytes(int64_t n, int64_t count, int dtype) {
+  return align_up((size_t)count * S_N * 8, 256) + align_up((size_t)count * kMaxGrid * 8, 256) +
+         align_up((size_t)count * 4, 256) + 3 * align_up((size_t)count * n * dtype_size(dtype), 256) + 1024;
+}
+
 int bl_pcg_solve(bl_operator_t* op, int dtype, int64_t n, const void* b, bl_precond_t* precond, int64_t max_steps,
                  int64_t min_steps, double atol, double rtol, int check_every, void* x, void* r,
                  int64_t* num_steps_host, void* workspace, size_t workspace_bytes, void* stream) {
@@ -490,10 +538,42 @@ int bl_pcg_solve(bl_operator_t* op, int dtype, int64_t n, const void* b, bl_prec
   if (check_every < 1) check_every = 8;
   cudaStream_t s = as_stream(stream);
   if (dtype == BL_F32)
-    return pcg_t<float>(op, dtype, n, (const float*)b, precond, max_steps, min_steps, atol, rtol, check_every, (float*)x,
-                        (float*)r, num_steps_host, workspace, workspace_bytes, s);
-  return pcg_t<double>(op, dtype, n, (const double*)b, precond, max_steps, min_steps, atol, rtol, check_every,
+    return pcg_t<float>(op, dtype, n, 1, n, (const float*)b, precond, max_steps, min_steps, atol, rtol, check_every,
+                        (float*)x, (float*)r, num_steps_host, workspace, workspace_bytes, s);
+  return pcg_t<double>(op, dtype, n, 1, n, (const double*)b, precond, max_steps, min_steps, atol, rtol, check_every,
                        (double*)x, (double*)r, num_steps_host, workspace, workspace_bytes, s);
+}
+
+int bl_pcg_solve_batch(bl_operator_t* op, int dtype, int64_t n, int64_t count, const void* B, int64_t ld,
+                       bl_precond_t* precond, int64_t max_steps, int64_t min_steps, double atol, double rtol,
+                       int check_every, void* X, void* R, int64_t* num_steps_host, void* workspace,
+                       size_t workspace_bytes, void* stream) {
+  BL_REQUIRE(op && B && X && R && workspace && n >= 1 && op->n == n && max_steps >= 0 && count >= 1 && count <= 65535,
+             "bad batched pcg arguments (1 <= count <= 65535)");
+  BL_REQUIRE(dtype == BL_F32 || dtype == BL_F64, "bad dtype");
+  BL_REQUIRE(ld >= n && (ld * (int64_t)dtype_size(dtype)) % 16 == 0, "row stride must be >= n and a multiple of 16 bytes");
+  BL_REQUIRE(!precond || (precond->n == n && precond->dtype == dtype && precond->shift > 0.0),
+             "preconditioner does not match (or has no shift: bl_precond_set_shift)");
+  if (check_every < 1) check_every = 8;
+  cudaStream_t s = as_stream(stream);
+  if (dtype == BL_F32)
+    return pcg_t<float>(op, dtype, n, count, ld, (const float*)B, precond, max_steps, min_steps, atol, rtol, check_every,
+                        (float*)X, (float*)R, num_steps_host, workspace, workspace_bytes, s);
+  return pcg_t<double>(op, dtype, n, count, ld, (const double*)B, precond, max_steps, min_steps, atol, rtol,
+                       check_every, (double*)X, (double*)R, num_steps_host, workspace, workspace_bytes, s);
+}
+
+int bl_rows_dot_pairs(int dtype, int64_t n, int64_t count, const void* X, const void* Y, int64_t ld, double* out,
+                      void* stream) {
+  BL_REQUIRE(X && Y && out && n >= 1 && count >= 1 && count <= INT32_MAX && ld >= n, "bad rows_dot_pairs arguments");
+  BL_REQUIRE(dtype == BL_F32 || dtype == BL_F64, "bad dtype");
+  cudaStream_t s = as_stream(stream);
+  if (dtype == BL_F32)
+    k_rows_dot<float><<<(unsigned)count, kThreads, 0, s>>>(n, (const float*)X, ld, (const float*)Y, ld, out);
+  else
+    k_rows_dot<double><<<(unsigned)count, kThreads, 0, s>>>(n, (const double*)X, ld, (const double*)Y, ld, out);
+  BL_LAUNCHED();
+  return BL_OK;
 }
 
 size_t bl_cholesky_workspace_bytes(int64_t n, int64_t rank, int dtype) {

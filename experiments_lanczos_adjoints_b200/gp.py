@@ -25,9 +25,9 @@ from __future__ import annotations
 
 import numpy as np
 
+from experiments_lanczos_adjoints_b200 import _lib, cg, hutchinson, lanczos
 from experiments_lanczos_adjoints_b200 import device as dev
-from experiments_lanczos_adjoints_b200 import hutchinson, lanczos
-from experiments_lanczos_adjoints_b200.operators import BoundOperator, GramOperator
+from experiments_lanczos_adjoints_b200.operators import BoundOperator, GramOperator, check_test_inputs
 
 
 # ---- parameter constraints (gp_util.py:187-201) ------------------------------------------------
@@ -249,3 +249,68 @@ def target_logml(model, likelihood, /):
     """`gp_util.target_logml` (`gp_util.py:15-33`): `mll(inputs, targets, *p_logpdf, params_mean=,
     params_kernel=, params_likelihood=) -> (value, info)`, plus `.value_and_grad`."""
     return _TargetLogML(model, likelihood)
+
+
+# ---- prediction ----------------------------------------------------------------------------------
+class _Posterior:
+    def __init__(self, model, likelihood: _Likelihood, block: int):
+        self._target = _TargetLogML(model, likelihood)  # shares its operator / preconditioner / residual set-up
+        self.block = int(block)
+
+    def __call__(self, inputs, targets, test_inputs, *, params_mean, params_kernel, params_likelihood, variance=True):
+        X_test = check_test_inputs(test_inputs, np.shape(inputs)[1])  # before any device work
+        dtype, _, _, A, P, info_pre, resid = self._target._setup(inputs, targets, params_mean, params_kernel,
+                                                                 params_likelihood)  # fmt: skip
+        solve = self._target.likelihood.logpdf_p.solve_p
+        alpha, info_solve = solve(A, resid, P)  # (K + s I)^{-1} (y - c); binds A
+        cross = A.op.cross(X_test)
+        c = float(np.asarray(params_mean["constant_value"], dtype=np.float64))
+        mean = cross.matvec(alpha).numpy().astype(np.float64) + c
+        info = {"precondition": info_pre, "solve": info_solve}
+        if not variance:
+            return mean.astype(dtype), None, info
+        M, n = len(X_test), A.n
+        prior = cross.prior_diag().numpy().astype(np.float64)
+        quad = np.empty(M, np.float64)
+        vsolve = cg.vmap_solver(solve)
+        steps = []
+        for t0 in range(0, M, self.block):
+            count = min(self.block, M - t0)
+            Kc = cross.columns(t0, count)  # rows k(x*_t, X)
+            Xc, info_c = vsolve(A, Kc, P)
+            q = dev.empty((count,), np.float64)
+            _lib.call("bl_rows_dot_pairs", dev.dtype_code(dtype), n, count, Kc.ptr, Xc.ptr, Kc.ld, q.ptr,
+                      dev.default_stream().ptr)  # fmt: skip
+            quad[t0 : t0 + count] = q.numpy()
+            if "num_steps" in info_c:
+                steps.append(info_c["num_steps"])
+        maxiter = vsolve._solver.max_steps
+        batch_steps = [int(s.max()) for s in steps] if steps else [maxiter] * ((M + self.block - 1) // self.block)
+        info["variance"] = {
+            "batches": len(batch_steps),
+            "batch_num_steps": batch_steps,  # the largest num_steps of each block
+            "num_steps_max": max(batch_steps),
+            "reached_maxiter": max(batch_steps) >= maxiter,
+        }
+        return mean.astype(dtype), (prior - quad).astype(dtype), info
+
+
+def posterior(model, likelihood, /, *, block: int = 1024):
+    """Posterior of the GP at test inputs: `(inputs, targets, test_inputs, *, params_mean=, params_kernel=,
+    params_likelihood=, variance=True) -> (mean, var, info)`, for the model and likelihood of `target_logml`.
+
+        mean_t = c + K(x*_t, X) alpha,                  alpha = (K + s I)^{-1} (y - c)
+        var_t  = k(x*_t, x*_t) - k_t^T (K + s I)^{-1} k_t,  k_t = K(X, x*_t)
+
+    This is the prediction half of the reference's GP utilities (its `likelihood_condition` /
+    `target_posterior` build the same two quantities); the calling convention here follows `target_logml`.
+    Every solve uses the likelihood's `solve_p` and preconditioner.  The variances are latent (no noise term)
+    and exact up to the solver tolerance: one solve per test point, `block` test points in lockstep
+    (`cg.vmap_solver`) sharing every Gram sweep; `k(x, x)` is the kernel formula at zero distance.  `info`
+    has the mean solve's info and, for the variances, the number of blocks, the largest `num_steps` of each
+    block and of all columns, and whether any column reached `maxiter` (a fixed-step solver reports its step
+    count and True).
+
+    fp32 on the tensor-core path: the squared distance of a test point that coincides with a training point
+    is O(eps |x|^2), not 0, and the Matérn square root magnifies that; predict at training points in fp64."""
+    return _Posterior(model, likelihood, block)

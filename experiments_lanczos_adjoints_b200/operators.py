@@ -231,6 +231,81 @@ class GramOperator(Operator):
     def grad_export(self, dtype, like=None, stream=None):
         return super().grad_export(dtype, like=[(self.d,), (1,), (1,)], stream=stream)
 
+    def cross(self, X_test):
+        """The cross-covariance `K(X_test, X)` with this operator's kernel (see `GramCross`)."""
+        return GramCross(self, X_test)
+
+
+def check_test_inputs(X_test, d: int) -> np.ndarray:
+    """`X_test` as a C-contiguous (M, d) float64 array; `ValueError` for another shape, no points or a
+    non-finite entry."""
+    X_test = np.ascontiguousarray(np.asarray(X_test, dtype=np.float64))
+    if X_test.ndim != 2 or X_test.shape[1] != d:
+        raise ValueError(f"X_test must be (M, {d}), got shape {X_test.shape}")
+    if X_test.shape[0] == 0:
+        raise ValueError("X_test has no points")
+    if not np.all(np.isfinite(X_test)):
+        raise ValueError("X_test has non-finite entries")
+    return X_test
+
+
+class GramCross:
+    """Cross-covariance of a `GramOperator` with `M` test points: `matvec(v) = K(X*, X) v` (M values),
+    `columns(first, count)` the rows `k(x*_t, X)` of `count` test points as a `(count, n)` device array (row
+    stride 16-byte aligned), `prior_diag()` = `k(x*_t, x*_t)` (the kernel formula at zero distance, so
+    `sigma (1 + sqrt(eps)) e^-sqrt(eps)` for Matérn-3/2).  Every call uses the kernel parameters the parent
+    operator was last bound with, in that dtype (bind it first); the noise is never read.
+
+    fp32 on the tensor-core path: `s2 = |x|^2 + |y|^2 - 2 x.y` is exact only on the square operator's diagonal,
+    where it is forced to zero.  A test point that coincides with a training point gets `s2 = O(eps |x|^2)`
+    instead of 0, which the Matérn square root magnifies; such points need fp64."""
+
+    def __init__(self, gram: GramOperator, X_test):
+        X_test = check_test_inputs(X_test, gram.d)
+        self.parent, self.m, self.n = gram, int(X_test.shape[0]), gram.n
+        h = C.c_void_p()
+        _lib.call("bl_gram_cross_create", gram._handle, self.m, X_test.ctypes.data, C.byref(h))
+        self._handle = h.value
+
+    def __del__(self):
+        h, self._handle = getattr(self, "_handle", None), None
+        if h:
+            try:
+                _lib.load().bl_gram_cross_destroy(h)
+            except Exception:
+                pass
+
+    def _dtype(self):
+        if self.parent._bound is None:
+            raise RuntimeError("bind the parent GramOperator first")
+        return self.parent._bound[0]
+
+    def matvec(self, v, stream=None):
+        stream = stream or dev.default_stream()
+        v = dev.asarray(v, dtype=self._dtype())
+        if v.shape != (self.n,):
+            raise ValueError(f"v must have {self.n} entries, got shape {v.shape}")
+        out = dev.empty((self.m,), v.dtype)
+        _lib.call("bl_gram_cross_matvec", self._handle, dev.dtype_code(v.dtype), v.ptr, out.ptr, stream.ptr)
+        return out
+
+    def columns(self, first, count, stream=None):
+        first, count = int(first), int(count)
+        if first < 0 or count < 1 or first + count > self.m:
+            raise ValueError(f"columns [{first}, {first + count}) out of range for {self.m} test points")
+        dtype = self._dtype()
+        out = dev.empty((count, self.n), dtype, ld=dev.basis_ld(self.n, dtype))
+        _lib.call("bl_gram_cross_columns", self._handle, dev.dtype_code(dtype), first, count, out.ptr, out.ld,
+                  (stream or dev.default_stream()).ptr)  # fmt: skip
+        return out
+
+    def prior_diag(self, stream=None):
+        dtype = self._dtype()
+        out = dev.empty((self.m,), dtype)
+        _lib.call("bl_gram_cross_prior_diag", self._handle, dev.dtype_code(dtype), out.ptr,
+                  (stream or dev.default_stream()).ptr)  # fmt: skip
+        return out
+
 
 class WaveStencilOperator(Operator):
     """`(u, du) -> (du, scale^2 * conv3x3(stencil, edge_pad(u)))` on a `g x g` grid

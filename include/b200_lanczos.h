@@ -212,6 +212,22 @@ int bl_op_gram_set_path(bl_operator_t* op, int path);
  * is added in the epilogue) for the tile of rows [128 row_tile, +128) x columns [256 col_tile, +256),
  * written to out_host[128][256] (fp32; entries beyond n are padding).  col_tile must be the first tile of a column split.  Synchronises `stream`. */
 int bl_op_gram_tile_distances(bl_operator_t* op, int64_t row_tile, int64_t col_tile, float* out_host, void* stream);
+/* Cross-covariance of a Gram operator with m test points X* (the prediction half of a GP): the test points
+ * are scaled (and packed for the tensor-core path) with the kernel parameters bound to `gram`, and again
+ * whenever `gram` is re-bound; its noise is never read.  `gram` must outlive the object.  Xtest_host is
+ * m x d row-major doubles.  dtype must be the dtype `gram` was last bound with.
+ *   matvec     : y (m) = K(X*, X) v (v of length n), the square sweeps' kernels on a rectangular operand;
+ *   columns    : out[b * ld + j] = k(x*_{first+b}, x_j), b < count <= 65535, j < n (ld >= n);
+ *   prior_diag : out[t] = k(x*_t, x*_t), the kernel formula at s2 = 0 (Matern: sigma (1 + sqrt(eps)) e^-sqrt(eps)).
+ * fp32 on tensor cores: s2 = |x|^2 + |y|^2 - 2 x.y is exact only on the square operator's diagonal, so a test
+ * point that coincides with a training point gets s2 = O(eps |x|^2) rather than 0. */
+typedef struct bl_gram_cross bl_gram_cross_t;
+int bl_gram_cross_create(bl_operator_t* gram, int64_t m, const double* Xtest_host, bl_gram_cross_t** out);
+int bl_gram_cross_destroy(bl_gram_cross_t* cross);
+int bl_gram_cross_matvec(bl_gram_cross_t* cross, int dtype, const void* v, void* y, void* stream);
+int bl_gram_cross_columns(bl_gram_cross_t* cross, int dtype, int64_t first, int64_t count, void* out, int64_t ld,
+                          void* stream);
+int bl_gram_cross_prior_diag(bl_gram_cross_t* cross, int dtype, void* out, void* stream);
 
 /* Wave-equation stencil operand (util/pde_util.py:126-157): state (u, du) of 2 g^2 values,
  * A(u,du) = (du, scale^2 * conv3x3(stencil, edge_pad(u))).  One parameter: scale (g*g). */
@@ -350,6 +366,22 @@ size_t bl_pcg_workspace_bytes(int64_t n, int dtype);
 int bl_pcg_solve(bl_operator_t* op, int dtype, int64_t n, const void* b, bl_precond_t* precond, int64_t max_steps,
                  int64_t min_steps, double atol, double rtol, int check_every, void* x, void* r,
                  int64_t* num_steps_host, void* workspace, size_t workspace_bytes, void* stream);
+/* `count` independent solves A X[c] = B[c] in lockstep, each column under bl_pcg_solve's rules (same
+ * modes, _safe_divide, min_steps, its own freeze).  Every iteration takes one matvec_batch over the columns
+ * the host still knows to be active (the Gram operator evaluates each kernel tile once for up to 16 of
+ * them); dots, step lengths and updates are one launch per vector operation for all columns.  The host
+ * reads the columns' flags back in one copy every `check_every` iterations.  B, X, R: count rows of n
+ * values, row stride ld (ld >= n, ld * dtype size a multiple of 16 bytes); num_steps_host: count values.
+ * The preconditioner is applied column by column. */
+/* workspace of bl_pcg_solve_batch: pass the row stride ld as n */
+size_t bl_pcg_batch_workspace_bytes(int64_t n, int64_t count, int dtype);
+int bl_pcg_solve_batch(bl_operator_t* op, int dtype, int64_t n, int64_t count, const void* B, int64_t ld,
+                       bl_precond_t* precond, int64_t max_steps, int64_t min_steps, double atol, double rtol,
+                       int check_every, void* X, void* R, int64_t* num_steps_host, void* workspace,
+                       size_t workspace_bytes, void* stream);
+/* out[j] = <X[j], Y[j]> for j < count (rows of n values, row stride ld; out: count doubles on the device) */
+int bl_rows_dot_pairs(int dtype, int64_t n, int64_t count, const void* X, const void* Y, int64_t ld, double* out,
+                      void* stream);
 
 /* Partial Cholesky factorisation of the lazily evaluated matrix of `op` (dense operand: its matrix; Gram
  * operand: the kernel matrix WITHOUT the noise term, gp_util.py:257-258).  pivot = 0: low_rank.py:63-118;
